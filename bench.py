@@ -23,6 +23,8 @@ every rank, the counts are merged with one all-reduce.
           all host cores, built -O3 -march=native on the host it runs on) on a bounded sample of the same workload
           -- a reported baseline, not the target
   --impl reference : that CPU path as its own arm (the upstream binaries are not in the image: kind "port")
+  --dump-outputs DIR : after the timed steps, what the last timed step computed as DIR/<name>.npy (float64), so that two
+          builds can be compared output for output on the same seeded inputs (see dump_outputs)
 """
 import argparse
 import json
@@ -55,7 +57,13 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 class Plan:
@@ -285,6 +293,38 @@ def load_truth_keys(name):
     return np.array(tk, dtype=np.uint64)
 
 
+DUMP_COUNT_COLS = 1 << 18                  # count-tensor columns dumped at most: 16 channels x 8 B x 262,144 = 32 MB
+
+
+def dump_outputs(dirname, s, r, stats, d_calls):
+    """what one resident step hands its caller, as float64 .npy files (every value is an int32 or a float32: exact)
+      counts.npy      [16, n]  the sample's count tensor (channel planes, include/quasimodo_b200.h) at the columns of
+                               counts_pos.npy: all of them, or a fixed seeded sample of 262,144 on a longer reference
+      counts_pos.npy  [n]      those columns (positions in the concatenated reference)
+      calls.npy       [c, 11]  the SNP calls: rid, pos, ref, alt, dp, ad_ref_f, ad_ref_r, ad_alt_f, ad_alt_r, qual, af
+      eval.npy        [4]      calls, TP, FP, FN against the truth set (the finish_sample tuple)
+      stats.npy       [2]      pairs added, executed ksw_extend2 cells
+    At most 32 MB of counts + 23 MB of calls (2^18 calls)."""
+    import numpy as np
+    import torch
+    from quasimodo_b200 import _lib
+    os.makedirs(dirname, exist_ok=True)
+    counts = s.counts_tensor()
+    n = counts.shape[1]
+    if n <= DUMP_COUNT_COLS:
+        pos = np.arange(n)
+        cols = counts.cpu().numpy()
+    else:
+        pos = np.sort(np.random.default_rng(0).choice(n, DUMP_COUNT_COLS, replace=False))
+        cols = counts[:, torch.from_numpy(pos).to(counts.device)].cpu().numpy()
+    calls = d_calls[:r[0] * _lib.CALL_DTYPE.itemsize].cpu().numpy().view(_lib.CALL_DTYPE)
+    fields = [f for f in _lib.CALL_DTYPE.names if not f.startswith("pad")]
+    out = {"counts": cols, "counts_pos": pos, "calls": np.column_stack([calls[f] for f in fields]).reshape(-1, len(fields)),
+           "eval": np.array(r), "stats": np.array(stats)}
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import ctypes as C
     import numpy as np
@@ -362,6 +402,7 @@ def run_ours(args):
     d_calls = torch.empty(max_calls * 40, dtype=torch.uint8, device=dev)
     copt = _lib.default_call_opt()
     results = {}
+    last_step = []                                    # (sample, finish_sample's result, stats) of the latest step
 
     def finish_sample(i, s, key):
         """all-reduce (N>1), call SNPs, classify against the truth set; returns (n_calls, tp, fp, fn)"""
@@ -400,7 +441,9 @@ def run_ours(args):
         r = finish_sample(j, s, key)
         if r is not None:
             results[W.name + (f"@{plan.window(j)}" if plan.cfg == 1 else "")] = r
-        return s.stats(st)[1]                          # executed ksw_extend2 cells of this step (8-byte read-back)
+        stats = s.stats(st)                            # (pairs, executed ksw_extend2 cells) of this step (8-byte read-back)
+        last_step[:] = [s, r, stats]
+        return stats[1]
 
     def barrier():
         torch.cuda.synchronize()
@@ -433,6 +476,8 @@ def run_ours(args):
     stage_ms, stage_launch = ctx.profile_collect()
     ctx.profile_enable(False)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:               # before the e2e steps reuse the samples
+        dump_outputs(args.dump_outputs, *last_step, d_calls)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -628,6 +673,7 @@ def run_ours(args):
 if __name__ == "__main__":
     # stdout carries exactly one JSON line: whatever else a library prints there (NCCL's version banner, for one) goes to
     # stderr -- file descriptor 1 is pointed at stderr for the whole run and the line is written to the saved original
+    sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written into it
     sys.stdout.flush()
     _json_out = os.fdopen(os.dup(1), "w")
     os.dup2(2, 1)

@@ -1,9 +1,12 @@
 """ctypes binding of the CPU oracle (oracle/libqmo.so).  TEST INFRASTRUCTURE ONLY: importable from
 tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs; never from the
 product package."""
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -37,11 +40,14 @@ BUILD_KIND = "-O3, portable x86-64"
 
 def use_native_build():
     """bench.py's CPU arms: rebuild the restatement with -O3 -march=native ON THIS HOST (never shipped) and use it from now on.
-    Falls back to the portable build when the compile fails."""
+    The library goes to a temporary directory, removed at exit: the tree may be read-only.  Falls back to the portable build
+    when the compile fails."""
     global _LIB, BUILD_KIND
-    so = os.path.join(_HERE, "libqmo_native.so")
+    d = tempfile.mkdtemp(prefix="qmo_native_")
+    atexit.register(shutil.rmtree, d, True)
+    so = os.path.join(d, "libqmo_native.so")
     try:
-        subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "libqmo_native.so"])
+        subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "native"], env=dict(os.environ, NATIVE_OUT=so))
     except (subprocess.CalledProcessError, OSError):
         return False
     _LIB = None

@@ -28,7 +28,6 @@ def test_index_equals_bwas_own_files(stem):
     assert again.bwt_bytes() == b and again.sa_bytes() == s
 
 
-@pytest.mark.skipif(not os.environ.get("QM_SLOW"), reason="9.3 M suffixes take ~15 s: QM_SLOW=1 (verified in the build container, DESIGN.md)")
 def test_ecoli_suffix_array_samples_equal_bwas_file():
     G = genomes.load("Ecoli")
     s = qmo_py.FmIndex(codes=G.codes).sa_bytes()

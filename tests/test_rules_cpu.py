@@ -1,58 +1,32 @@
-"""Static check of the drop-in boundary (SURVEY.md 8b): every `output:` / `log:` path the reference's rules `bwa`, `rmdup`,
-`mpileup` and `bcftools` declare is one quasimodo_b200.rules knows and the driver command writes.  Parses the reference's own
-rule files, so it only runs where /root/reference exists (the build container)."""
+"""Static check of the drop-in boundary (SURVEY.md 8b): every `output:` / `log:` / `benchmark:` path the reference's rules `bwa`,
+`rmdup`, `mpileup` and `bcftools` declare is one quasimodo_b200.rules knows and the driver command writes.  What the reference's
+own rule files declare is stored in tests/golden/rule_contract.json (made by tests/golden/make_rules_golden.py from a Quasimodo
+checkout)."""
+import json
 import os
-import re
-
-import pytest
 
 from quasimodo_b200 import rules
 
-REF = "/root/reference/rules"
+GOLD = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "rule_contract.json")))
 
 
-def parse_rule(path, rule):
-    """-> (outputs {name: (dir variable, pattern)}, log (dir variable, pattern) or None) of `rule` in a .smk file"""
-    text = open(path).read()
-    m = re.search(rf"^rule {rule}:\n(.*?)(?=^rule |\Z)", text, re.S | re.M)
-    assert m, f"rule {rule} not found in {path}"
-    body = m.group(1)
-
-    def section(key):
-        s = re.search(rf"^    {key}:\s*\n((?:^        .*\n|^\s*\n)*)", body, re.M)
-        return s.group(1) if s else ""
-
-    def entries(sec):
-        out = {}
-        for ln in sec.splitlines():
-            ln = ln.split("#")[0].strip().rstrip(",")
-            if not ln:
-                continue
-            e = re.match(r'(?:(\w+)\s*=\s*)?(\w+)\s*\+\s*"([^"]+)"$', ln)
-            assert e, f"unparsed line in rule {rule}: {ln!r}"
-            out[e.group(1) or ""] = (e.group(2), e.group(3))
-        return out
-
-    outs = entries(section("output"))
-    log = entries(section("log"))
-    bench = entries(section("benchmark"))
-    return outs, (log.get("") if log else None), (bench.get("") if bench else None)
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is not on this machine")
 def test_declared_outputs_of_the_replaced_rules_are_all_produced():
-    where = {"bwa": "bwa.smk", "rmdup": "rmdup.smk", "mpileup": "vcfcall.smk", "bcftools": "vcfcall.smk"}
-    for rule, f in where.items():
-        outs, log, bench = parse_rule(os.path.join(REF, f), rule)
+    assert sorted(GOLD["rules"]) == sorted(rules.RULE_OUTPUTS)
+    for rule, want in GOLD["rules"].items():
+        outs = {k: tuple(v) for k, v in want["output"].items()}
         assert outs == rules.RULE_OUTPUTS[rule], (rule, outs)
-        assert log == rules.RULE_LOGS.get(rule), (rule, log)
-        assert bench == rules.RULE_BENCHMARKS.get(rule), (rule, bench)
+        assert (tuple(want["log"]) if want["log"] else None) == rules.RULE_LOGS.get(rule), (rule, want["log"])
+        assert (tuple(want["benchmark"]) if want["benchmark"] else None) == rules.RULE_BENCHMARKS.get(rule), (rule, want["benchmark"])
         for name in outs:
             assert (rule, name) in rules.DRIVER_OPTION, f"output {name!r} of rule {rule} has no driver option"
     # the shell lines' side files: `samtools index` after bwa and rmdup, `tabix -p vcf` after bcftools
-    assert "samtools index {output.sortedbam}" in open(os.path.join(REF, "bwa.smk")).read()
-    assert "samtools index {output.rmdupbam}" in open(os.path.join(REF, "rmdup.smk")).read()
-    assert "tabix -p vcf {output.vcf_bgz}" in open(os.path.join(REF, "vcfcall.smk")).read()
+    side = {}
+    for f, lines in GOLD["shell"].items():
+        rule_of = {o: r for r, w in GOLD["rules"].items() if w["file"] == f for o in w["output"]}
+        for ln in lines:
+            out = ln.rsplit("{output.", 1)[1].rstrip("}")
+            side[(rule_of[out], out)] = ".bai" if ln.startswith("samtools index ") else ".tbi"
+    assert side == rules.SIDE_FILES
 
 
 def test_sample_command_names_every_path(tmp_path):
