@@ -184,7 +184,8 @@ int qm_pair_finish(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
  *  15 admitted reads whose leftmost aligned base is here
  * Admission as bcftools mpileup: skip UNMAP|SECONDARY|QCFAIL|DUP, MAPQ < min_mapq, and paired reads that
  * are not proper pairs unless count_orphans; mate-overlap quality rewrite unless ignore_overlaps; BAQ off
- * (-B) and no depth cap (deliberate, SURVEY.md A.8).  Accumulates (+=) into d_counts. */
+ * (-B) and no depth cap (deliberate, SURVEY.md A.8).  Accumulates (+=) into d_counts.
+ * Reads as in the read batch layout, lens[r] <= stride; stride <= 512 (QM_ELIMIT otherwise, nothing counted). */
 #define QM_NCH 16
 typedef struct {
     int32_t min_mapq;        /* -q (0)   */

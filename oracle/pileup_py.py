@@ -197,29 +197,26 @@ def mpileup_text(ref_codes, ref_offs, ref_lens, contig_names, alns, codes, quals
         v = view[r]
         a, L, rid = v["a"], v["L"], int(v["a"]["rid"])
         ops = [(int(c) & 15, int(c) >> 4) for c in a["cigar"][:int(a["n_cigar"])]]
-        follows = {}                                       # reference position of the last base of an M / D run -> the indel right after it
+        # htslib resolve_cigar2 gives a deleted base the query cursor at its D operation (p->qpos = s->y): the first query
+        # base behind the deletion in read order, whatever operation holds it (M, I or S), or l_qseq when the read ends there.
+        # samtools takes that base's quality (0 past the end) and prints an insertion as the bases at qpos + 1 .. qpos + n.
+        follows = {}                                       # reference position of the last base of an M / D run -> (indel after it, its qpos)
+        del_q = {}                                         # reference position of a deleted base -> its qpos
         q, pos = 0, int(a["pos"])
         for i, (op, ln) in enumerate(ops):
+            if op == D:
+                del_q.update((pos + j, q) for j in range(ln))
             if op in (M, D):
                 pos += ln
                 if i + 1 < len(ops) and ops[i + 1][0] in (I, D):
-                    follows[pos - 1] = (ops[i + 1][0], ops[i + 1][1], q + (ln if op == M else 0))
+                    follows[pos - 1] = (ops[i + 1][0], ops[i + 1][1], q + ln - 1 if op == M else q)
             if op in (M, I, S):
                 q += ln
         last = pos - 1
         letters = "acgtn" if v["rev"] else "ACGTN"
-        nxt = {}                                           # a deleted base borrows the quality of the query base after the deletion
-        pending = []
-        for cpos, qp in v["cols"]:
-            if qp is None:
-                pending.append(cpos)
-            else:
-                for d in pending:
-                    nxt[d] = qp
-                pending = []
         for cpos, qp in v["cols"]:
             col = columns.setdefault((rid, cpos), [[], []])
-            qq = qp if qp is not None else nxt.get(cpos, L)
+            qq = qp if qp is not None else del_q[cpos]
             qual = int(v["q"][qq]) if qq < L else 0
             if qual < min_bq:
                 continue
@@ -232,9 +229,9 @@ def mpileup_text(ref_codes, ref_offs, ref_lens, contig_names, alns, codes, quals
                 b = int(v["seq"][qp])
                 s += ("," if v["rev"] else ".") if b < 4 and b == int(ref_codes[int(ref_offs[rid]) + cpos]) else letters[b]
             if cpos in follows:
-                kind, ln, q_after = follows[cpos]
+                kind, ln, qpos = follows[cpos]
                 if kind == I:
-                    s += "+%d" % ln + "".join(letters[int(v["seq"][q_after + j])] if q_after + j < L else letters[4] for j in range(ln))
+                    s += "+%d" % ln + "".join(letters[int(v["seq"][qpos + j])] if qpos + j < L else letters[4] for j in range(1, ln + 1))
                 else:
                     s += "-%d" % ln + "".join(letters[int(ref_codes[int(ref_offs[rid]) + cpos + 1 + j])] if cpos + 1 + j < int(ref_lens[rid]) else letters[4]
                                               for j in range(ln))

@@ -473,6 +473,8 @@ int qm_pileup_accumulate_masked(qm_ctx *ctx, const qm_index *idx, const qm_pileu
         return QM_EINVAL;
     if (tab && tab->ctx != ctx) return qm_fail(ctx, QM_EINVAL, "the indel table belongs to another context");
     if (n_pairs == 0) return QM_OK;
+    // the kernel stages at most kMaxLen bases per read; a longer read would otherwise be dropped without a word
+    if (stride > kMaxLen) return qm_fail(ctx, QM_ELIMIT, "qm_pileup_accumulate: reads longer than %d bases (stride %d)", kMaxLen, stride);
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
     int64_t blocks = (n_pairs + kWarpsPerBlock - 1) / kWarpsPerBlock;
     const int64_t cap = (int64_t)ctx->sm_count * 16;       // persistent: 16 blocks x 4 warps per SM
