@@ -376,11 +376,57 @@ int qm_sample_kept_alns_host(qm_sample *s, qm_aln *h_alns, int64_t max_records);
 int qm_depth_cap(qm_ctx *ctx, const qm_pileup_opt *po, int n_chunks, const qm_aln *const *d_alns, const int64_t *n_pairs, int max_depth,
                  uint8_t *const *d_drop, int64_t *h_n_dropped, void *stream);
 int qm_sample_set_max_depth(qm_sample *s, int max_depth);
+/* qm_sample_finish decides over this object's pairs only, even with a communicator set: a sample sharded over ranks finishes with
+ * qm_sample_finish_comm (below). */
 int qm_sample_finish(qm_sample *s, int64_t *n_dup_pairs, int64_t *n_capped_reads, void *stream);
 /* base alignment quality for the sample's pileup (qm_baq_apply above): 0 = off (default, `-B`), 3 = extended BAQ as both mpileups of
  * the reference flow run it, 1 = plain BAQ; before the first pairs.  Works with the immediate and the deferred (rmdup / depth cap)
  * counting; duplicate marking keeps the reads' own qualities. */
 int qm_sample_set_baq(qm_sample *s, int flag);
+
+/* ---- duplicate marking and depth cap over a sample sharded across ranks ----
+ * Both decisions split into an export and a decide step.  Every rank exports one small tuple per pair (duplicates) or per
+ * admitted read (cap), tagged with a sample-wide id; the ranks all-gather the tuples; every rank runs the decision over the union
+ * and applies it to its own records.  The decision sees identical data on every rank, so the result is the one of a single
+ * device holding the whole sample, and every rank reaches the same verdict on an invalid union.
+ * Pair ids must be unique across ranks (a pair's id is what its position in the sample is on one device: the running pair
+ * offset; gaps are allowed).  Chunk c holds pairs pair_id0[c] .. pair_id0[c] + n_pairs[c] - 1.  Read ids are 2 * pair id + mate
+ * and must fit in an int32 (pair ids below 2^30).
+ * qm_dup_keys: one qm_dup_key per pair with a placed end (pairs without one are never duplicates and are left out), in no
+ * particular order; d_out holds up to sum(n_pairs) records, *h_n_out receives the number written.  end0 / end1: the 31-bit codes of
+ * the two ends of a fully placed pair, 0xffffffff for none.  Synchronous; QM_ELIMIT when an end code does not fit (as
+ * qm_mark_duplicates).
+ * qm_mark_duplicates_keys: d_all is the union of every rank's tuples (any order).  Orders it by pair id (a repeated id: QM_EINVAL,
+ * nothing flagged), decides as qm_mark_duplicates with ties to the lowest pair id, and sets 0x400 on the records of the local
+ * chunks only.  *h_n_dup_all: duplicate pairs of the whole union.  Synchronous.
+ * qm_cap_keys: one qm_cap_key per read the pileup admits (po: min_mapq, count_orphans; reads flagged 0x400 are out), any order;
+ * d_out holds up to 2 * sum(n_pairs) records.  Synchronous.
+ * qm_depth_cap_keys: d_all is the union of every rank's cap tuples.  Orders it by read id (a repeated id: QM_EINVAL, nothing
+ * written), then stably by key (BAM order, ties in read order), replays htslib's iterator on the host as qm_depth_cap and writes
+ * the drop bytes of the local reads (d_drop[c]: 2 * n_pairs[c] bytes).  *h_n_dropped_all: reads dropped in the whole union.
+ * Synchronous.
+ * Memory per rank: the whole union of tuples plus its sort scratch on the device (about 150 bytes per pair of the sample for
+ * duplicates, 70 per admitted read for the cap, the all-gather's buffers included) and 17 bytes per admitted read of the sample on the host for the replay. */
+typedef struct {
+    int64_t  pair_id;
+    uint64_t key;                         /* the duplicate key: both ends of a fully placed pair, or the one placed end (bit 63) */
+    uint32_t end0, end1;                  /* end codes of a fully placed pair; 0xffffffff = none */
+    int32_t  score, pad;                  /* sum of base qualities >= 15 over the placed ends */
+} qm_dup_key;
+typedef struct {
+    uint64_t key;                         /* contig << 33 | start << 1 | reverse */
+    int32_t  read_id;                     /* 2 * pair id + mate */
+    int32_t  end;                         /* end of the read's reference span (exclusive) */
+} qm_cap_key;
+int qm_dup_keys(qm_ctx *ctx, int n_chunks, const qm_aln *const *d_alns, const uint8_t *const *d_quals, const int32_t *strides,
+                const int32_t *const *d_lens, const int64_t *n_pairs, const int64_t *pair_id0, qm_dup_key *d_out, int64_t *h_n_out,
+                void *stream);
+int qm_mark_duplicates_keys(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all, int n_chunks, qm_aln *const *d_alns,
+                            const int64_t *n_pairs, const int64_t *pair_id0, int64_t *h_n_dup_all, void *stream);
+int qm_cap_keys(qm_ctx *ctx, const qm_pileup_opt *po, int n_chunks, const qm_aln *const *d_alns, const int64_t *n_pairs,
+                const int64_t *pair_id0, qm_cap_key *d_out, int64_t *h_n_out, void *stream);
+int qm_depth_cap_keys(qm_ctx *ctx, const qm_cap_key *d_all, int64_t n_all, int max_depth, int n_chunks, const int64_t *n_pairs,
+                      const int64_t *pair_id0, uint8_t *const *d_drop, int64_t *h_n_dropped_all, void *stream);
 
 /* ---- text pileup (replaces `samtools mpileup -f ref bam`, rules/vcfcall.smk:39; consumer: the VarScan rule) ----
  * One line per column covered by an admitted read: chrom, 1-based position, reference base, number of entries with base
@@ -427,6 +473,18 @@ int  qm_comm_allgather(qm_ctx *ctx, qm_comm *comm, const void *d_send, void *d_r
  * into every rank's table); synchronous.  Set the communicator before the first pairs; NULL clears. */
 int  qm_sample_set_comm(qm_sample *s, qm_comm *comm);
 int  qm_sample_allreduce_counts(qm_sample *s, void *stream);
+/* Deferred counting (rmdup / depth cap) of a sample spread over the ranks of `comm`.  qm_sample_finish decides over this object's
+ * pairs only, even when a communicator is set: a duplicate whose original lies on another rank stays unflagged there.
+ * qm_sample_finish_comm decides over the whole sample: each rank exports its duplicate tuples (qm_dup_keys, ids = the pair_id0 its
+ * pairs were added with), the ranks all-gather them (counts first, then the tuples padded to the largest count), every rank marks
+ * its own records (qm_mark_duplicates_keys); the same for the cap tuples (qm_cap_keys, qm_depth_cap_keys); then each rank counts its
+ * survivors.  Collective: every rank of `comm` calls it, with one host thread per GPU when one process drives several.  It does not
+ * sum the counts: call qm_sample_allreduce_counts or qm_counts_allreduce next.  *n_dup_pairs and *n_capped_reads are sample-wide and
+ * equal on every rank.  The communicator is an argument, not the sample's own (a one-process driver sets none on its samples).
+ * Pair ids must be unique across ranks; memory per rank as for qm_mark_duplicates_keys / qm_depth_cap_keys.  A rank that fails
+ * before the first all-gather (QM_ELIMIT from an export, out of memory) leaves the other ranks waiting in it, as with the other
+ * collectives; errors of the decision (a repeated id) are reached by every rank alike.  Synchronous. */
+int  qm_sample_finish_comm(qm_sample *s, qm_comm *comm, int64_t *n_dup_pairs, int64_t *n_capped_reads, void *stream);
 
 /* ---- stage timers: CUDA events recorded on the launching stream around every kernel group ----
  * stages: 0 seed+chain, 1 advance (extension state machine), 2 extend (ksw_extend2 kernels), 3 pair+CIGAR,

@@ -62,6 +62,9 @@ REG_DTYPE = np.dtype([("rb", "<i8"), ("re", "<i8"), ("qb", "<i4"), ("qe", "<i4")
 ALN_DTYPE = np.dtype([("rid", "<i4"), ("pos", "<i4"), ("flag", "<u2"), ("mapq", "u1"), ("n_cigar", "u1"),
                       ("score", "<i4"), ("sub", "<i4"), ("nm", "<i4"), ("mate_rid", "<i4"), ("mate_pos", "<i4"),
                       ("tlen", "<i4"), ("qb", "<i4"), ("qe", "<i4"), ("cigar", "<u4", (MAX_CIGAR,))])
+DUP_KEY_DTYPE = np.dtype([("pair_id", "<i8"), ("key", "<u8"), ("end0", "<u4"), ("end1", "<u4"), ("score", "<i4"), ("pad", "<i4")])
+CAP_KEY_DTYPE = np.dtype([("key", "<u8"), ("read_id", "<i4"), ("end", "<i4")])
+assert DUP_KEY_DTYPE.itemsize == 32 and CAP_KEY_DTYPE.itemsize == 16
 PESTAT_DTYPE = np.dtype([("low", "<i4"), ("high", "<i4"), ("failed", "<i4"), ("pad", "<i4"), ("avg", "<f8"), ("std", "<f8")])
 assert REG_DTYPE.itemsize == 64 and ALN_DTYPE.itemsize == 128 and SEED_DTYPE.itemsize == 16 and PESTAT_DTYPE.itemsize == 32
 QM_EXT_BAND_RETRY = 1
@@ -123,6 +126,11 @@ SIGNATURES = {
     "qm_sample_kept_alns_host": (C.c_int, [_P, _P, _L]),
     "qm_depth_cap": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, _P, C.POINTER(C.c_int64), _P]),
     "qm_sample_set_max_depth": (C.c_int, [_P, C.c_int]),
+    "qm_dup_keys": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, _P, _P, _P, C.POINTER(C.c_int64), _P]),
+    "qm_mark_duplicates_keys": (C.c_int, [_P, _P, _L, C.c_int, _P, _P, _P, C.POINTER(C.c_int64), _P]),
+    "qm_cap_keys": (C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P, C.POINTER(C.c_int64), _P]),
+    "qm_depth_cap_keys": (C.c_int, [_P, _P, _L, C.c_int, C.c_int, _P, _P, _P, C.POINTER(C.c_int64), _P]),
+    "qm_sample_finish_comm": (C.c_int, [_P, _P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P]),
     "qm_sample_finish": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P]),
     "qm_sample_set_baq": (C.c_int, [_P, C.c_int]),
     "qm_baq_apply": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _I, _P, _P]),

@@ -19,6 +19,21 @@ def _ptr(t):
     return C.c_void_p(0 if t is None else t.data_ptr())
 
 
+def _ptrs(ts):
+    """array of device pointers of a list of torch tensors"""
+    return (C.c_void_p * max(1, len(ts)))(*[t.data_ptr() for t in ts])
+
+
+def _i64(v):
+    """ctypes int64 array of a list of ints (passed as the object itself, so it lives through the call)"""
+    return (C.c_int64 * max(1, len(v)))(*[int(x) for x in v])
+
+
+def _n_pairs(d_alns):
+    """pairs in a device tensor of alignment records (2 records of 128 bytes per pair)"""
+    return d_alns.numel() * d_alns.element_size() // 256
+
+
 class Index:
     """Device-resident k-mer hash index + reference bases (qm_index)."""
 
@@ -83,6 +98,21 @@ class Comm:
         buf = (C.c_uint8 * 128).from_buffer_copy(bytes(uid))
         _check(ctx._h, _lib.lib().qm_comm_init_rank(ctx._h, int(n_ranks), int(rank), buf, C.byref(self._h)), "qm_comm_init_rank")
         self.rank, self.size = int(rank), int(n_ranks)
+
+    @classmethod
+    def init_all(cls, ctxs):
+        """one communicator per context, all in this process (qm_comm_init_all): comms[i] belongs to ctxs[i]; call the collectives
+        from one host thread per GPU"""
+        n = len(ctxs)
+        hs = (C.c_void_p * n)(*[c._h for c in ctxs])
+        out = (C.c_void_p * n)()
+        _check(ctxs[0]._h, _lib.lib().qm_comm_init_all(n, hs, out), "qm_comm_init_all")
+        comms = []
+        for r, c in enumerate(ctxs):
+            cm = cls.__new__(cls)
+            cm.ctx, cm._h, cm.rank, cm.size = c, C.c_void_p(out[r]), r, n
+            comms.append(cm)
+        return comms
 
     def close(self):
         if getattr(self, "_h", None):
@@ -189,6 +219,14 @@ class Sample:
         """deferred counting (rmdup and / or depth cap) -> (duplicate pairs, reads the cap dropped)"""
         nd, nc = C.c_int64(), C.c_int64()
         _check(self.ctx._h, _lib.lib().qm_sample_finish(self._h, C.byref(nd), C.byref(nc), C.c_void_p(stream)), "qm_sample_finish")
+        return nd.value, nc.value
+
+    def finish_comm(self, comm, stream=0):
+        """deferred counting of a sample sharded over the ranks of `comm` (collective: every rank calls it) -> sample-wide (duplicate
+        pairs, reads the cap dropped); this rank's count tensor then holds its survivors' counts: all-reduce them next"""
+        nd, nc = C.c_int64(), C.c_int64()
+        _check(self.ctx._h, _lib.lib().qm_sample_finish_comm(self._h, comm._h, C.byref(nd), C.byref(nc), C.c_void_p(stream)),
+               "qm_sample_finish_comm")
         return nd.value, nc.value
 
     def rmdup_finish(self, stream=0):
@@ -417,6 +455,74 @@ class Context:
         buf = C.create_string_buffer(max(1, nbytes.value))
         _check(self._h, _lib.lib().qm_mpileup_text_fetch(self._h, buf, nbytes.value), "qm_mpileup_text_fetch")
         return buf.raw[:nbytes.value]
+
+    # ---- duplicate marking and depth cap on device-resident records.  A chunk list gives one rank's records: d_alns[c] holds the
+    # records (2 per pair) of pairs pair_id0[c] .. pair_id0[c] + n - 1 (any torch tensor, n = its bytes / 256) ----
+    def mark_duplicates(self, d_alns, d_quals, d_lens, stream=0):
+        """qm_mark_duplicates over the chunks (input order, pair ids = running offsets): flags 0x400 in place -> duplicate pairs"""
+        n = [_n_pairs(a) for a in d_alns]
+        strides = (C.c_int32 * max(1, len(n)))(*[q.shape[1] for q in d_quals])
+        nd = C.c_int64()
+        rc = _lib.lib().qm_mark_duplicates(self._h, len(n), _ptrs(d_alns), _ptrs(d_quals), strides, _ptrs(d_lens),
+                                           _i64(n), C.byref(nd), C.c_void_p(stream))
+        _check(self._h, rc, "qm_mark_duplicates")
+        return nd.value
+
+    def dup_keys(self, d_alns, d_quals, d_lens, pair_id0, stream=0):
+        """one rank's duplicate tuples (qm_dup_keys) -> torch uint8 tensor [n, 32] on the device (rows of DUP_KEY_DTYPE)"""
+        import torch
+        n = [_n_pairs(a) for a in d_alns]
+        strides = (C.c_int32 * max(1, len(n)))(*[q.shape[1] for q in d_quals])
+        out = torch.empty((max(1, sum(n)), 32), dtype=torch.uint8, device=f"cuda:{self.device}")
+        n_out = C.c_int64()
+        rc = _lib.lib().qm_dup_keys(self._h, len(n), _ptrs(d_alns), _ptrs(d_quals), strides, _ptrs(d_lens), _i64(n),
+                                    _i64(pair_id0), _ptr(out), C.byref(n_out), C.c_void_p(stream))
+        _check(self._h, rc, "qm_dup_keys")
+        return out[:n_out.value]
+
+    def mark_duplicates_keys(self, d_all, d_alns, pair_id0, stream=0):
+        """decide over the union d_all (uint8 [n, 32]) and flag this rank's chunks (qm_mark_duplicates_keys) -> duplicate pairs of the union"""
+        n = [_n_pairs(a) for a in d_alns]
+        nd = C.c_int64()
+        rc = _lib.lib().qm_mark_duplicates_keys(self._h, _ptr(d_all), d_all.shape[0], len(n), _ptrs(d_alns), _i64(n),
+                                                _i64(pair_id0), C.byref(nd), C.c_void_p(stream))
+        _check(self._h, rc, "qm_mark_duplicates_keys")
+        return nd.value
+
+    def depth_cap(self, d_alns, max_depth, stream=0, popt=None):
+        """qm_depth_cap over the chunks (input order) -> ([uint8 drop mask [2n] per chunk on the device], reads dropped)"""
+        import torch
+        popt = popt or self.pileup_opt
+        n = [_n_pairs(a) for a in d_alns]
+        drops = [torch.zeros(max(1, 2 * k), dtype=torch.uint8, device=f"cuda:{self.device}") for k in n]
+        nd = C.c_int64()
+        rc = _lib.lib().qm_depth_cap(self._h, C.byref(popt), len(n), _ptrs(d_alns), _i64(n), int(max_depth), _ptrs(drops),
+                                     C.byref(nd), C.c_void_p(stream))
+        _check(self._h, rc, "qm_depth_cap")
+        return [d[:2 * k] for d, k in zip(drops, n)], nd.value
+
+    def cap_keys(self, d_alns, pair_id0, stream=0, popt=None):
+        """one rank's depth-cap tuples (qm_cap_keys) -> torch uint8 tensor [n, 16] on the device (rows of CAP_KEY_DTYPE)"""
+        import torch
+        popt = popt or self.pileup_opt
+        n = [_n_pairs(a) for a in d_alns]
+        out = torch.empty((max(1, 2 * sum(n)), 16), dtype=torch.uint8, device=f"cuda:{self.device}")
+        n_out = C.c_int64()
+        rc = _lib.lib().qm_cap_keys(self._h, C.byref(popt), len(n), _ptrs(d_alns), _i64(n), _i64(pair_id0),
+                                    _ptr(out), C.byref(n_out), C.c_void_p(stream))
+        _check(self._h, rc, "qm_cap_keys")
+        return out[:n_out.value]
+
+    def depth_cap_keys(self, d_all, max_depth, n_pairs, pair_id0, stream=0):
+        """replay over the union d_all (uint8 [n, 16]) for this rank's chunks of n_pairs[c] pairs (qm_depth_cap_keys)
+        -> ([uint8 drop mask [2 n_pairs[c]] per chunk on the device], reads dropped in the union)"""
+        import torch
+        drops = [torch.zeros(max(1, 2 * int(k)), dtype=torch.uint8, device=f"cuda:{self.device}") for k in n_pairs]
+        nd = C.c_int64()
+        rc = _lib.lib().qm_depth_cap_keys(self._h, _ptr(d_all), d_all.shape[0], int(max_depth), len(n_pairs), _i64(n_pairs),
+                                          _i64(pair_id0), _ptrs(drops), C.byref(nd), C.c_void_p(stream))
+        _check(self._h, rc, "qm_depth_cap_keys")
+        return [d[:2 * int(k)] for d, k in zip(drops, n_pairs)], nd.value
 
     def counts_to_rows(self, idx, d_planes, stream=0):
         import torch

@@ -22,8 +22,9 @@ struct qm_ctx {
     int device = -1;
     int sm_count = 0;
     std::string err;
-    // scratch arenas grown on demand (never shrunk); index = purpose
-    qm_scratch scratch[32];
+    // scratch arenas grown on demand (never shrunk); index = purpose.  32-36: the tuples of duplicate marking and the depth cap
+    // (dedup.cu, depthcap.cu, sort.cu, sample.cu)
+    qm_scratch scratch[40];
     cudaStream_t own_stream = nullptr, copy_stream = nullptr;
     // side streams: the independent per-class extension kernels of one round run concurrently (fork/join by events)
     cudaStream_t side[12] = {};

@@ -3,16 +3,20 @@
 //
 // A pair with both ends placed is keyed by {contig, unclipped 5' coordinate, strand} of both ends (ends in
 // coordinate order); among pairs with the same key the one with the highest sum of base qualities >= 15 over both
-// mates stays, ties go to the earliest pair of the input.  A read whose mate is unplaced ("fragment") is keyed by its
+// mates stays, ties go to the earliest pair of the input (the lowest pair id).  A read whose mate is unplaced ("fragment") is keyed by its
 // own {contig, unclipped 5' coordinate, strand}: it is a duplicate whenever an end of some fully placed pair has that
 // key, otherwise the best fragment of the key stays.  Pairs with no placed end are never duplicates.
-// On the device: one 64-bit key + score per pair, the stable radix sort of sort.cu, then one pass over the sorted
-// runs.  Duplicates get SAM flag 0x400, which the pileup's read admission already skips.
+// On the device: one 32-byte tuple per pair with a placed end (key, score, end codes, pair id), the stable radix sort of sort.cu,
+// then one pass over the sorted runs.  The tuples are what crosses GPUs when a sample is sharded (qm_sample_finish_comm): every
+// rank decides over the union of all ranks' tuples and flags its own records.  Duplicates get SAM flag 0x400, which the pileup's
+// read admission already skips.
+#include <vector>
 #include "pipeline.cuh"
 
 namespace {
 
 constexpr uint64_t kNoKey = ~0ull;
+constexpr uint32_t kNoEnd = 0xffffffffu;                 // end code of a missing end in qm_dup_key
 constexpr int kCoordBias = 4096;                 // unclipped coordinates can be negative (clipped bases before the contig)
 
 // {contig, unclipped 5' coordinate} of a placed record as a 30-bit code, and its strand
@@ -37,16 +41,16 @@ __device__ __forceinline__ uint32_t end_code(const qm_aln &a, int *rev, int *bad
 
 __device__ __forceinline__ bool placed(const qm_aln &a) { return !(a.flag & 0x4) && a.rid >= 0 && a.n_cigar != 0 && a.n_cigar != 255; }
 
-// key, score and (for fully placed pairs) the two end keys of every pair
+// key, score and (for fully placed pairs) the two end codes of every pair with a placed end, appended at an atomic cursor
 __global__ void __launch_bounds__(128)
 dup_keys_kernel(const qm_aln *__restrict__ alns, const uint8_t *__restrict__ quals, int stride, const int32_t *__restrict__ lens,
-                int64_t n_pairs, int64_t pair0, uint64_t *__restrict__ keys, int32_t *__restrict__ scores, uint64_t *__restrict__ ends,
-                unsigned long long *__restrict__ n_bad)
+                int64_t n_pairs, int64_t pair_id0, qm_dup_key *__restrict__ out, unsigned long long *__restrict__ cnt)
 {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n_pairs) return;
     const qm_aln a = alns[2 * i], b = alns[2 * i + 1];
     const bool pa = placed(a), pb = placed(b);
+    if (!pa && !pb) return;                             // never a duplicate, and no end of it can make one
     int sc[2] = {0, 0};
     for (int e = 0; e < 2; ++e) {
         const uint8_t *q = quals + (2 * i + e) * (int64_t)stride;
@@ -55,29 +59,46 @@ dup_keys_kernel(const qm_aln *__restrict__ alns, const uint8_t *__restrict__ qua
         for (int j = 0; j < L; ++j) { const int v = q[j]; s += v >= 15 ? v : 0; }
         sc[e] = s;
     }
-    uint64_t key = kNoKey, e0 = kNoKey, e1 = kNoKey;
-    int score = 0, bad = 0;
+    qm_dup_key t;
+    t.pair_id = pair_id0 + i;
+    t.end0 = t.end1 = kNoEnd;
+    t.pad = 0;
+    int bad = 0;
     if (pa && pb) {
         int ra, rb;
         uint32_t ca = end_code(a, &ra, &bad), cb = end_code(b, &rb, &bad);
-        if (cb < ca || (cb == ca && rb < ra)) { const uint32_t t = ca; ca = cb; cb = t; const int u = ra; ra = rb; rb = u; }
-        key = ((uint64_t)ca << 32) | ((uint64_t)cb << 2) | (uint64_t)(ra << 1 | rb);
-        e0 = (uint64_t)ca << 1 | (uint64_t)ra; e1 = (uint64_t)cb << 1 | (uint64_t)rb;
-        score = sc[0] + sc[1];
-    } else if (pa || pb) {
+        if (cb < ca || (cb == ca && rb < ra)) { const uint32_t u = ca; ca = cb; cb = u; const int v = ra; ra = rb; rb = v; }
+        t.key = ((uint64_t)ca << 32) | ((uint64_t)cb << 2) | (uint64_t)(ra << 1 | rb);
+        t.end0 = ca << 1 | (uint32_t)ra; t.end1 = cb << 1 | (uint32_t)rb;
+        t.score = sc[0] + sc[1];
+    } else {
         int r;
         const uint32_t c = end_code(pa ? a : b, &r, &bad);
-        key = (1ull << 63) | ((uint64_t)c << 1) | (uint64_t)r;
-        score = pa ? sc[0] : sc[1];
+        t.key = (1ull << 63) | ((uint64_t)c << 1) | (uint64_t)r;
+        t.score = pa ? sc[0] : sc[1];
     }
-    if (bad) atomicAdd(n_bad, 1ull);
-    keys[pair0 + i] = key;
-    scores[pair0 + i] = score;
-    ends[2 * (pair0 + i)] = e0; ends[2 * (pair0 + i) + 1] = e1;
+    if (bad) atomicAdd(cnt + 1, 1ull);
+    out[atomicAdd(cnt, 1ull)] = t;
+}
+
+// the union in pair-id order: ids[] sorted, perm[] their input positions.  Scatters key, score and end codes into sorted order and
+// raises *rep where an id repeats
+__global__ void __launch_bounds__(128)
+dup_gather_kernel(const qm_dup_key *__restrict__ all, const uint64_t *__restrict__ ids, const uint32_t *__restrict__ perm, int64_t n,
+                  uint64_t *__restrict__ keys, int32_t *__restrict__ scores, uint64_t *__restrict__ ends, unsigned long long *__restrict__ rep)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    if (i > 0 && ids[i - 1] == ids[i]) atomicAdd(rep, 1ull);
+    const qm_dup_key t = all[perm[i]];
+    keys[i] = t.key;
+    scores[i] = t.score;
+    ends[2 * i] = t.end0 == kNoEnd ? kNoKey : (uint64_t)t.end0;
+    ends[2 * i + 1] = t.end1 == kNoEnd ? kNoKey : (uint64_t)t.end1;
 }
 
 // one thread per sorted position: the head of a run of equal keys picks the run's representative (highest score, first in
-// input order on ties -- the sort is stable, so that is the first of the run) and flags the others
+// pair-id order on ties -- the sort is stable, so that is the first of the run) and flags the others
 __global__ void __launch_bounds__(128)
 dup_mark_kernel(const uint64_t *__restrict__ skeys, const uint32_t *__restrict__ perm, const int32_t *__restrict__ scores, int64_t n,
                 const uint64_t *__restrict__ sorted_ends, int64_t n_ends, uint8_t *__restrict__ dup)
@@ -103,69 +124,143 @@ dup_mark_kernel(const uint64_t *__restrict__ skeys, const uint32_t *__restrict__
 }
 
 __global__ void __launch_bounds__(128)
-dup_apply_kernel(qm_aln *__restrict__ alns, int64_t n_pairs, int64_t pair0, const uint8_t *__restrict__ dup, unsigned long long *__restrict__ n_dup)
+dup_count_kernel(const uint8_t *__restrict__ dup, int64_t n, unsigned long long *__restrict__ n_dup)
 {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i >= n_pairs || !dup[pair0 + i]) return;
+    if (i < n && dup[i]) atomicAdd(n_dup, 1ull);
+}
+
+// local pair i of a chunk finds its verdict by its id in the sorted ids of the union (absent: no placed end, never a duplicate)
+__global__ void __launch_bounds__(128)
+dup_apply_kernel(qm_aln *__restrict__ alns, int64_t n_pairs, int64_t pair_id0, const uint64_t *__restrict__ ids, int64_t n_all,
+                 const uint8_t *__restrict__ dup)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n_pairs) return;
+    const uint64_t want = (uint64_t)(pair_id0 + i);
+    int64_t lo = 0, hi = n_all;
+    while (lo < hi) { const int64_t mid = (lo + hi) >> 1; if (ids[mid] < want) lo = mid + 1; else hi = mid; }
+    if (lo == n_all || ids[lo] != want || !dup[lo]) return;
     for (int e = 0; e < 2; ++e)
         if (!(alns[2 * i + e].flag & 0x4)) alns[2 * i + e].flag |= 0x400;      // an unplaced mate is never a duplicate
-    atomicAdd(n_dup, 1ull);
+}
+
+__global__ void __launch_bounds__(256)
+dup_ids_kernel(const qm_dup_key *__restrict__ all, int64_t n, uint64_t *__restrict__ ids)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i < n) ids[i] = (uint64_t)all[i].pair_id;
 }
 
 }  // namespace
 
 extern "C" {
 
-// chunks: the sample's records in input order, chunk c = pairs [pair0[c], pair0[c] + n[c]).  Synchronous.
-int qm_mark_duplicates(qm_ctx *ctx, int n_chunks, qm_aln *const *d_alns, const uint8_t *const *d_quals, const int32_t *strides,
-                       const int32_t *const *d_lens, const int64_t *n_pairs, int64_t *h_n_dup, void *stream)
+// one qm_dup_key per pair with a placed end, chunk c = pairs pair_id0[c] .. pair_id0[c] + n_pairs[c] - 1.  Synchronous.
+int qm_dup_keys(qm_ctx *ctx, int n_chunks, const qm_aln *const *d_alns, const uint8_t *const *d_quals, const int32_t *strides,
+                const int32_t *const *d_lens, const int64_t *n_pairs, const int64_t *pair_id0, qm_dup_key *d_out, int64_t *h_n_out,
+                void *stream)
 {
-    if (!ctx || n_chunks < 0 || (n_chunks > 0 && (!d_alns || !d_quals || !strides || !d_lens || !n_pairs))) return QM_EINVAL;
+    if (!ctx || !h_n_out || n_chunks < 0 || (n_chunks > 0 && (!d_alns || !d_quals || !strides || !d_lens || !n_pairs || !pair_id0)))
+        return QM_EINVAL;
+    *h_n_out = 0;
+    int64_t N = 0;
+    for (int c = 0; c < n_chunks; ++c) { if (n_pairs[c] < 0 || pair_id0[c] < 0) return QM_EINVAL; N += n_pairs[c]; }
+    if (N == 0) return QM_OK;
+    if (!d_out) return QM_EINVAL;
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    int64_t N = 0;
-    for (int c = 0; c < n_chunks; ++c) { if (n_pairs[c] < 0) return QM_EINVAL; N += n_pairs[c]; }
-    if (h_n_dup) *h_n_dup = 0;
-    if (N == 0) return QM_OK;
-    if (2 * N > 0xffffffffll) return qm_fail(ctx, QM_ELIMIT, "qm_mark_duplicates: more than 2^31 pairs");
-    // scratch 15: keys | ends | scores | perm | end perm | dup flags | counter
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t o_keys = 0, o_ends = o_keys + al((size_t)N * 8), o_sc = o_ends + al((size_t)2 * N * 8), o_perm = o_sc + al((size_t)N * 4);
-    const size_t o_eperm = o_perm + al((size_t)N * 4), o_dup = o_eperm + al((size_t)2 * N * 4), o_cnt = o_dup + al((size_t)N);
     void *p = nullptr;
-    int rc = qm_scratch_reserve(ctx, 15, o_cnt + 256, &p);
+    int rc = qm_scratch_reserve(ctx, 33, 256, &p);
     if (rc) return rc;
-    char *b = (char *)p;
-    uint64_t *keys = (uint64_t *)(b + o_keys), *ends = (uint64_t *)(b + o_ends);
-    int32_t *scores = (int32_t *)(b + o_sc);
-    uint32_t *perm = (uint32_t *)(b + o_perm), *eperm = (uint32_t *)(b + o_eperm);
-    uint8_t *dup = (uint8_t *)(b + o_dup);
-    unsigned long long *cnt = (unsigned long long *)(b + o_cnt);
-    QM_CUDA(ctx, cudaMemsetAsync(dup, 0, (size_t)N, st));
-    QM_CUDA(ctx, cudaMemsetAsync(cnt, 0, 16, st));             // cnt[0] = duplicates, cnt[1] = pairs whose end code does not fit
-    int64_t p0 = 0;
-    for (int c = 0; c < n_chunks; ++c) {
-        if (n_pairs[c]) dup_keys_kernel<<<(unsigned)((n_pairs[c] + 127) / 128), 128, 0, st>>>(d_alns[c], d_quals[c], strides[c], d_lens[c], n_pairs[c], p0,
-                                                                                        keys, scores, ends, cnt + 1);
-        p0 += n_pairs[c];
-    }
-    rc = qm_sort_pairs(ctx, keys, perm, N, 64, st);
-    if (rc) return rc;
-    rc = qm_sort_pairs(ctx, ends, eperm, 2 * N, 32, st);          // end keys are 31 bits; kNoKey's low word is all ones: sorts last
-    if (rc) return rc;
-    dup_mark_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(keys, perm, scores, N, ends, 2 * N, dup);
-    p0 = 0;
-    for (int c = 0; c < n_chunks; ++c) {
-        if (n_pairs[c]) dup_apply_kernel<<<(unsigned)((n_pairs[c] + 127) / 128), 128, 0, st>>>(d_alns[c], n_pairs[c], p0, dup, cnt);
-        p0 += n_pairs[c];
-    }
+    unsigned long long *cnt = (unsigned long long *)p;           // cnt[0] = tuples written, cnt[1] = pairs whose end code does not fit
+    QM_CUDA(ctx, cudaMemsetAsync(cnt, 0, 16, st));
+    for (int c = 0; c < n_chunks; ++c)
+        if (n_pairs[c]) dup_keys_kernel<<<(unsigned)((n_pairs[c] + 127) / 128), 128, 0, st>>>(d_alns[c], d_quals[c], strides[c], d_lens[c],
+                                                                                        n_pairs[c], pair_id0[c], d_out, cnt);
     QM_CUDA(ctx, cudaGetLastError());
     unsigned long long h[2] = {0, 0};
     QM_CUDA(ctx, cudaMemcpyAsync(h, cnt, 16, cudaMemcpyDeviceToHost, st));
     QM_CUDA(ctx, cudaStreamSynchronize(st));
     if (h[1]) return qm_fail(ctx, QM_ELIMIT, "qm_mark_duplicates: %llu pairs lie beyond what the 30-bit end code holds (contigs of up to 2^26 - 4096 bases, 16 contigs)", h[1]);
-    if (h_n_dup) *h_n_dup = (int64_t)h[0];
+    *h_n_out = (int64_t)h[0];
     return QM_OK;
+}
+
+// the decision over the union of every rank's tuples, applied to this rank's chunks.  Synchronous.
+int qm_mark_duplicates_keys(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all, int n_chunks, qm_aln *const *d_alns,
+                            const int64_t *n_pairs, const int64_t *pair_id0, int64_t *h_n_dup_all, void *stream)
+{
+    if (!ctx || n_all < 0 || (n_all > 0 && !d_all) || n_chunks < 0 || (n_chunks > 0 && (!d_alns || !n_pairs || !pair_id0))) return QM_EINVAL;
+    for (int c = 0; c < n_chunks; ++c) if (n_pairs[c] < 0 || pair_id0[c] < 0) return QM_EINVAL;
+    if (h_n_dup_all) *h_n_dup_all = 0;
+    if (n_all == 0) return QM_OK;
+    if (2 * n_all > 0xffffffffll) return qm_fail(ctx, QM_ELIMIT, "qm_mark_duplicates: more than 2^31 pairs");
+    QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t N = n_all;
+    // scratch 15: ids | id perm | keys | ends | scores | perm | end perm | dup flags | counters
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t o_ids = 0, o_iperm = o_ids + al((size_t)N * 8), o_keys = o_iperm + al((size_t)N * 4), o_ends = o_keys + al((size_t)N * 8);
+    const size_t o_sc = o_ends + al((size_t)2 * N * 8), o_perm = o_sc + al((size_t)N * 4), o_eperm = o_perm + al((size_t)N * 4);
+    const size_t o_dup = o_eperm + al((size_t)2 * N * 4), o_cnt = o_dup + al((size_t)N);
+    void *p = nullptr;
+    int rc = qm_scratch_reserve(ctx, 15, o_cnt + 256, &p);
+    if (rc) return rc;
+    char *b = (char *)p;
+    uint64_t *ids = (uint64_t *)(b + o_ids), *keys = (uint64_t *)(b + o_keys), *ends = (uint64_t *)(b + o_ends);
+    int32_t *scores = (int32_t *)(b + o_sc);
+    uint32_t *iperm = (uint32_t *)(b + o_iperm), *perm = (uint32_t *)(b + o_perm), *eperm = (uint32_t *)(b + o_eperm);
+    uint8_t *dup = (uint8_t *)(b + o_dup);
+    unsigned long long *cnt = (unsigned long long *)(b + o_cnt);
+    QM_CUDA(ctx, cudaMemsetAsync(dup, 0, (size_t)N, st));
+    QM_CUDA(ctx, cudaMemsetAsync(cnt, 0, 16, st));             // cnt[0] = duplicates, cnt[1] = repeated ids
+    // the union in pair-id order: the same input on every rank, whatever order the all-gather delivered it in
+    dup_ids_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(d_all, N, ids);
+    rc = qm_sort_ids(ctx, ids, iperm, N, "qm_mark_duplicates_keys", st);
+    if (rc) return rc;
+    dup_gather_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(d_all, ids, iperm, N, keys, scores, ends, cnt + 1);
+    QM_CUDA(ctx, cudaGetLastError());
+    unsigned long long h[2] = {0, 0};
+    QM_CUDA(ctx, cudaMemcpyAsync(h + 1, cnt + 1, 8, cudaMemcpyDeviceToHost, st));
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    if (h[1]) return qm_fail(ctx, QM_EINVAL, "qm_mark_duplicates_keys: %llu pair ids occur more than once in the union", h[1]);
+    rc = qm_sort_pairs(ctx, keys, perm, N, 64, st);
+    if (rc) return rc;
+    rc = qm_sort_pairs(ctx, ends, eperm, 2 * N, 32, st);          // end keys are 31 bits; kNoKey's low word is all ones: sorts last
+    if (rc) return rc;
+    dup_mark_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(keys, perm, scores, N, ends, 2 * N, dup);
+    dup_count_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(dup, N, cnt);
+    for (int c = 0; c < n_chunks; ++c)
+        if (n_pairs[c]) dup_apply_kernel<<<(unsigned)((n_pairs[c] + 127) / 128), 128, 0, st>>>(d_alns[c], n_pairs[c], pair_id0[c], ids, N, dup);
+    QM_CUDA(ctx, cudaGetLastError());
+    QM_CUDA(ctx, cudaMemcpyAsync(h, cnt, 8, cudaMemcpyDeviceToHost, st));
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    if (h_n_dup_all) *h_n_dup_all = (int64_t)h[0];
+    return QM_OK;
+}
+
+// chunks: the sample's records in input order, chunk c = pairs [pair0[c], pair0[c] + n[c]): the export and the decision above on one
+// device, pair ids = running pair offsets.  Synchronous.
+int qm_mark_duplicates(qm_ctx *ctx, int n_chunks, qm_aln *const *d_alns, const uint8_t *const *d_quals, const int32_t *strides,
+                       const int32_t *const *d_lens, const int64_t *n_pairs, int64_t *h_n_dup, void *stream)
+{
+    if (!ctx || n_chunks < 0 || (n_chunks > 0 && (!d_alns || !d_quals || !strides || !d_lens || !n_pairs))) return QM_EINVAL;
+    int64_t N = 0;
+    std::vector<int64_t> id0((size_t)n_chunks);
+    for (int c = 0; c < n_chunks; ++c) { if (n_pairs[c] < 0) return QM_EINVAL; id0[(size_t)c] = N; N += n_pairs[c]; }
+    if (h_n_dup) *h_n_dup = 0;
+    if (N == 0) return QM_OK;
+    if (2 * N > 0xffffffffll) return qm_fail(ctx, QM_ELIMIT, "qm_mark_duplicates: more than 2^31 pairs");
+    QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    void *p = nullptr;
+    int rc = qm_scratch_reserve(ctx, 32, (size_t)N * sizeof(qm_dup_key), &p);
+    if (rc) return rc;
+    qm_dup_key *tuples = (qm_dup_key *)p;
+    int64_t n_t = 0;
+    rc = qm_dup_keys(ctx, n_chunks, d_alns, d_quals, strides, d_lens, n_pairs, id0.data(), tuples, &n_t, stream);
+    if (rc) return rc;
+    return qm_mark_duplicates_keys(ctx, tuples, n_t, n_chunks, d_alns, n_pairs, id0.data(), h_n_dup, stream);
 }
 
 }  // extern "C"

@@ -17,7 +17,9 @@
 //        --no-rescue 1 = bwa mem -S (mate rescue off; on by default as in the reference's command line)
 //        --rmdup: duplicates are marked on the device with picard MarkDuplicates' rule (rules/rmdup.smk:13-16) before
 //        anything is counted, as in the reference where every caller reads the .rmdup.bam; --bam still holds all records
-//        (duplicates flagged 0x400), --rmdup-bam is the REMOVE_DUPLICATES=true file
+//        (duplicates flagged 0x400), --rmdup-bam is the REMOVE_DUPLICATES=true file.  With --gpus the reads and records stay on
+//        their GPUs: duplicates and the --max-depth cap are decided over small per-pair / per-read tuples all-gathered over NCCL,
+//        so every output is the one-GPU output
 //        = rules/bwa.smk:15-18 (bwa mem | samtools view | samtools sort | samtools index -> BAM + BAI),
 //          rules/vcfcall.smk:39 (pileup path: count TSV, SURVEY.md B.3) and rules/vcfcall.smk:115-117 (VCF)
 //   qm_driver decontam --ref CONTAMINANT.fa[,MORE.fa] --r1 .. --r2 .. --out-r1 CLEAN1.fq --out-r2 CLEAN2.fq
@@ -737,6 +739,22 @@ std::string trim_float3(double x)
     return s;
 }
 
+// --gpus: batches are dealt round-robin, batch i to GPU i % n_gpu; a GPU keeps the records of its batches in the order it got them
+int batch_gpu(int64_t batch, int n_gpu) { return (int)(batch % n_gpu); }
+
+// where each batch's records lie among those its GPU kept (qm_sample_kept_alns_host): {GPU, first record} per batch
+std::vector<std::pair<int, int64_t>> batch_sources(const std::vector<int64_t> &batch_pairs, int n_gpu)
+{
+    std::vector<std::pair<int, int64_t>> src(batch_pairs.size());
+    std::vector<int64_t> next((size_t)n_gpu, 0);
+    for (size_t i = 0; i < batch_pairs.size(); ++i) {
+        const int d = batch_gpu((int64_t)i, n_gpu);
+        src[i] = {d, next[(size_t)d]};
+        next[(size_t)d] += 2 * batch_pairs[i];
+    }
+    return src;
+}
+
 // An indel allele that passes the caller's thresholds (same rule as the SNPs: raw depth at the anchor >= min_dp, supporting
 // reads >= min_alt and >= min_af x depth), as the VCF shows it: anchor base first, POS = anchor (the convention of
 // program/mummer2vcf.py for the truth set and of bcftools).
@@ -1143,13 +1161,12 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     const bool rmdup = !decontam && atoi(a.get("rmdup", "0").c_str()) != 0;
     const std::string rmdup_bam = a.get("rmdup-bam"), metrics = a.get("metrics");
     if (!rmdup && (!rmdup_bam.empty() || !metrics.empty())) die(1, "--rmdup-bam / --metrics need --rmdup 1");
-    if (rmdup && n_gpu > 1) die(1, "--rmdup 1 needs the records of the whole sample on one device: run it with one GPU");
-    if (rmdup) L.check(qm_sample_set_rmdup(smp, 1), "qm_sample_set_rmdup");
+    if (rmdup) for (int d = 0; d < n_gpu; ++d) Ls[d].check(qm_sample_set_rmdup(smps[d], 1), "qm_sample_set_rmdup");
     // --max-depth N: bcftools mpileup -d N (htslib's order-dependent depth cap); 0 / absent = no cap (DESIGN.md 5)
     const int max_depth = atoi(a.get("max-depth", "0").c_str());
     if (max_depth < 0) die(1, "--max-depth must be >= 0");
-    if (max_depth > 0 && n_gpu > 1) die(1, "--max-depth needs the records of the whole sample on one device: run it with one GPU");
-    if (max_depth > 0) L.check(qm_sample_set_max_depth(smp, max_depth), "qm_sample_set_max_depth");
+    if (max_depth > 0) for (int d = 0; d < n_gpu; ++d) Ls[d].check(qm_sample_set_max_depth(smps[d], max_depth), "qm_sample_set_max_depth");
+    const bool deferred = rmdup || max_depth > 0;      // counting waits for the whole sample (qm_sample_finish / _finish_comm)
     // --baq 1: base alignment quality on, as both mpileups of the reference flow run (no -B at rules/vcfcall.smk:39,115): extended BAQ
     // caps the base qualities the counts, the calls and the text pileup see.  Off by default (the parity configuration is -B).
     const int baq = atoi(a.get("baq", "0").c_str()) ? 3 : 0;
@@ -1179,7 +1196,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     int64_t n_batches = 0;
     const auto t_loop = std::chrono::steady_clock::now();
     while (read_batch(fr, batch_pairs, raw)) {
-        const int d = (int)(n_batches % n_gpu);
+        const int d = batch_gpu(n_batches, n_gpu);
         join_worker(d);
         batches.emplace_back();
         Batch &b = batches.back();
@@ -1254,37 +1271,44 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             fprintf(stderr, "[qm_driver] GPU %d stages (ms of device time): %s; total %.1f in %lld launches\n", devs[d], line.c_str(), tot, (long long)nl);
         }
     }
+    int64_t n_dup = 0, n_capped = 0;
     if (n_gpu > 1) {
-        // per-GPU int32 count tensors -> one NCCL all-reduce over NVLink; every GPU ends up with the sample's totals
+        // per-GPU int32 count tensors -> one NCCL all-reduce over NVLink; every GPU ends up with the sample's totals.  Deferred
+        // counting first: every GPU marks duplicates and applies the cap over the tuples of the whole sample, counts its survivors
         std::vector<qm_ctx *> ctxs;
         for (auto &x : Ls) ctxs.push_back(x.ctx);
         std::vector<qm_comm *> comms((size_t)n_gpu, nullptr);
         L.check(qm_comm_init_all(n_gpu, ctxs.data(), comms.data()), "qm_comm_init_all");
         std::vector<std::thread> team;
+        std::vector<int64_t> nd((size_t)n_gpu, 0), ncap((size_t)n_gpu, 0);
         for (int d = 0; d < n_gpu; ++d)
             team.emplace_back([&, d]() {
+                if (deferred) Ls[d].check(qm_sample_finish_comm(smps[d], comms[d], &nd[(size_t)d], &ncap[(size_t)d], nullptr), "qm_sample_finish_comm");
                 Ls[d].check(qm_counts_allreduce(Ls[d].ctx, comms[d], qm_sample_counts(smps[d]), (int64_t)QM_NCH * (int64_t)g.codes.size(), nullptr),
                             "qm_counts_allreduce");
                 Ls[d].check(qm_sample_stats_sync(smps[d], nullptr, nullptr, nullptr), "qm_sample_stats_sync");
             });
         for (auto &t : team) t.join();
         for (auto c : comms) qm_comm_destroy(c);
+        n_dup = nd[0]; n_capped = ncap[0];                 // sample-wide, the same on every GPU
         fprintf(stderr, "[qm_driver] count tensors of %d GPUs merged (ncclAllReduce, int32 sum, %lld values)\n", n_gpu,
                 (long long)QM_NCH * (long long)g.codes.size());
-    }
-    int64_t n_dup = 0;
-    if (rmdup || max_depth > 0) {
-        int64_t n_capped = 0;
-        L.check(qm_sample_finish(smp, &n_dup, &n_capped, nullptr), "qm_sample_finish");
+    } else if (deferred) L.check(qm_sample_finish(smp, &n_dup, &n_capped, nullptr), "qm_sample_finish");
+    if (deferred) {
         if (rmdup) fprintf(stderr, "[qm_driver] rmdup: %lld of %lld pairs are duplicates\n", (long long)n_dup, (long long)n_pairs);
         if (max_depth > 0) fprintf(stderr, "[qm_driver] depth cap %d: %lld reads dropped by the pileup iterator\n", max_depth, (long long)n_capped);
     }
     if (rmdup) {
-        if (want_batches) {                            // final flags of every record, batch by batch
-            std::vector<qm_aln> all((size_t)2 * n_pairs);
-            L.check(qm_sample_kept_alns_host(smp, all.data(), (int64_t)all.size()), "qm_sample_kept_alns_host");
-            size_t off = 0;
-            for (auto &b : batches) { memcpy(b.alns, all.data() + off, (size_t)2 * b.n_pairs * sizeof(qm_aln)); off += (size_t)2 * b.n_pairs; }
+        if (want_batches) {                            // final flags of every record, batch by batch, from the GPU that held the batch
+            std::vector<int64_t> bp;
+            for (auto &b : batches) bp.push_back(b.n_pairs);
+            const auto src = batch_sources(bp, n_gpu);
+            std::vector<std::vector<qm_aln>> all((size_t)n_gpu);
+            for (size_t i = 0; i < bp.size(); ++i) all[(size_t)src[i].first].resize((size_t)(src[i].second + 2 * bp[i]));
+            for (int d = 0; d < n_gpu; ++d)
+                Ls[d].check(qm_sample_kept_alns_host(smps[d], all[(size_t)d].data(), (int64_t)all[(size_t)d].size()), "qm_sample_kept_alns_host");
+            for (size_t i = 0; i < bp.size(); ++i)
+                memcpy(batches[i].alns, all[(size_t)src[i].first].data() + src[i].second, (size_t)2 * bp[i] * sizeof(qm_aln));
         }
         if (!metrics.empty()) {
             FILE *fm = fopen(metrics.c_str(), "w");
@@ -1579,6 +1603,13 @@ int main(int argc, char **argv)
         for (size_t i = 0; ok && i < 5; ++i) ok = (int64_t)M[i].key == want[i][0] && M[i].n_fwd == want[i][1] && M[i].n_rev == want[i][2];
         ok = ok && merge_indel_tables(A, nullptr, 0).size() == 3 && merge_indel_tables({}, B.data(), 4).size() == 4 && merge_indel_tables({}, nullptr, 0).empty();
         if (!ok) die(2, "selftest: merge_indel_tables is wrong");
+        // batch -> (GPU, first record among that GPU's kept records) for batches of 3, 5, 2, 7, 4 pairs
+        const std::vector<int64_t> bp = {3, 5, 2, 7, 4};
+        const std::vector<std::pair<int, int64_t>> w1 = {{0, 0}, {0, 6}, {0, 16}, {0, 20}, {0, 34}}, w2 = {{0, 0}, {1, 0}, {0, 6}, {1, 10}, {0, 10}},
+                                                   w3 = {{0, 0}, {1, 0}, {2, 0}, {0, 6}, {1, 10}}, w8 = {{0, 0}, {1, 0}, {2, 0}, {3, 0}, {4, 0}};
+        ok = batch_sources(bp, 1) == w1 && batch_sources(bp, 2) == w2 && batch_sources(bp, 3) == w3 && batch_sources(bp, 8) == w8 &&
+             batch_sources({}, 2).empty();
+        if (!ok) die(2, "selftest: batch_sources is wrong");
         printf("selftest ok\n");
         return 0;
     }

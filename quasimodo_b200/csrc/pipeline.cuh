@@ -192,6 +192,10 @@ int qm_ext_launch_classes(qm_ctx *ctx, const ExtParams &P, const IndexView &V, c
                           const int *h_counts, qm_ext_result *d_out, int *d_fb_lists, int *d_fb_ctr, cudaStream_t st,
                           bool scores_fit_bytes = false, const int64_t *h_list_off = nullptr);
 
+// internal (sort.cu): the ids of a union of exported tuples sorted stably over the bits in use, d_perm = input positions;
+// QM_EINVAL on a negative id.  Synchronous.
+int qm_sort_ids(qm_ctx *ctx, uint64_t *d_ids, uint32_t *d_perm, int64_t n, const char *who, cudaStream_t st);
+
 // internal: qm_pileup_accumulate_indels with a per-read drop mask (depth cap)
 struct qm_indel_table;
 extern "C" int qm_pileup_accumulate_masked(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns,

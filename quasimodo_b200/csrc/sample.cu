@@ -46,7 +46,7 @@ struct qm_sample {
     int max_depth = 0;                            // > 0: `bcftools mpileup -d` depth cap (qm_sample_set_max_depth): deferred counting too
     int baq = 0;                                  // 1 / 3: base alignment quality (plain / extended) caps the qualities the pileup sees (qm_sample_set_baq)
     bool rmdup_finished = false;                  // qm_sample_rmdup_finish has run: no more pairs, no second finish until a reset
-    struct Kept { uint8_t *codes, *quals; int32_t *lens; qm_aln *alns; int64_t n; int32_t stride; };
+    struct Kept { uint8_t *codes, *quals; int32_t *lens; qm_aln *alns; int64_t n; int32_t stride; int64_t pair0; };   // pair0: id of the first pair
     std::vector<Kept> kept;
 };
 
@@ -132,7 +132,7 @@ int sample_chunk(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_quals, i
     if (rc) return rc;
     if (s->rmdup || s->max_depth > 0) {
         // keep the chunk for qm_sample_rmdup_finish: duplicates are a property of the whole sample
-        qm_sample::Kept k = {nullptr, nullptr, nullptr, nullptr, n, stride};
+        qm_sample::Kept k = {nullptr, nullptr, nullptr, nullptr, n, stride, pair_id0};
         const size_t sb = (size_t)2 * n * stride;
         cudaError_t e;
         if ((e = cudaMalloc(&k.codes, sb)) != cudaSuccess || (e = cudaMalloc(&k.quals, sb)) != cudaSuccess ||
@@ -260,6 +260,24 @@ int qm_sample_set_baq(qm_sample *s, int flag)
     return QM_OK;
 }
 
+// the last step of a deferred sample: count what survived duplicate marking (0x400) and the cap (drop[c], may be NULL), then release
+// the kept reads; the records stay for qm_sample_kept_alns_host
+static int count_survivors(qm_sample *s, const std::vector<uint8_t *> &drop, void *stream)
+{
+    qm_ctx *ctx = s->ctx;
+    for (size_t c = 0; c < s->kept.size(); ++c) {
+        const auto &k = s->kept[c];
+        const uint8_t *pq = nullptr;
+        int rc = sample_pileup_quals(s, k.alns, k.codes, k.quals, k.stride, k.lens, 2 * k.n, (cudaStream_t)stream, &pq);
+        if (!rc) rc = qm_pileup_accumulate_masked(ctx, s->idx, &s->popt, k.alns, k.codes, pq, k.stride, k.lens, k.n, s->d_counts, s->indels, drop[c], stream);
+        if (rc) return rc;
+    }
+    QM_CUDA(ctx, cudaStreamSynchronize((cudaStream_t)stream));
+    for (auto &k : s->kept) { cudaFree(k.codes); cudaFree(k.quals); cudaFree(k.lens); k.codes = k.quals = nullptr; k.lens = nullptr; }
+    s->rmdup_finished = true;
+    return QM_OK;
+}
+
 // Deferred counting: marks the duplicates among everything added since the last reset (rmdup mode), replays htslib's depth
 // cap over the records that are left (max_depth mode), then counts what survives both.
 int qm_sample_finish(qm_sample *s, int64_t *n_dup_pairs, int64_t *n_capped_reads, void *stream)
@@ -290,18 +308,9 @@ int qm_sample_finish(qm_sample *s, int64_t *n_dup_pairs, int64_t *n_capped_reads
         rc = qm_depth_cap(ctx, &s->popt, nc, a.data(), n.data(), s->max_depth, drop.data(), n_capped_reads, stream);
         if (rc) { for (auto d : drop) cudaFree(d); return rc; }
     }
-    for (int c = 0; c < nc; ++c) {
-        const auto &k = s->kept[c];
-        const uint8_t *pq = nullptr;
-        rc = sample_pileup_quals(s, k.alns, k.codes, k.quals, k.stride, k.lens, 2 * k.n, (cudaStream_t)stream, &pq);
-        if (!rc) rc = qm_pileup_accumulate_masked(ctx, s->idx, &s->popt, k.alns, k.codes, pq, k.stride, k.lens, k.n, s->d_counts, s->indels, drop[c], stream);
-        if (rc) { for (auto d : drop) cudaFree(d); return rc; }
-    }
-    QM_CUDA(ctx, cudaStreamSynchronize((cudaStream_t)stream));
+    rc = count_survivors(s, drop, stream);
     for (auto d : drop) cudaFree(d);
-    for (auto &k : s->kept) { cudaFree(k.codes); cudaFree(k.quals); cudaFree(k.lens); k.codes = k.quals = nullptr; k.lens = nullptr; }
-    s->rmdup_finished = true;
-    return QM_OK;
+    return rc;
 }
 
 // marks the duplicates among everything added since the last reset (flag 0x400 on their records), then counts the rest
@@ -385,6 +394,95 @@ int qm_sample_allreduce_counts(qm_sample *s, void *stream)
         }
     QM_CUDA(ctx, cudaStreamSynchronize(st));
     return QM_OK;
+}
+
+// every rank's n_mine tuples of `rec` bytes at d_mine -> the union of all ranks' tuples (*d_union, *n_union; rank order, no padding).
+// The counts cross first (8 bytes per rank), then the tuples padded to the largest count.  Collective, synchronous.
+static int allgather_tuples(qm_ctx *ctx, qm_comm *comm, const void *d_mine, int64_t n_mine, size_t rec, void **d_union, int64_t *n_union,
+                            cudaStream_t st)
+{
+    const int size = qm_comm_size(comm);
+    void *p = nullptr;
+    int rc = qm_scratch_reserve(ctx, 34, 256 + (size_t)size * 8, &p);                 // scratch 34: my count | every rank's count
+    if (rc) return rc;
+    int64_t *d_n = (int64_t *)p, *d_all_n = (int64_t *)((char *)p + 256);
+    QM_CUDA(ctx, cudaMemcpyAsync(d_n, &n_mine, 8, cudaMemcpyHostToDevice, st));
+    rc = qm_comm_allgather(ctx, comm, d_n, d_all_n, 8, st);
+    if (rc) return rc;
+    std::vector<int64_t> all_n((size_t)size);
+    QM_CUDA(ctx, cudaMemcpyAsync(all_n.data(), d_all_n, (size_t)size * 8, cudaMemcpyDeviceToHost, st));
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    int64_t mx = 0, tot = 0;
+    for (int64_t v : all_n) { mx = v > mx ? v : mx; tot += v; }
+    *d_union = nullptr; *n_union = tot;
+    if (mx == 0) return QM_OK;
+    // both buffers before the all-gather: growing one frees device memory, which is not done while a collective is in flight
+    void *u = nullptr;
+    rc = qm_scratch_reserve(ctx, 35, (size_t)(size + 1) * mx * rec, &p);             // scratch 35: send (mx records) | receive (size x mx)
+    if (!rc) rc = qm_scratch_reserve(ctx, 36, (size_t)tot * rec, &u);                 // scratch 36: the union, padding dropped
+    if (rc) return rc;
+    char *send = (char *)p, *recv = send + (size_t)mx * rec;
+    if (n_mine) QM_CUDA(ctx, cudaMemcpyAsync(send, d_mine, (size_t)n_mine * rec, cudaMemcpyDeviceToDevice, st));
+    if (n_mine < mx) QM_CUDA(ctx, cudaMemsetAsync(send + (size_t)n_mine * rec, 0, (size_t)(mx - n_mine) * rec, st));
+    rc = qm_comm_allgather(ctx, comm, send, recv, (size_t)mx * rec, st);
+    if (rc) return rc;
+    size_t off = 0;
+    for (int r = 0; r < size; ++r) {
+        if (all_n[(size_t)r]) QM_CUDA(ctx, cudaMemcpyAsync((char *)u + off, recv + (size_t)r * mx * rec, (size_t)all_n[(size_t)r] * rec,
+                                                           cudaMemcpyDeviceToDevice, st));
+        off += (size_t)all_n[(size_t)r] * rec;
+    }
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    *d_union = u;
+    return QM_OK;
+}
+
+// Deferred counting of a sample sharded over the ranks of `comm`: duplicates and the cap decided over the union of every rank's
+// tuples, this rank's survivors counted (the caller all-reduces the counts next).  Collective.
+int qm_sample_finish_comm(qm_sample *s, qm_comm *comm, int64_t *n_dup_pairs, int64_t *n_capped_reads, void *stream)
+{
+    if (!s || !comm) return QM_EINVAL;
+    qm_ctx *ctx = s->ctx;
+    if (!s->rmdup && s->max_depth <= 0) return qm_fail(ctx, QM_EINVAL, "qm_sample_finish_comm: the sample counts as it goes (neither rmdup nor a depth cap is set)");
+    if (s->rmdup_finished) return qm_fail(ctx, QM_EINVAL, "qm_sample_finish_comm: already finished; reset the sample first");
+    QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    QM_CUDA(ctx, cudaDeviceSynchronize());                 // chunks may have been added on any stream
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nc = (int)s->kept.size();
+    std::vector<qm_aln *> a(nc);
+    std::vector<const uint8_t *> q(nc);
+    std::vector<const int32_t *> l(nc);
+    std::vector<int32_t> sd(nc);
+    std::vector<int64_t> n(nc), id0(nc);
+    int64_t N = 0;
+    for (int c = 0; c < nc; ++c) {
+        const auto &k = s->kept[c];
+        a[c] = k.alns; q[c] = k.quals; l[c] = k.lens; sd[c] = k.stride; n[c] = k.n; id0[c] = k.pair0;
+        N += k.n;
+    }
+    if (n_dup_pairs) *n_dup_pairs = 0;
+    if (n_capped_reads) *n_capped_reads = 0;
+    void *p = nullptr, *all = nullptr;
+    int64_t n_mine = 0, n_all = 0;
+    int rc = qm_scratch_reserve(ctx, 32, (size_t)(N > 0 ? N : 1) * 32, &p);          // scratch 32: this rank's tuples (32 bytes per pair either way)
+    if (rc) return rc;
+    if (s->rmdup) {
+        rc = qm_dup_keys(ctx, nc, a.data(), q.data(), sd.data(), l.data(), n.data(), id0.data(), (qm_dup_key *)p, &n_mine, stream);
+        if (!rc) rc = allgather_tuples(ctx, comm, p, n_mine, sizeof(qm_dup_key), &all, &n_all, st);
+        if (!rc) rc = qm_mark_duplicates_keys(ctx, (const qm_dup_key *)all, n_all, nc, a.data(), n.data(), id0.data(), n_dup_pairs, stream);
+        if (rc) return rc;
+    }
+    std::vector<uint8_t *> drop((size_t)nc, nullptr);
+    if (s->max_depth > 0) {
+        for (int c = 0; c < nc; ++c) if (n[c]) QM_CUDA(ctx, cudaMalloc(&drop[c], (size_t)2 * n[c]));
+        rc = qm_cap_keys(ctx, &s->popt, nc, a.data(), n.data(), id0.data(), (qm_cap_key *)p, &n_mine, stream);
+        if (!rc) rc = allgather_tuples(ctx, comm, p, n_mine, sizeof(qm_cap_key), &all, &n_all, st);
+        if (!rc) rc = qm_depth_cap_keys(ctx, (const qm_cap_key *)all, n_all, s->max_depth, nc, n.data(), id0.data(), drop.data(), n_capped_reads, stream);
+        if (rc) { for (auto d : drop) cudaFree(d); return rc; }
+    }
+    rc = count_survivors(s, drop, stream);
+    for (auto d : drop) cudaFree(d);
+    return rc;
 }
 
 qm_indel_table *qm_sample_indel_table(qm_sample *s) { return s ? s->indels : nullptr; }

@@ -130,7 +130,36 @@ radix_scatter_kernel(const uint64_t *__restrict__ keys_in, const uint32_t *__res
     }
 }
 
+__global__ void __launch_bounds__(256)
+max_key_kernel(const uint64_t *__restrict__ keys, int64_t n, unsigned long long *__restrict__ mx)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    unsigned long long v = i < n ? keys[i] : 0ull;
+    for (int o = 16; o > 0; o >>= 1) { const unsigned long long u = __shfl_xor_sync(0xffffffffu, v, o); v = u > v ? u : v; }
+    if ((threadIdx.x & 31) == 0 && v) atomicMax(mx, v);
+}
+
 }  // namespace
+
+// The ids of a union of exported tuples (dedup.cu, depthcap.cu), stably sorted over just the bits the largest id needs; d_perm[i] =
+// input position of the id at sorted position i.  Ids are int64 values cast to uint64: a negative one is QM_EINVAL.  Synchronous.
+int qm_sort_ids(qm_ctx *ctx, uint64_t *d_ids, uint32_t *d_perm, int64_t n, const char *who, cudaStream_t st)
+{
+    if (n == 0) return QM_OK;
+    void *p = nullptr;
+    int rc = qm_scratch_reserve(ctx, 33, 256, &p);
+    if (rc) return rc;
+    unsigned long long *mx = (unsigned long long *)p, h = 0;
+    QM_CUDA(ctx, cudaMemsetAsync(mx, 0, 8, st));
+    max_key_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_ids, n, mx);
+    QM_CUDA(ctx, cudaGetLastError());
+    QM_CUDA(ctx, cudaMemcpyAsync(&h, mx, 8, cudaMemcpyDeviceToHost, st));
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    if (h >> 63) return qm_fail(ctx, QM_EINVAL, "%s: negative id in the union", who);
+    int bits = 1;
+    while (bits < 63 && (h >> bits)) ++bits;
+    return qm_sort_pairs(ctx, d_ids, d_perm, n, bits, st);
+}
 
 extern "C" {
 
