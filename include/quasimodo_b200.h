@@ -222,6 +222,11 @@ int  qm_indel_table_merge(qm_indel_table *t, const qm_indel *d_records, int64_t 
 int  qm_pileup_accumulate_indels(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns,
                                  const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
                                  int64_t n_pairs, int32_t *d_counts, qm_indel_table *tab, void *stream);
+/* the same with a per-read drop mask: d_drop[r] != 0 (2 * n_pairs bytes, may be NULL) leaves read r out, as the depth cap's
+ * verdict (qm_depth_cap, qm_bam_pairs.d_drop) asks */
+int  qm_pileup_accumulate_masked(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns,
+                                 const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
+                                 int64_t n_pairs, int32_t *d_counts, qm_indel_table *tab, const uint8_t *d_drop, void *stream);
 /* ---- base alignment quality (SURVEY.md 8f-2; htslib 1.9 realn.c sam_prob_realn over probaln.c kpa_glocal) ----
  * Both mpileups of the reference flow run WITHOUT -B (rules/vcfcall.smk:39 and :115), i.e. with BAQ on: every read is re-aligned
  * to its reference window by a banded profile HMM in double precision and each aligned base's quality is capped by the phred-scaled
@@ -442,6 +447,48 @@ int qm_mpileup_text_host(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *
                          const uint8_t *h_quals, int32_t stride, const int32_t *h_lens, int64_t n_pairs, const char *const *names,
                          int64_t *h_bytes);
 int qm_mpileup_text_fetch(qm_ctx *ctx, char *h_out, int64_t bytes);
+/* the same with the order given: reads reach a column in the order of d_rank[r] (one int64 per read; a negative rank sorts after
+ * every ranked read, and such a read must not be placed).  The ranked order must list the placed reads by contig, then position.
+ * qm_bam_pairs.d_row_file is such an order: the reads of a coordinate-sorted BAM reach a column in file order, as in htslib. */
+int qm_mpileup_text_ranked(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns, const uint8_t *d_codes,
+                           const uint8_t *d_quals, int32_t stride, const int32_t *d_lens, int64_t n_pairs, const char *const *names,
+                           const int64_t *d_rank, const char **d_text, int64_t *h_bytes, void *stream);
+
+/* ---- BAM records in (the way in of rules `mpileup` / `bcftools`, rules/vcfcall.smk:39,115, which read {sample}.rmdup.bam) ----
+ * d_bytes: the uncompressed record stream of a BAM (BGZF inflated); d_rec_off[i]: byte offset of record i's block_size field.
+ * The records are the caller's selection, in file order, and must be valid: the library does not re-check them.  The driver
+ * (qm_driver pileup) checks on the host: a CIGAR of at most QM_MAX_CIGAR operations besides H and without N or P, a query length
+ * equal to l_seq, l_seq <= 512, SEQ and QUAL stored, contig and span inside the reference, coordinate order; and it leaves out the
+ * records neither mpileup admits (flag 0x4, 0x100, 0x200 or 0x400, no CIGAR, no contig).
+ * Each record becomes a read in the read-batch layout (qm_aln, codes 0..4 -- '=' and IUPAC codes are N -- and qualities at one
+ * `stride`, lengths), a reverse-strand record turned back to the orientation it was sequenced in.  CIGAR '=' and 'X' become M, H
+ * is dropped, neighbouring operations of one kind merge.  rid, pos, flag, mapq, mate_rid, mate_pos, tlen come from the record;
+ * nm, score, sub from its NM, AS, XS tags (0 without); qb = 0, qe = l_seq.
+ * Pairing: the two primary records of a name (one flagged 0x40, the other 0x80, neither 0x100 nor 0x800) are one pair, matched by
+ * a 64-bit name hash and then byte for byte; the one that comes first in the file is row 2i.  Every other record (supplementary
+ * records, a read whose mate is not among the records, single-end reads, a third primary record of a name) is a pair of its own
+ * with an empty placeholder mate (flag 0x4, rid -1, no CIGAR, length 0).  Pair i is the i-th pair in the file order of its row 2i.
+ * max_depth > 0: htslib's depth cap (qm_depth_cap) over the reads in FILE order -- the order the cap depends on -- under po;
+ * d_drop then holds the verdict per row.  baq 1 / 3: d_quals are the qualities capped by base alignment quality (qm_baq_apply).
+ * The layout lives in library scratch, valid until the next qm_bam_to_pairs* call on the context.
+ * Limits: stride <= 512 (QM_ELIMIT), n_recs < 2^31 (QM_ELIMIT); QM_EINVAL on NULL pointers, stride < 1, baq not 0 / 1 / 3.
+ * Device memory: about 2 * (150 + 2 * stride) bytes per record (file-order rows and pairing state, then the pair layout, a
+ * third copy of the qualities with BAQ) plus the sort's scratch; the _host form stages the record stream (its size) and 8 bytes
+ * per record.  Synchronous. */
+typedef struct {
+    int64_t  n_pairs;                   /* rows 2i / 2i + 1 of pair i, i < n_pairs                               */
+    int32_t  stride, pad;
+    const qm_aln  *d_alns;
+    const uint8_t *d_codes, *d_quals;   /* with baq: the capped qualities                                        */
+    const int32_t *d_lens;
+    const int64_t *d_row_file;          /* index of each row's record among the n_recs handed in, -1 = placeholder */
+    const uint8_t *d_drop;              /* max_depth > 0: 1 = the depth cap refuses the read; else NULL          */
+    int64_t  n_capped;                  /* reads the cap refuses                                                 */
+} qm_bam_pairs;
+int qm_bam_to_pairs(qm_ctx *ctx, const qm_index *idx, const uint8_t *d_bytes, const int64_t *d_rec_off, int64_t n_recs, int32_t stride,
+                    const qm_pileup_opt *po, int baq, int max_depth, qm_bam_pairs *out, void *stream);
+int qm_bam_to_pairs_host(qm_ctx *ctx, const qm_index *idx, const uint8_t *h_bytes, int64_t n_bytes, const int64_t *h_rec_off, int64_t n_recs,
+                         int32_t stride, const qm_pileup_opt *po, int baq, int max_depth, qm_bam_pairs *out);
 
 /* ---- multi-GPU: the one collective of the path (north_star: "per-GPU int32 count tensors are merged with one NCCL allreduce
  * over NVLink"; SURVEY.md 8b, 8e).  Reads shard by pair index with no data-path exchange; what crosses GPUs is the count

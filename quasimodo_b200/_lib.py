@@ -36,6 +36,13 @@ class PileupOpt(C.Structure):
                 ("ignore_overlaps", C.c_int32)]
 
 
+class BamPairs(C.Structure):
+    """qm_bam_pairs: the pair layout qm_bam_to_pairs leaves in library scratch (device pointers)"""
+    _fields_ = [("n_pairs", C.c_int64), ("stride", C.c_int32), ("pad", C.c_int32), ("d_alns", C.c_void_p), ("d_codes", C.c_void_p),
+                ("d_quals", C.c_void_p), ("d_lens", C.c_void_p), ("d_row_file", C.c_void_p), ("d_drop", C.c_void_p),
+                ("n_capped", C.c_int64)]
+
+
 class CallOpt(C.Structure):
     _fields_ = [("min_dp", C.c_int32), ("min_alt", C.c_int32), ("min_af", C.c_float), ("reserved", C.c_int32)]
 
@@ -138,6 +145,10 @@ SIGNATURES = {
     "qm_mpileup_text": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _P, _P]),
     "qm_mpileup_text_host": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P]),
     "qm_mpileup_text_fetch": (C.c_int, [_P, _P, _L]),
+    "qm_mpileup_text_ranked": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _P, _P, _P]),
+    "qm_bam_to_pairs": (C.c_int, [_P, _P, _P, _P, _L, _I, _P, C.c_int, C.c_int, C.POINTER(BamPairs), _P]),
+    "qm_bam_to_pairs_host": (C.c_int, [_P, _P, _P, _L, _P, _L, _I, _P, C.c_int, C.c_int, C.POINTER(BamPairs)]),
+    "qm_pileup_accumulate_masked": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _P, _P]),
     "qm_profile_enable": (C.c_int, [_P, C.c_int]),
     "qm_profile_collect": (C.c_int, [_P, _P, _P]),
     "qm_simulate_pairs_host": (C.c_int, [_P, _P, _P, _P, _P, _L, _L, _I, _P, _P, _P, _P]),

@@ -23,7 +23,8 @@ struct qm_ctx {
     int sm_count = 0;
     std::string err;
     // scratch arenas grown on demand (never shrunk); index = purpose.  32-36: the tuples of duplicate marking and the depth cap
-    // (dedup.cu, depthcap.cu, sort.cu, sample.cu)
+    // (dedup.cu, depthcap.cu, sort.cu, sample.cu);
+    // 37-39: BAM records in (bamin.cu: staged record stream, file-order rows and pairing state, pair layout)
     qm_scratch scratch[40];
     cudaStream_t own_stream = nullptr, copy_stream = nullptr;
     // side streams: the independent per-class extension kernels of one round run concurrently (fork/join by events)

@@ -28,6 +28,14 @@
 //          ((flag & 12) == 12 && !(flag & 256)), re-emitted as FASTQ with /1 /2 names, as sequenced.
 //          With --keep-contigs N the first N contigs of the (concatenated) reference are the target genome and
 //          a pair is dropped iff a mate maps to a later (contaminant) contig: one pass instead of three.
+//   qm_driver pileup   --ref REF.fa[,MORE.fa...] --bam IN.bam [--counts OUT.tsv] [--vcf OUT.vcf [--vcf-gz 0]] [--mpileup OUT.mpileup]
+//                      [--max-depth N] [--baq 1] [-q -Q --count-orphans 1 --ignore-overlaps 1] [--min-dp --min-alt --min-af] [--indels 0]
+//                      [--sample NAME] [--gpu I] [-t THREADS] [--stage-ms 1]
+//        = rules/vcfcall.smk:39 (`mpileup`: samtools mpileup -f ref {rmdup.bam}) and rules/vcfcall.smk:115-119 (`bcftools`): the
+//          count TSV, VCF (+ .gz + .tbi) and text pileup of an existing coordinate-sorted BAM, through the writers of `sample`, with
+//          the same defaults (BAQ off, no depth cap); the BAM of `sample` read back gives `sample`'s bytes.  The file is inflated
+//          and validated on the host before a CUDA context exists (a bad file exits 2 with or without a GPU); the records are
+//          decoded and paired on the device (qm_bam_to_pairs); the depth cap follows the file's order of the reads.
 //   qm_driver bam-from-records --ref .. --r1 .. --r2 .. --alns ALNS.bin [--perm PERM.bin] --bam OUT.bam
 //        = the BAM/BAI writer alone on given qm_aln records (test entry; with --perm no GPU is touched)
 //   qm_driver fastq-check --r1 .. --r2 .. [-t THREADS]
@@ -51,7 +59,9 @@
 #include <cmath>
 #include <cstring>
 #include <deque>
+#include <functional>
 #include <map>
+#include <mutex>
 #include <string>
 #include <thread>
 #include <vector>
@@ -1074,6 +1084,101 @@ struct PhaseClock {
     }
 };
 
+// --stage-ms 1: the library's CUDA-event stage timers of one GPU, one line in the log
+void print_stage_ms(Lib &L, int dev)
+{
+    static const char *const kStage[QM_N_STAGES] = {"seed+chain", "advance", "extend", "pair+cigar", "pileup", "h2d", "d2h", "other", "rescue"};
+    double ms[QM_N_STAGES];
+    int64_t launches[QM_N_STAGES];
+    L.check(qm_profile_collect(L.ctx, ms, launches), "qm_profile_collect");
+    std::string line;
+    double tot = 0;
+    int64_t nl = 0;
+    for (int i = 0; i < QM_N_STAGES; ++i) {
+        char buf[64];
+        snprintf(buf, sizeof buf, "%s%s %.1f", i ? ", " : "", kStage[i], ms[i]);
+        line += buf;
+        tot += ms[i];
+        nl += launches[i];
+    }
+    fprintf(stderr, "[qm_driver] GPU %d stages (ms of device time): %s; total %.1f in %lld launches\n", dev, line.c_str(), tot, (long long)nl);
+}
+
+// The outputs of the reference's rules `mpileup` and `bcftools` from a counted sample (smps[0]: count tensor and indel allele
+// table; with several GPUs the counts are summed already and the indel tables of smps[1..] are merged here): the count TSV
+// (--counts), the calls and indel records as VCF (--vcf, + .gz and .tbi unless --vcf-gz 0) and the text pileup (--mpileup).
+// make_text() leaves the text pileup on the device (qm_mpileup_text*) and returns its length.  `sample` and `pileup` both
+// write through here, so that the same counts give the same bytes.
+void write_outputs(const Args &a, const Genome &g, std::vector<Lib> &Ls, const std::vector<qm_index *> &idxs, const std::vector<qm_sample *> &smps,
+                   int threads, const std::function<int64_t()> &make_text)
+{
+    Lib &L = Ls[0];
+    qm_sample *smp = smps[0];
+    qm_index *idx = idxs[0];
+    const int n_gpu = (int)smps.size();
+    const std::string counts = a.get("counts"), vcf = a.get("vcf"), mpileup = a.get("mpileup");
+    if (!counts.empty()) {
+        std::vector<int32_t> rows(g.codes.size() * QM_NCH);
+        L.check(qm_sample_counts_host(smp, rows.data()), "qm_sample_counts_host");
+        write_count_tsv(counts, g, rows);
+    }
+    if (!vcf.empty()) {
+        qm_call_opt copt; qm_call_opt_default(&copt);
+        if (a.has("min-dp")) copt.min_dp = atoi(a.get("min-dp").c_str());
+        if (a.has("min-alt")) copt.min_alt = atoi(a.get("min-alt").c_str());
+        if (a.has("min-af")) copt.min_af = (float)atof(a.get("min-af").c_str());
+        std::vector<qm_call> calls(g.codes.size() * 3 + 16);                   // at most 3 alternative bases per position
+        int64_t nc = 0;
+        L.check(qm_sample_call_snps_host(smp, &copt, calls.data(), (int64_t)calls.size(), &nc), "qm_sample_call_snps_host");
+        calls.resize((size_t)nc);
+        // indel records (--indels 0 leaves them out): the sample's allele table against the raw depth at the anchor
+        std::vector<IndelCall> icalls;
+        if (atoi(a.get("indels", "1").c_str())) {
+            std::vector<qm_indel> tab((size_t)1 << 18);
+            int64_t nt = 0;
+            L.check(qm_indel_table_fetch_host(qm_sample_indel_table(smp), idx, tab.data(), (int64_t)tab.size(), &nt), "qm_indel_table_fetch_host");
+            if (n_gpu > 1) {
+                // the sparse part of the merge (SURVEY.md 8e: "host merge of the sparse indel-allele table"): every GPU tallied the
+                // alleles of its own batches; the tables (a few thousand records, sorted by key) are added up by key here
+                tab.resize((size_t)nt);
+                std::vector<qm_indel> other((size_t)1 << 18);
+                for (int d = 1; d < n_gpu; ++d) {
+                    int64_t no = 0;
+                    Ls[d].check(qm_indel_table_fetch_host(qm_sample_indel_table(smps[d]), idxs[d], other.data(), (int64_t)other.size(), &no), "qm_indel_table_fetch_host");
+                    tab = merge_indel_tables(tab, other.data(), no);
+                }
+                nt = (int64_t)tab.size();
+            }
+            std::vector<int32_t> rows(g.codes.size() * QM_NCH);
+            L.check(qm_sample_counts_host(smp, rows.data()), "qm_sample_counts_host");
+            for (int64_t i = 0; i < nt; ++i) {
+                const qm_indel &x = tab[(size_t)i];
+                const int dp = rows[(size_t)(g.offs[x.rid] + x.pos) * QM_NCH + 14], ad = x.n_fwd + x.n_rev;
+                if (dp < copt.min_dp || ad < copt.min_alt || (double)ad < (double)copt.min_af * dp) continue;
+                IndelCall c;
+                c.a = x; c.dp = dp; c.af = dp > 0 ? (double)ad / dp : 0.0;
+                const double f = c.af > 1.0 ? 1.0 : c.af, e = 0.002;     // same Chernoff-bound QUAL as the SNP records
+                double kl = f > 0 ? f * log(f / e) : 0.0;
+                if (f < 1.0) kl += (1.0 - f) * log((1.0 - f) / (1.0 - e));
+                const double q = f > e ? 4.342944819032518 * dp * kl : 0.0;
+                c.qual = q > 999.0 ? 999.0 : q;
+                icalls.push_back(c);
+            }
+        }
+        write_vcf(vcf, g, a.get("sample", "sample"), split(a.get("ref"), ',')[0], calls, icalls);
+        // rule `bcftools` declares vcf_bgz = vcf + ".gz" and tabix-indexes it (rules/vcfcall.smk:107,118-119): written unless --vcf-gz 0
+        if (atoi(a.get("vcf-gz", "1").c_str())) write_vcf_gz_tbi(vcf, vcf + ".gz", threads);
+    }
+    if (!mpileup.empty()) {
+        const int64_t bytes = make_text();
+        std::vector<char> text((size_t)bytes);
+        L.check(qm_mpileup_text_fetch(L.ctx, text.data(), bytes), "qm_mpileup_text_fetch");
+        FILE *fp = fopen(mpileup.c_str(), "w");
+        if (!fp || (bytes && fwrite(text.data(), 1, (size_t)bytes, fp) != (size_t)bytes) || fclose(fp) != 0) die(2, "cannot write %s", mpileup.c_str());
+        fprintf(stderr, "[qm_driver] text pileup: %lld bytes\n", (long long)bytes);
+    }
+}
+
 int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
 {
     PhaseClock pc;
@@ -1252,25 +1357,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     fprintf(stderr, "[qm_driver] %d GPU(s), %lld batch(es): %.2f s from the first read to the last record, %.3f M pairs/s, %.1f G extension cells/s "
                     "(FASTQ parsing included)\n", n_gpu, (long long)n_batches, loop_s, loop_s > 0 ? n_pairs / loop_s / 1e6 : 0.0,
             loop_s > 0 ? cells / loop_s / 1e9 : 0.0);
-    if (stage_ms) {
-        static const char *const kStage[QM_N_STAGES] = {"seed+chain", "advance", "extend", "pair+cigar", "pileup", "h2d", "d2h", "other", "rescue"};
-        for (int d = 0; d < n_gpu; ++d) {
-            double ms[QM_N_STAGES];
-            int64_t launches[QM_N_STAGES];
-            Ls[d].check(qm_profile_collect(Ls[d].ctx, ms, launches), "qm_profile_collect");
-            std::string line;
-            double tot = 0;
-            int64_t nl = 0;
-            for (int i = 0; i < QM_N_STAGES; ++i) {
-                char buf[64];
-                snprintf(buf, sizeof buf, "%s%s %.1f", i ? ", " : "", kStage[i], ms[i]);
-                line += buf;
-                tot += ms[i];
-                nl += launches[i];
-            }
-            fprintf(stderr, "[qm_driver] GPU %d stages (ms of device time): %s; total %.1f in %lld launches\n", devs[d], line.c_str(), tot, (long long)nl);
-        }
-    }
+    if (stage_ms) for (int d = 0; d < n_gpu; ++d) print_stage_ms(Ls[d], devs[d]);
     int64_t n_dup = 0, n_capped = 0;
     if (n_gpu > 1) {
         // per-GPU int32 count tensors -> one NCCL all-reduce over NVLink; every GPU ends up with the sample's totals.  Deferred
@@ -1321,59 +1408,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     }
 
     pc.mark("merge / deferred counting");
-    if (!counts.empty()) {
-        std::vector<int32_t> rows(g.codes.size() * QM_NCH);
-        L.check(qm_sample_counts_host(smp, rows.data()), "qm_sample_counts_host");
-        write_count_tsv(counts, g, rows);
-    }
-    if (!vcf.empty()) {
-        qm_call_opt copt; qm_call_opt_default(&copt);
-        if (a.has("min-dp")) copt.min_dp = atoi(a.get("min-dp").c_str());
-        if (a.has("min-alt")) copt.min_alt = atoi(a.get("min-alt").c_str());
-        if (a.has("min-af")) copt.min_af = (float)atof(a.get("min-af").c_str());
-        std::vector<qm_call> calls(g.codes.size() * 3 + 16);                   // at most 3 alternative bases per position
-        int64_t nc = 0;
-        L.check(qm_sample_call_snps_host(smp, &copt, calls.data(), (int64_t)calls.size(), &nc), "qm_sample_call_snps_host");
-        calls.resize((size_t)nc);
-        // indel records (--indels 0 leaves them out): the sample's allele table against the raw depth at the anchor
-        std::vector<IndelCall> icalls;
-        if (atoi(a.get("indels", "1").c_str())) {
-            std::vector<qm_indel> tab((size_t)1 << 18);
-            int64_t nt = 0;
-            L.check(qm_indel_table_fetch_host(qm_sample_indel_table(smp), idx, tab.data(), (int64_t)tab.size(), &nt), "qm_indel_table_fetch_host");
-            if (n_gpu > 1) {
-                // the sparse part of the merge (SURVEY.md 8e: "host merge of the sparse indel-allele table"): every GPU tallied the
-                // alleles of its own batches; the tables (a few thousand records, sorted by key) are added up by key here
-                tab.resize((size_t)nt);
-                std::vector<qm_indel> other((size_t)1 << 18);
-                for (int d = 1; d < n_gpu; ++d) {
-                    int64_t no = 0;
-                    Ls[d].check(qm_indel_table_fetch_host(qm_sample_indel_table(smps[d]), idxs[d], other.data(), (int64_t)other.size(), &no), "qm_indel_table_fetch_host");
-                    tab = merge_indel_tables(tab, other.data(), no);
-                }
-                nt = (int64_t)tab.size();
-            }
-            std::vector<int32_t> rows(g.codes.size() * QM_NCH);
-            L.check(qm_sample_counts_host(smp, rows.data()), "qm_sample_counts_host");
-            for (int64_t i = 0; i < nt; ++i) {
-                const qm_indel &x = tab[(size_t)i];
-                const int dp = rows[(size_t)(g.offs[x.rid] + x.pos) * QM_NCH + 14], ad = x.n_fwd + x.n_rev;
-                if (dp < copt.min_dp || ad < copt.min_alt || (double)ad < (double)copt.min_af * dp) continue;
-                IndelCall c;
-                c.a = x; c.dp = dp; c.af = dp > 0 ? (double)ad / dp : 0.0;
-                const double f = c.af > 1.0 ? 1.0 : c.af, e = 0.002;     // same Chernoff-bound QUAL as the SNP records
-                double kl = f > 0 ? f * log(f / e) : 0.0;
-                if (f < 1.0) kl += (1.0 - f) * log((1.0 - f) / (1.0 - e));
-                const double q = f > e ? 4.342944819032518 * dp * kl : 0.0;
-                c.qual = q > 999.0 ? 999.0 : q;
-                icalls.push_back(c);
-            }
-        }
-        write_vcf(vcf, g, a.get("sample", "sample"), split(a.get("ref"), ',')[0], calls, icalls);
-        // rule `bcftools` declares vcf_bgz = vcf + ".gz" and tabix-indexes it (rules/vcfcall.smk:107,118-119): written unless --vcf-gz 0
-        if (atoi(a.get("vcf-gz", "1").c_str())) write_vcf_gz_tbi(vcf, vcf + ".gz", threads);
-    }
-    if (!mpileup.empty()) {
+    write_outputs(a, g, Ls, idxs, smps, threads, [&]() {
         // text pileup (samtools mpileup format) of the whole sample: records, reads and qualities go to the device once more,
         // at one common stride; the text comes back in one piece
         int32_t stride = 1;
@@ -1401,12 +1436,8 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         int64_t bytes = 0;
         L.check(qm_mpileup_text_host(L.ctx, idx, &popt, alns.data(), codes.data(), quals.data(), stride, lens.data(), n_pairs, nm.data(), &bytes),
                 "qm_mpileup_text_host");
-        std::vector<char> text((size_t)bytes);
-        L.check(qm_mpileup_text_fetch(L.ctx, text.data(), bytes), "qm_mpileup_text_fetch");
-        FILE *fp = fopen(mpileup.c_str(), "w");
-        if (!fp || (bytes && fwrite(text.data(), 1, (size_t)bytes, fp) != (size_t)bytes) || fclose(fp) != 0) die(2, "cannot write %s", mpileup.c_str());
-        fprintf(stderr, "[qm_driver] text pileup: %lld bytes\n", (long long)bytes);
-    }
+        return bytes;
+    });
     pc.mark("count TSV + calls + VCF + text pileup");
     if (want_bam) {
         // coordinate sort on the device: keys from the records, stable radix sort, gather through the permutation
@@ -1514,6 +1545,260 @@ int cmd_bam_from_records(const Args &a, const std::string &cmdline)
     return 0;
 }
 
+
+// ------------------------------------------------------------------------------------------------
+// BAM reader (`pileup`): the input of the reference's rules `mpileup` and `bcftools` (rules/vcfcall.smk:39,115 read
+// {sample}.{ref_name}.rmdup.bam).  Everything here runs before a CUDA context exists, so a bad file fails the same way with
+// or without a GPU.
+inline uint32_t le16(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8; }
+inline uint32_t le32(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24; }
+
+// the whole file, BGZF members inflated on the -t threads into one stream.  Every member's gzip header and BC field, its CRC32
+// and ISIZE, and the end-of-file block are checked (a file cut at a block boundary still lacks the EOF block).
+std::vector<uint8_t> inflate_bgzf(const std::string &path)
+{
+    std::vector<uint8_t> raw;
+    {
+        const int fd = open(path.c_str(), O_RDONLY);
+        if (fd < 0) die(2, "cannot open %s", path.c_str());
+        const off_t sz = lseek(fd, 0, SEEK_END);
+        if (sz < 0) die(2, "cannot read %s", path.c_str());
+        raw.resize((size_t)sz);
+        size_t got = 0;
+        while (got < raw.size()) {
+            const ssize_t n = pread(fd, raw.data() + got, raw.size() - got, (off_t)got);
+            if (n < 0 && errno == EINTR) continue;
+            if (n <= 0) die(2, "read error in %s", path.c_str());
+            got += (size_t)n;
+        }
+        close(fd);
+    }
+    struct Member { size_t off, data, clen, uoff; uint32_t isize; };
+    std::vector<Member> mem;
+    size_t p = 0, total = 0;
+    while (p < raw.size()) {
+        const uint8_t *h = raw.data() + p;
+        if (raw.size() - p < 18) die(2, "%s: truncated BGZF block at byte %zu", path.c_str(), p);
+        if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4))
+            die(2, "%s: bad BGZF magic at byte %zu: not a BGZF-compressed BAM", path.c_str(), p);
+        const size_t xlen = le16(h + 10);
+        size_t bsize = 0;
+        for (size_t x = 12; x + 4 <= 12 + xlen && p + x + 4 <= raw.size();) {
+            const size_t slen = le16(h + x + 2);
+            if (h[x] == 'B' && h[x + 1] == 'C' && slen == 2 && p + x + 6 <= raw.size()) bsize = le16(h + x + 4) + 1;
+            x += 4 + slen;
+        }
+        if (bsize == 0) die(2, "%s: bad BGZF magic at byte %zu: gzip member without a BC field", path.c_str(), p);
+        if (bsize < 12 + xlen + 8) die(2, "%s: BGZF block at byte %zu is too short", path.c_str(), p);
+        if (p + bsize > raw.size()) die(2, "%s: truncated BGZF block at byte %zu", path.c_str(), p);
+        const uint32_t isize = le32(h + bsize - 4);
+        if (isize > 65536) die(2, "%s: BGZF block at byte %zu claims %u bytes (at most 65536)", path.c_str(), p, isize);
+        mem.push_back({p, p + 12 + xlen, bsize - 12 - xlen - 8, total, isize});
+        total += isize;
+        p += bsize;
+    }
+    static const uint8_t kEof[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+    if (mem.empty() || raw.size() - mem.back().off != 28 || memcmp(raw.data() + mem.back().off, kEof, 28) != 0)
+        die(2, "%s: no BGZF end-of-file block: the file is truncated", path.c_str());
+    std::vector<uint8_t> out(total);
+    std::vector<uint8_t> err(mem.size(), 0);                   // 1 does not inflate to ISIZE, 2 CRC32 mismatch
+    std::atomic<size_t> next{0};
+    auto work = [&]() {
+        z_stream zs;
+        memset(&zs, 0, sizeof zs);
+        if (inflateInit2(&zs, -15) != Z_OK) return;
+        for (size_t i; (i = next.fetch_add(64)) < mem.size();)
+            for (size_t k = i; k < std::min(mem.size(), i + 64); ++k) {
+                const Member &m = mem[k];
+                inflateReset(&zs);
+                zs.next_in = raw.data() + m.data; zs.avail_in = (uInt)m.clen;
+                zs.next_out = out.data() + m.uoff; zs.avail_out = m.isize;
+                uint8_t spare;
+                if (m.isize == 0) { zs.next_out = &spare; zs.avail_out = 1; }
+                if (inflate(&zs, Z_FINISH) != Z_STREAM_END || zs.total_out != m.isize) { err[k] = 1; continue; }
+                const uint32_t crc = (uint32_t)crc32(crc32(0L, Z_NULL, 0), out.data() + m.uoff, m.isize);
+                if (crc != le32(raw.data() + m.data + m.clen)) err[k] = 2;
+            }
+        inflateEnd(&zs);
+    };
+    std::vector<std::thread> team;
+    for (int t = 1; t < std::min<int>(g_threads, (int)(mem.size() / 64) + 1); ++t) team.emplace_back(work);
+    work();
+    for (auto &t : team) t.join();
+    for (size_t k = 0; k < mem.size(); ++k) {
+        if (err[k] == 1) die(2, "%s: BGZF block at byte %zu does not inflate to its ISIZE of %u bytes", path.c_str(), mem[k].off, mem[k].isize);
+        if (err[k] == 2) die(2, "%s: CRC32 mismatch in the BGZF block at byte %zu", path.c_str(), mem[k].off);
+    }
+    return out;
+}
+
+// what the validation walk leaves for the device: the byte offsets of the records the pileup may admit, in file order
+struct BamRecords {
+    std::vector<int64_t> off;
+    int32_t max_len = 0;
+    int64_t n_total = 0, n_left_out = 0;
+};
+
+// The header must list the FASTA's contigs (names, lengths, order), as bcftools refuses a mismatched -f; then one walk over the
+// records: coordinate order (as htslib's pileup checks it: placed records without 0x4, contig, then position), and on every
+// record the pileup may admit what the device decode relies on.  Records neither mpileup admits (0x4, 0x100, 0x200, 0x400, no
+// contig, no CIGAR) are left out.  Every failure names the read and exits 2.
+BamRecords scan_bam(const std::string &path, const std::vector<uint8_t> &d, const Genome &g)
+{
+    const char *fn = path.c_str();
+    if (d.size() < 12 || memcmp(d.data(), "BAM\1", 4) != 0) die(2, "%s: bad BAM magic: not a BAM file", fn);
+    size_t p = 8 + (size_t)le32(d.data() + 4);
+    if (p + 4 > d.size()) die(2, "%s: truncated BAM header", fn);
+    const uint32_t n_ref = le32(d.data() + p);
+    p += 4;
+    std::vector<std::string> names;
+    std::vector<int64_t> lens;
+    for (uint32_t i = 0; i < n_ref; ++i) {
+        if (p + 4 > d.size()) die(2, "%s: truncated BAM header", fn);
+        const size_t ln = le32(d.data() + p);
+        if (ln < 1 || p + 8 + ln > d.size()) die(2, "%s: truncated BAM header", fn);
+        names.emplace_back((const char *)d.data() + p + 4, ln - 1);
+        lens.push_back((int64_t)le32(d.data() + p + 4 + ln));
+        p += 8 + ln;
+    }
+    if (names.size() != g.names.size())
+        die(2, "%s: the header lists %zu contigs (@SQ), the reference %zu: the BAM was not aligned to this reference", fn, names.size(), g.names.size());
+    for (size_t i = 0; i < names.size(); ++i)
+        if (names[i] != g.names[i] || lens[i] != g.lens[i])
+            die(2, "%s: @SQ %zu is %s of %lld bp, contig %zu of the reference is %s of %lld bp: the BAM was not aligned to this reference",
+                fn, i + 1, names[i].c_str(), (long long)lens[i], i + 1, g.names[i].c_str(), (long long)g.lens[i]);
+    // the record offsets (a serial chain of block_size fields) and the coordinate order
+    std::vector<int64_t> all;
+    int32_t last_tid = -1, last_pos = -1;
+    for (; p < d.size();) {
+        if (p + 36 > d.size()) die(2, "%s: truncated record at byte %zu of the BAM stream", fn, p);
+        const uint8_t *r = d.data() + p;
+        const size_t bs = le32(r);
+        if (bs < 32 || p + 4 + bs > d.size() || 32 + (size_t)r[12] > bs) die(2, "%s: malformed or truncated record at byte %zu of the BAM stream", fn, p);
+        const int32_t tid = (int32_t)le32(r + 4), pos = (int32_t)le32(r + 8);
+        if (tid >= 0 && !(le16(r + 18) & 0x4)) {
+            if (tid < last_tid || (tid == last_tid && pos < last_pos))
+                die(2, "%s: the file is not coordinate-sorted: read %.*s at %s:%d comes after %s:%d", fn, std::max(0, (int)r[12] - 1), (const char *)r + 36,
+                    tid < (int32_t)names.size() ? names[(size_t)tid].c_str() : "?", pos + 1, names[(size_t)last_tid].c_str(), last_pos + 1);
+            last_tid = tid; last_pos = pos;
+        }
+        all.push_back((int64_t)p);
+        p += 4 + bs;
+    }
+    // the per-record checks, on the -t threads; the first failure in file order is reported
+    std::vector<uint8_t> keep(all.size(), 0);
+    std::vector<std::pair<size_t, std::string>> bad;
+    std::mutex mu;
+    parallel_ranges(all.size(), [&](size_t b, size_t e) {
+        for (size_t i = b; i < e; ++i) {
+            const uint8_t *r = d.data() + all[i];
+            const size_t bs = le32(r), l_name = r[12], n_cig = le16(r + 16);
+            const int flag = (int)le16(r + 18);
+            const int32_t tid = (int32_t)le32(r + 4), pos = (int32_t)le32(r + 8), l_seq = (int32_t)le32(r + 20);
+            const std::string name((const char *)r + 36, l_name ? l_name - 1 : 0);
+            auto fail = [&](const std::string &why) { std::lock_guard<std::mutex> lk(mu); bad.emplace_back(i, "read " + name + ": " + why); };
+            if (l_seq < 0 || 36 + l_name + 4 * n_cig + (size_t)(l_seq + 1) / 2 + (size_t)l_seq > 4 + bs) { fail("malformed record"); return; }
+            if (tid >= (int32_t)names.size()) { fail("contig id " + std::to_string(tid) + " is not in the header"); return; }
+            if ((flag & (0x4 | 0x100 | 0x200 | 0x400)) || tid < 0 || n_cig == 0) continue;       // never admitted: left out
+            const uint8_t *cig = r + 36 + l_name;
+            int n_ops = 0;
+            int64_t qlen = 0, span = 0;
+            for (size_t k = 0; k < n_cig; ++k) {
+                const uint32_t w = le32(cig + 4 * k), op = w & 0xf, len = w >> 4;
+                if (op == 3 || op == 6) { fail(std::string("CIGAR operation ") + "MIDNSHP=X"[op] + ": N and P are not supported"); return; }
+                if (op > 8) { fail("invalid CIGAR operation"); return; }
+                if (op != 5) ++n_ops;
+                if (op == 0 || op == 1 || op == 4 || op == 7 || op == 8) qlen += len;
+                if (op == 0 || op == 2 || op == 7 || op == 8) span += len;
+            }
+            if (l_seq == 0) { fail("no stored SEQ ('*')"); return; }
+            if (r[36 + l_name + 4 * n_cig + (size_t)(l_seq + 1) / 2] == 0xff) { fail("no stored QUAL ('*')"); return; }
+            if (l_seq > 512) { fail(std::to_string(l_seq) + " bases: reads longer than 512 bases are not supported"); return; }
+            if (n_ops > QM_MAX_CIGAR) { fail(std::to_string(n_ops) + " CIGAR operations: at most " + std::to_string(QM_MAX_CIGAR) + " besides H are supported"); return; }
+            if (qlen != l_seq) { fail("CIGAR query length " + std::to_string(qlen) + " differs from the " + std::to_string(l_seq) + " bases of SEQ"); return; }
+            if (pos < 0 || pos + span > g.lens[(size_t)tid]) { fail("alignment outside contig " + names[(size_t)tid]); return; }
+            keep[i] = 1;
+        }
+    });
+    if (!bad.empty()) {
+        auto it = std::min_element(bad.begin(), bad.end(), [](const auto &x, const auto &y) { return x.first < y.first; });
+        die(2, "%s: %s", fn, it->second.c_str());
+    }
+    BamRecords out;
+    out.n_total = (int64_t)all.size();
+    for (size_t i = 0; i < all.size(); ++i)
+        if (keep[i]) { out.off.push_back(all[i]); out.max_len = std::max(out.max_len, (int32_t)le32(d.data() + all[i] + 20)); }
+    out.n_left_out = out.n_total - (int64_t)out.off.size();
+    return out;
+}
+
+// counts, calls and text pileup of an existing coordinate-sorted BAM: rules `mpileup` and `bcftools` one for one
+int cmd_pileup(const Args &a)
+{
+    PhaseClock pc;
+    require_known(a, "pileup", {"ref", "bam", "counts", "vcf", "vcf-gz", "mpileup", "max-depth", "baq", "min-mapq", "q", "min-bq", "Q",
+                                "count-orphans", "ignore-overlaps", "min-dp", "min-alt", "min-af", "indels", "sample", "gpu", "t", "threads", "stage-ms"});
+    if (!a.has("ref") || !a.has("bam")) die(1, "--ref and --bam are required");
+    const int threads = std::max(1, atoi(a.get("t", a.get("threads", "4")).c_str()));
+    g_threads = threads;
+    qm_pileup_opt popt; qm_pileup_opt_default(&popt);
+    apply_mpileup_options(a, popt);
+    // the defaults of `sample`: no depth cap and BAQ off (the parity configuration); --max-depth caps the counts and calls only
+    const int max_depth = a.has("max-depth") ? parse_int("max-depth", a.get("max-depth")) : 0;
+    const int baq = a.has("baq") && parse_int("baq", a.get("baq")) ? 3 : 0;
+    Genome g;
+    load_refs(a.get("ref"), g);
+    pc.mark("reference");
+    const std::string path = a.get("bam");
+    const std::vector<uint8_t> data = inflate_bgzf(path);
+    pc.mark("BGZF inflate");
+    const BamRecords recs = scan_bam(path, data, g);
+    pc.mark("validation walk");
+    fprintf(stderr, "[qm_driver] %s: %lld records, %lld left out (unmapped, secondary, QC-failed, duplicate or without CIGAR)\n", path.c_str(),
+            (long long)recs.n_total, (long long)recs.n_left_out);
+    Lib L;
+    const int dev = atoi(a.get("gpu", "0").c_str());
+    const int rc = qm_ctx_create(dev, &L.ctx);
+    if (rc != QM_OK) die(3, "qm_ctx_create(%d) failed (%d): no usable B200 (there is no CPU fallback)", dev, rc);
+    const bool stage_ms = atoi(a.get("stage-ms", "0").c_str()) != 0;
+    if (stage_ms) L.check(qm_profile_enable(L.ctx, 1), "qm_profile_enable");
+    qm_opt opt; qm_opt_default(&opt);
+    std::vector<qm_index *> idxs(1, nullptr);
+    std::vector<qm_sample *> smps(1, nullptr);
+    L.check(qm_index_build(L.ctx, g.codes.data(), (int)g.names.size(), g.lens.data(), opt.min_seed_len, &idxs[0]), "qm_index_build");
+    L.check(qm_sample_begin(L.ctx, idxs[0], &opt, &popt, &smps[0]), "qm_sample_begin");      // holds the count tensor and the indel table
+    pc.mark("context + reference on the device");
+    const int32_t stride = std::max<int32_t>(16, (recs.max_len + 15) & ~15);
+    qm_bam_pairs bp;
+    L.check(qm_bam_to_pairs_host(L.ctx, idxs[0], data.data(), (int64_t)data.size(), recs.off.data(), (int64_t)recs.off.size(), stride, &popt, baq,
+                                 max_depth, &bp), "qm_bam_to_pairs_host");
+    pc.mark("device decode + pairing");
+    L.check(qm_pileup_accumulate_masked(L.ctx, idxs[0], &popt, bp.d_alns, bp.d_codes, bp.d_quals, bp.stride, bp.d_lens, bp.n_pairs,
+                                        qm_sample_counts(smps[0]), qm_sample_indel_table(smps[0]), bp.d_drop, nullptr), "qm_pileup_accumulate_masked");
+    L.check(qm_sample_stats_sync(smps[0], nullptr, nullptr, nullptr), "qm_sample_stats_sync");
+    pc.mark("counting");
+    fprintf(stderr, "[qm_driver] %lld records in %lld pairs (rows 2i / 2i + 1, a placeholder mate where a record has none)\n",
+            (long long)recs.off.size(), (long long)bp.n_pairs);
+    if (max_depth > 0) fprintf(stderr, "[qm_driver] depth cap %d: %lld reads dropped by the pileup iterator\n", max_depth, (long long)bp.n_capped);
+    std::vector<Lib> Ls(1, L);
+    write_outputs(a, g, Ls, idxs, smps, threads, [&]() {
+        // the uncapped text pileup, reads in file order at every column as htslib's iterator delivers them
+        std::vector<const char *> nm;
+        for (auto &s : g.names) nm.push_back(s.c_str());
+        const char *d_text = nullptr;
+        int64_t bytes = 0;
+        L.check(qm_mpileup_text_ranked(L.ctx, idxs[0], &popt, bp.d_alns, bp.d_codes, bp.d_quals, bp.stride, bp.d_lens, bp.n_pairs, nm.data(),
+                                       bp.d_row_file, &d_text, &bytes, nullptr), "qm_mpileup_text_ranked");
+        return bytes;
+    });
+    pc.mark("outputs");
+    if (stage_ms) print_stage_ms(L, dev);
+    qm_sample_destroy(smps[0]);
+    qm_index_destroy(L.ctx, idxs[0]);
+    qm_ctx_destroy(L.ctx);
+    pc.report();
+    return 0;
+}
 }  // namespace
 
 // --benchmark FILE (any command): the job's resources in the shape of a Snakemake `benchmark:` file (one header line, one row:
@@ -1556,7 +1841,7 @@ int main(int argc, char **argv)
 {
     g_benchmark_t0 = std::chrono::steady_clock::now();
     g_benchmark_cpu0 = clock();
-    if (argc < 2) die(1, "usage: qm_driver sample|decontam|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
+    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
     std::string cmdline;
     for (int i = 0; i < argc; ++i) { if (i) cmdline += ' '; cmdline += argv[i]; }
     const std::string cmd = argv[1];
@@ -1569,6 +1854,7 @@ int main(int argc, char **argv)
     if (cmd == "sample") return cmd_sample(a, cmdline, false);
     if (cmd == "decontam") return cmd_sample(a, cmdline, true);
     if (cmd == "bam-from-records") return cmd_bam_from_records(a, cmdline);
+    if (cmd == "pileup") return cmd_pileup(a);
     if (cmd == "fastq-check") {                        // host only: parse the two mate files as `sample` would, report what is there
         require_known(a, "fastq-check", {"r1", "r2", "t", "threads"});
         if (!a.has("r1") || !a.has("r2")) die(1, "--r1 --r2 are required");

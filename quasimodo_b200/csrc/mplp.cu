@@ -144,6 +144,13 @@ __global__ void mplp_starts_kernel(const uint32_t *__restrict__ perm, const qm_a
     sinfo[k] = s;
 }
 
+// sort keys from a caller-given order: rank[r] >= 0 is record r's place, a negative rank puts the record after every ranked one
+__global__ void mplp_rank_keys_kernel(const int64_t *__restrict__ rank, int64_t n, uint64_t *__restrict__ keys)
+{
+    const int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (r < n) keys[r] = rank[r] >= 0 ? (uint64_t)rank[r] : (uint64_t)(n + r);
+}
+
 __device__ __forceinline__ int n_digits(int v) { int d = 1; while (v >= 10) { v /= 10; ++d; } return d; }
 
 // what a record contributes to the column at contig position p (htslib resolve_cigar2)
@@ -289,15 +296,12 @@ mplp_column_kernel(IndexView V, qm_pileup_opt po, const qm_aln *__restrict__ aln
     }
 }
 
-}  // namespace
-
-extern "C" {
-
 // Text pileup of the device-resident records of one sample.  *d_text points into library scratch (valid until the next
 // call on this context that produces text); *h_bytes = its length.  names: contig names, '\0'-terminated, n_contigs of them.
-int qm_mpileup_text(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns, const uint8_t *d_codes,
-                    const uint8_t *d_quals, int32_t stride, const int32_t *d_lens, int64_t n_pairs, const char *const *names,
-                    const char **d_text, int64_t *h_bytes, void *stream)
+// d_rank NULL: reads reach a column in samtools' sort order (ties in record order); else in the order of d_rank.
+int mplp_text(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns, const uint8_t *d_codes,
+              const uint8_t *d_quals, int32_t stride, const int32_t *d_lens, int64_t n_pairs, const char *const *names,
+              const int64_t *d_rank, const char **d_text, int64_t *h_bytes, void *stream)
 {
     if (!ctx || !idx || !po || !names || !d_text || !h_bytes || n_pairs < 0 || (n_pairs > 0 && (!d_alns || !d_codes || !d_quals || !d_lens)))
         return QM_EINVAL;
@@ -341,8 +345,14 @@ int qm_mpileup_text(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, c
     const int blocks = ctx->sm_count * 8;
     mplp_prepare_kernel<<<blocks, kWarps * 32, 0, st>>>(V, *po, d_alns, d_codes, d_quals, stride, d_lens, n_pairs, tq, info, max_span);
     int key_bits = 0;
-    rc = qm_aln_sort_keys(ctx, idx, d_alns, n, keys, &key_bits, stream);
-    if (rc) return rc;
+    if (d_rank) {
+        mplp_rank_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_rank, n, keys);
+        key_bits = 1;
+        while (key_bits < 63 && ((uint64_t)2 * n >> key_bits)) ++key_bits;
+    } else {
+        rc = qm_aln_sort_keys(ctx, idx, d_alns, n, keys, &key_bits, stream);
+        if (rc) return rc;
+    }
     rc = qm_sort_pairs(ctx, keys, perm, n, key_bits, stream);
     if (rc) return rc;
     mplp_starts_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(perm, d_alns, info, d_lens, V, n, starts, sinfo);
@@ -362,6 +372,25 @@ int qm_mpileup_text(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, c
     QM_CUDA(ctx, cudaStreamSynchronize(st));
     *d_text = (const char *)tp; *h_bytes = total;
     return QM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int qm_mpileup_text(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns, const uint8_t *d_codes,
+                    const uint8_t *d_quals, int32_t stride, const int32_t *d_lens, int64_t n_pairs, const char *const *names,
+                    const char **d_text, int64_t *h_bytes, void *stream)
+{
+    return mplp_text(ctx, idx, po, d_alns, d_codes, d_quals, stride, d_lens, n_pairs, names, nullptr, d_text, h_bytes, stream);
+}
+
+int qm_mpileup_text_ranked(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns, const uint8_t *d_codes,
+                           const uint8_t *d_quals, int32_t stride, const int32_t *d_lens, int64_t n_pairs, const char *const *names,
+                           const int64_t *d_rank, const char **d_text, int64_t *h_bytes, void *stream)
+{
+    if (!d_rank && n_pairs > 0) return QM_EINVAL;
+    return mplp_text(ctx, idx, po, d_alns, d_codes, d_quals, stride, d_lens, n_pairs, names, d_rank, d_text, h_bytes, stream);
 }
 
 // host entry for the driver: records, reads and qualities of the whole sample in host memory; the text stays on the device

@@ -196,11 +196,10 @@ int qm_ext_launch_classes(qm_ctx *ctx, const ExtParams &P, const IndexView &V, c
 // QM_EINVAL on a negative id.  Synchronous.
 int qm_sort_ids(qm_ctx *ctx, uint64_t *d_ids, uint32_t *d_perm, int64_t n, const char *who, cudaStream_t st);
 
-// internal: qm_pileup_accumulate_indels with a per-read drop mask (depth cap)
-struct qm_indel_table;
-extern "C" int qm_pileup_accumulate_masked(qm_ctx *ctx, const qm_index *idx, const qm_pileup_opt *po, const qm_aln *d_alns,
-                                const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
-                                int64_t n_pairs, int32_t *d_counts, qm_indel_table *tab, const uint8_t *d_drop, void *stream);
+// bamin.cu: qm_bam_to_pairs with the name hash cut to hash_bits bits (tests: pairing through colliding hashes)
+extern "C" int qm_bam_to_pairs_hashbits(qm_ctx *ctx, const qm_index *idx, const uint8_t *d_bytes, const int64_t *d_rec_off, int64_t n_recs,
+                                        int32_t stride, const qm_pileup_opt *po, int baq, int max_depth, int hash_bits, qm_bam_pairs *out,
+                                        void *stream);
 
 // sample.cu: packed reads (2 bits per base + N flags) -> one code byte per base, rows [0, n_reads)
 cudaError_t qm_unpack_reads_launch(const uint8_t *d_bases2, const uint8_t *d_nmask, int stride, int stride_p, int stride_m, int64_t n_reads,

@@ -2,7 +2,8 @@
 paths of rules `bwa` (rules/bwa.smk:1-19), `rmdup` (rules/rmdup.smk:1-18), `mpileup` (rules/vcfcall.smk:26-40) and `bcftools`
 (rules/vcfcall.smk:101-120), and the ONE `qm_driver sample` invocation that produces all of them.  Snakemake deletes a job
 whose declared output is missing, so tests/test_rules_cpu.py checks these tables against the reference's rule files and
-tests/test_driver_gpu.py checks that the command really writes every path."""
+tests/test_driver_gpu.py checks that the command really writes every path.  pileup_commands gives rules `mpileup` and
+`bcftools` one `qm_driver pileup` job each, on the .rmdup.bam a separate alignment step left."""
 import os
 
 # rule -> {output name ("" = the rule's single unnamed output): (directory variable, path pattern)}
@@ -18,7 +19,8 @@ RULE_LOGS = {
     "rmdup": ("report_dir", "/picard/{sample}.{ref_name}.rmdup.metrics.txt"),
 }
 # `benchmark:` files of the replaced rules (rules/vcfcall.smk:32-33,108-109; `bwa` and `rmdup` declare none): one driver job stands
-# for all four rules, its `--benchmark` file goes to the last rule's path
+# for all four rules, its `--benchmark` file goes to the last rule's path; the per-rule `qm_driver pileup` jobs
+# (pileup_commands) write one each
 RULE_BENCHMARKS = {
     "mpileup": ("report_dir", "/benchmarks/{sample}.{ref_name}.mpileup.benchmark.txt"),
     "bcftools": ("report_dir", "/benchmarks/{sample}.{ref_name}.bcftools.benchmark.txt"),
@@ -61,3 +63,30 @@ def sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads=4, ex
         os.makedirs(os.path.dirname(b), exist_ok=True)
         argv += ["--benchmark", b]
     return argv + list(extra), paths
+
+
+def pileup_commands(driver, dirs, sample, ref_name, ref_fa, threads=4, extra=(), benchmark=False):
+    """-> {rule: (argv, [every path the rule declares or leaves behind])} for the per-rule replacements of `mpileup` and
+    `bcftools`: each runs `qm_driver pileup` on the rule's own input, {sample}.{ref_name}.rmdup.bam (rules/vcfcall.smk:29,104),
+    writes only the rule's declared outputs and, with benchmark=True, its own `benchmark:` file (so that Snakemake can rerun
+    one of them without the alignment)."""
+    bam = expand(dirs, "rmdup", "rmdupbam", sample, ref_name)
+    out = {}
+    for rule in ("mpileup", "bcftools"):
+        argv = [driver, "pileup", "--ref", ref_fa, "--bam", bam, "--sample", sample, "-t", str(threads)]
+        paths = []
+        for name in RULE_OUTPUTS[rule]:
+            p = expand(dirs, rule, name, sample, ref_name)
+            os.makedirs(os.path.dirname(p), exist_ok=True)
+            paths.append(p)
+            opt = DRIVER_OPTION[(rule, name)]
+            if opt:
+                argv += [opt, p]
+            if (rule, name) in SIDE_FILES:
+                paths.append(p + SIDE_FILES[(rule, name)])
+        if benchmark:
+            b = benchmark_path(dirs, rule, sample, ref_name)
+            os.makedirs(os.path.dirname(b), exist_ok=True)
+            argv += ["--benchmark", b]
+        out[rule] = (argv + list(extra), paths)
+    return out
