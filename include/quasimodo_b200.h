@@ -490,6 +490,35 @@ int qm_bam_to_pairs(qm_ctx *ctx, const qm_index *idx, const uint8_t *d_bytes, co
 int qm_bam_to_pairs_host(qm_ctx *ctx, const qm_index *idx, const uint8_t *h_bytes, int64_t n_bytes, const int64_t *h_rec_off, int64_t n_recs,
                          int32_t stride, const qm_pileup_opt *po, int baq, int max_depth, qm_bam_pairs *out);
 
+/* ---- duplicate marking of a coordinate-sorted BAM (the rule `rmdup`, rules/rmdup.smk:13-16: picard MarkDuplicates
+ * REMOVE_DUPLICATES=true on a sorted file; qm_driver rmdup) ----
+ * d_bytes: the uncompressed record stream; d_rec_off[i]: byte offset of record i's block_size field, for EVERY record of the file in
+ * file order.  The records must be well-formed (the library does not re-check them); N and P operations, any number of CIGAR
+ * operations, any read length and a missing SEQ or QUAL are fine.  d_dup[i] = 1: record i is a duplicate.
+ * The rule (dedup.cu's, SURVEY.md B.9, stated for a file):
+ *  - units: the two primary records of a name (one 0x40, one 0x80, neither 0x100 nor 0x800, the only two such records of the
+ *    name; qm_bam_to_pairs' pairing rule) are a pair unit; every other primary record is a lone unit.  The pairing runs over all
+ *    records, 0x4, 0x200 and 0x400 included;
+ *  - a record is placed when it lacks 0x4, has a contig id >= 0 and a CIGAR.  Its end is {contig, unclipped 5' coordinate,
+ *    strand}: pos - (S and H at the start) forward, pos + reference span - 1 + (S and H at the end) reverse, the span counting
+ *    M D N = X;
+ *  - a unit with two placed ends gets a pair key, one with a single placed end a fragment key, one without is never a candidate.
+ *    The score is the sum of the stored qualities >= 15 of the placed ends (a QUAL of '*' scores 0);
+ *  - a unit's id is the file index of its end with the smaller {contig, unclipped 5' coordinate} (the earlier record on a tie), or
+ *    of its one placed record; ties of the decision go to the lowest id, which is picard's read1IndexInFile (recalled, not
+ *    checked against picard);
+ *  - a duplicate unit loses its placed records; unplaced mates, secondary and supplementary records are never duplicates, and a
+ *    0x400 flag in the input is ignored (picard's behaviour on sorted input as recalled).
+ * *h_n_units: all units (picard's READ_PAIRS_EXAMINED as qm_driver reports it); *h_n_dup_units: duplicate units.
+ * Limits: the 30-bit end code (16 contigs, contigs under 2^26 - 4096 bases, QM_ELIMIT when an end does not fit), n_recs < 2^31
+ * (QM_ELIMIT).  Device memory: about 90 bytes per record for the records' state and tuples, plus the decision's 70 bytes per unit
+ * with a placed end and the sorts' scratch; the _host form stages the record stream (its size) and 9 bytes per record.
+ * The _host form reads the records from and writes the verdicts to host memory.  Synchronous. */
+int qm_bam_mark_duplicates(qm_ctx *ctx, const uint8_t *d_bytes, const int64_t *d_rec_off, int64_t n_recs, uint8_t *d_dup, int64_t *h_n_units,
+                           int64_t *h_n_dup_units, void *stream);
+int qm_bam_mark_duplicates_host(qm_ctx *ctx, const uint8_t *h_bytes, int64_t n_bytes, const int64_t *h_rec_off, int64_t n_recs, uint8_t *h_dup,
+                                int64_t *h_n_units, int64_t *h_n_dup_units);
+
 /* ---- multi-GPU: the one collective of the path (north_star: "per-GPU int32 count tensors are merged with one NCCL allreduce
  * over NVLink"; SURVEY.md 8b, 8e).  Reads shard by pair index with no data-path exchange; what crosses GPUs is the count
  * tensor (one in-place integer sum per sample: order independent, bit-exact for any number of GPUs) and the 128 bytes of the

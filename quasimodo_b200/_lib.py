@@ -148,6 +148,8 @@ SIGNATURES = {
     "qm_mpileup_text_ranked": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _P, _P, _P]),
     "qm_bam_to_pairs": (C.c_int, [_P, _P, _P, _P, _L, _I, _P, C.c_int, C.c_int, C.POINTER(BamPairs), _P]),
     "qm_bam_to_pairs_host": (C.c_int, [_P, _P, _P, _L, _P, _L, _I, _P, C.c_int, C.c_int, C.POINTER(BamPairs)]),
+    "qm_bam_mark_duplicates": (C.c_int, [_P, _P, _P, _L, _P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P]),
+    "qm_bam_mark_duplicates_host": (C.c_int, [_P, _P, _L, _P, _L, _P, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "qm_pileup_accumulate_masked": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _P, _P, _P, _P]),
     "qm_profile_enable": (C.c_int, [_P, C.c_int]),
     "qm_profile_collect": (C.c_int, [_P, _P, _P]),

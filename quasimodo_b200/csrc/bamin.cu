@@ -15,12 +15,9 @@
 //      depends on the order of the reads in the file, and the cap looks at every read alone.  Its verdict moves to the pair
 //      layout through the permutation.
 #include <cub/device/device_scan.cuh>
-#include "pipeline.cuh"
+#include "bamrec.cuh"
 
 namespace {
-
-__device__ __forceinline__ uint32_t ld_u32(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24; }
-__device__ __forceinline__ uint32_t ld_u16(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8; }
 
 // SAM's 4-bit base codes -> 0..4: '=' and the IUPAC codes are N (htslib seq_nt16_int)
 __constant__ uint8_t kNt16Code[16] = {4, 0, 1, 4, 2, 4, 4, 4, 3, 4, 4, 4, 4, 4, 4, 4};
@@ -41,13 +38,13 @@ __device__ int32_t aux_int(const uint8_t *p, const uint8_t *end, char t0, char t
         int sz = 0;
         switch (ty) {
         case 'A': case 'c': case 'C': sz = 1; v = ty == 'c' ? (int32_t)(int8_t)p[0] : (int32_t)p[0]; break;
-        case 's': case 'S': sz = 2; v = ty == 's' ? (int32_t)(int16_t)ld_u16(p) : (int32_t)ld_u16(p); break;
-        case 'i': case 'I': case 'f': sz = 4; v = (int32_t)ld_u32(p); break;
+        case 's': case 'S': sz = 2; v = ty == 's' ? (int32_t)(int16_t)qm_ld_u16(p) : (int32_t)qm_ld_u16(p); break;
+        case 'i': case 'I': case 'f': sz = 4; v = (int32_t)qm_ld_u32(p); break;
         case 'Z': case 'H': while (p + sz < end && p[sz]) ++sz; ++sz; break;
         case 'B': {
             const char sub = (char)p[0];
             const int es = (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : 4;
-            sz = 5 + es * (int)ld_u32(p + 1);
+            sz = 5 + es * (int)qm_ld_u32(p + 1);
             break;
         }
         default: return 0;                                 // malformed: no tag
@@ -62,7 +59,7 @@ __device__ int32_t aux_int(const uint8_t *p, const uint8_t *end, char t0, char t
 __global__ void __launch_bounds__(128)
 bam_decode_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__ rec_off, int64_t n, int64_t n_rows, int stride,
                   int hash_bits, qm_aln *__restrict__ alns, uint8_t *__restrict__ codes, uint8_t *__restrict__ quals,
-                  int32_t *__restrict__ lens, uint64_t *__restrict__ hash)
+                  int32_t *__restrict__ lens, uint16_t *__restrict__ flags, uint64_t *__restrict__ hash)
 {
     const int lane = threadIdx.x & 31;
     const int64_t f = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
@@ -70,12 +67,12 @@ bam_decode_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__
     uint8_t *c = codes + f * stride, *q = quals + f * stride;
     if (f >= n) {
         for (int i = lane; i < stride; i += 32) { c[i] = 4; q[i] = 0; }
-        if (lane == 0) { qm_aln a; placeholder(a); alns[f] = a; lens[f] = 0; hash[f] = ~0ull; }
+        if (lane == 0) { qm_aln a; placeholder(a); alns[f] = a; lens[f] = 0; flags[f] = 0x4; hash[f] = ~0ull; }
         return;
     }
     const uint8_t *r = bytes + rec_off[f];
-    const int l_name = r[12], n_cig = (int)ld_u16(r + 16);
-    const int flag = (int)ld_u16(r + 18), L = (int)ld_u32(r + 20);
+    const int l_name = r[12], n_cig = (int)qm_ld_u16(r + 16);
+    const int flag = (int)qm_ld_u16(r + 18), L = (int)qm_ld_u32(r + 20);
     const int64_t o_seq = 36 + l_name + 4 * n_cig, o_qual = o_seq + (L + 1) / 2;
     const bool rev = (flag & 0x10) != 0;
     for (int i = lane; i < stride; i += 32) {
@@ -89,13 +86,13 @@ bam_decode_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__
     if (lane != 0) return;
     qm_aln a;
     memset(&a, 0, sizeof a);
-    a.rid = (int32_t)ld_u32(r + 4); a.pos = (int32_t)ld_u32(r + 8);
+    a.rid = (int32_t)qm_ld_u32(r + 4); a.pos = (int32_t)qm_ld_u32(r + 8);
     a.mapq = r[13]; a.flag = (uint16_t)flag;
-    a.mate_rid = (int32_t)ld_u32(r + 24); a.mate_pos = (int32_t)ld_u32(r + 28); a.tlen = (int32_t)ld_u32(r + 32);
+    a.mate_rid = (int32_t)qm_ld_u32(r + 24); a.mate_pos = (int32_t)qm_ld_u32(r + 28); a.tlen = (int32_t)qm_ld_u32(r + 32);
     // CIGAR: '=' and 'X' are M, H is dropped, neighbours of one kind merge (the host refused N, P and more than QM_MAX_CIGAR ops)
     int nc = 0;
     for (int k = 0; k < n_cig; ++k) {
-        const uint32_t w = ld_u32(r + 36 + l_name + 4 * k);
+        const uint32_t w = qm_ld_u32(r + 36 + l_name + 4 * k);
         int op = (int)(w & 0xf);
         const uint32_t len = w >> 4;
         if (op == 5 || len == 0) continue;
@@ -105,19 +102,12 @@ bam_decode_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__
     }
     a.n_cigar = (uint8_t)nc;
     a.qb = 0; a.qe = L;
-    const uint8_t *aux = r + o_qual + L, *end = r + 4 + ld_u32(r);
+    const uint8_t *aux = r + o_qual + L, *end = r + 4 + qm_ld_u32(r);
     a.nm = aux_int(aux, end, 'N', 'M'); a.score = aux_int(aux, end, 'A', 'S'); a.sub = aux_int(aux, end, 'X', 'S');
     alns[f] = a;
     lens[f] = L;
-    uint64_t h = 1469598103934665603ull;                           // FNV-1a over the name without its NUL
-    for (int i = 0; i + 1 < l_name; ++i) { h ^= r[36 + i]; h *= 1099511628211ull; }
-    hash[f] = hash_bits >= 64 ? h : h & ((1ull << hash_bits) - 1);
-}
-
-__device__ __forceinline__ bool pairing_primary(const qm_aln &a)
-{
-    const int m = a.flag & 0xc0;
-    return (m == 0x40 || m == 0x80) && !(a.flag & 0x900);
+    flags[f] = (uint16_t)flag;
+    hash[f] = qm_bam_name_hash(r, hash_bits);
 }
 
 __device__ bool same_name(const uint8_t *bytes, const int64_t *rec_off, int64_t f, int64_t g)
@@ -131,15 +121,15 @@ __device__ bool same_name(const uint8_t *bytes, const int64_t *rec_off, int64_t 
 // step 2: sorted position k (keys[k] = hash, perm[k] = file index).  partner[f] = file index of f's mate, -1 = f stays alone:
 // f and g pair iff they are the only two primary records of their name and one is the first, the other the last segment
 __global__ void __launch_bounds__(256)
-bam_pair_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__ rec_off, const qm_aln *__restrict__ alns,
+bam_pair_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__ rec_off, const uint16_t *__restrict__ flags,
                 const uint64_t *__restrict__ keys, const uint32_t *__restrict__ perm, int64_t n, int32_t *__restrict__ partner)
 {
     const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (k >= n) return;
     const int64_t f = perm[k];
     partner[f] = -1;
-    const qm_aln &a = alns[f];
-    if (!pairing_primary(a)) return;
+    const uint32_t fl = flags[f];
+    if (!qm_bam_pairing_primary(fl)) return;
     const uint64_t h = keys[k];
     int64_t lo = k, hi = k + 1;
     while (lo > 0 && keys[lo - 1] == h) --lo;
@@ -149,10 +139,10 @@ bam_pair_kernel(const uint8_t *__restrict__ bytes, const int64_t *__restrict__ r
     for (int64_t j = lo; j < hi && found < 2; ++j) {
         if (j == k) continue;
         const int64_t g = perm[j];
-        if (!pairing_primary(alns[g]) || !same_name(bytes, rec_off, f, g)) continue;
+        if (!qm_bam_pairing_primary(flags[g]) || !same_name(bytes, rec_off, f, g)) continue;
         mate = g; ++found;
     }
-    if (found == 1 && (alns[mate].flag & 0xc0) != (a.flag & 0xc0)) partner[f] = (int32_t)mate;
+    if (found == 1 && (flags[mate] & 0xc0) != (fl & 0xc0)) partner[f] = (int32_t)mate;
 }
 
 // a row opens a pair when it stays alone or comes before its mate in the file
@@ -213,6 +203,13 @@ inline size_t al256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 }  // namespace
 
+cudaError_t qm_bam_pair_launch(const uint8_t *d_bytes, const int64_t *d_rec_off, const uint16_t *d_flags, const uint64_t *d_keys,
+                               const uint32_t *d_perm, int64_t n, int32_t *d_partner, cudaStream_t st)
+{
+    bam_pair_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_bytes, d_rec_off, d_flags, d_keys, d_perm, n, d_partner);
+    return cudaGetLastError();
+}
+
 extern "C" {
 
 // the body of qm_bam_to_pairs with the name hash cut to hash_bits bits (1..64): the tests pair through colliding hashes with it
@@ -237,7 +234,8 @@ int qm_bam_to_pairs_hashbits(qm_ctx *ctx, const qm_index *idx, const uint8_t *d_
     const size_t o_alns = 0, o_codes = al256((size_t)nr * sizeof(qm_aln)), o_quals = o_codes + al256(nr * sb), o_lens = o_quals + al256(nr * sb);
     const size_t o_hash = o_lens + al256((size_t)nr * 4), o_perm = o_hash + al256((size_t)nr * 8), o_partner = o_perm + al256((size_t)nr * 4);
     const size_t o_lead = o_partner + al256((size_t)nr * 4), o_pidx = o_lead + al256((size_t)(n + 1) * 4);
-    const size_t o_frow = o_pidx + al256((size_t)(n + 1) * 4), o_fdrop = o_frow + al256((size_t)n * 8), o_cub = o_fdrop + al256((size_t)nr);
+    const size_t o_frow = o_pidx + al256((size_t)(n + 1) * 4), o_fdrop = o_frow + al256((size_t)n * 8), o_flags = o_fdrop + al256((size_t)nr);
+    const size_t o_cub = o_flags + al256((size_t)nr * 2);
     void *p = nullptr;
     int rc = qm_scratch_reserve(ctx, 38, o_cub + al256(cub_bytes), &p);
     if (rc) return rc;
@@ -246,15 +244,16 @@ int qm_bam_to_pairs_hashbits(qm_ctx *ctx, const qm_index *idx, const uint8_t *d_
     uint8_t *f_codes = (uint8_t *)(b + o_codes), *f_quals = (uint8_t *)(b + o_quals), *f_drop = (uint8_t *)(b + o_fdrop);
     int32_t *f_lens = (int32_t *)(b + o_lens), *partner = (int32_t *)(b + o_partner), *lead = (int32_t *)(b + o_lead), *pidx = (int32_t *)(b + o_pidx);
     uint64_t *hash = (uint64_t *)(b + o_hash);
+    uint16_t *flags = (uint16_t *)(b + o_flags);
     uint32_t *perm = (uint32_t *)(b + o_perm);
     int64_t *file_row = (int64_t *)(b + o_frow);
     const int sp = qm_prof_begin(ctx, QM_ST_OTHER, st);
-    bam_decode_kernel<<<(unsigned)((nr * 32 + 127) / 128), 128, 0, st>>>(d_bytes, d_rec_off, n, nr, stride, hash_bits, f_alns, f_codes, f_quals, f_lens, hash);
+    bam_decode_kernel<<<(unsigned)((nr * 32 + 127) / 128), 128, 0, st>>>(d_bytes, d_rec_off, n, nr, stride, hash_bits, f_alns, f_codes, f_quals, f_lens, flags, hash);
     QM_CUDA(ctx, cudaGetLastError());
     iota_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(perm, n);
     rc = qm_sort_pairs(ctx, hash, perm, n, hash_bits, st);          // stable: a run of equal hashes keeps file order
     if (rc) return rc;
-    bam_pair_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_bytes, d_rec_off, f_alns, hash, perm, n, partner);
+    QM_CUDA(ctx, qm_bam_pair_launch(d_bytes, d_rec_off, flags, hash, perm, n, partner, st));
     bam_leader_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partner, n, lead);
     QM_CUDA(ctx, cudaMemsetAsync(lead + n, 0, 4, st));
     QM_CUDA(ctx, cub::DeviceScan::ExclusiveSum(b + o_cub, cub_bytes, lead, pidx, (int)(n + 1), st));

@@ -24,8 +24,9 @@ struct qm_ctx {
     std::string err;
     // scratch arenas grown on demand (never shrunk); index = purpose.  32-36: the tuples of duplicate marking and the depth cap
     // (dedup.cu, depthcap.cu, sort.cu, sample.cu);
-    // 37-39: BAM records in (bamin.cu: staged record stream, file-order rows and pairing state, pair layout)
-    qm_scratch scratch[40];
+    // 37-39: BAM records in (bamin.cu: staged record stream, file-order rows and pairing state, pair layout);
+    // 40-41: duplicate marking of a BAM (bamdup.cu: staged record stream and verdicts, per-record state and tuples)
+    qm_scratch scratch[42];
     cudaStream_t own_stream = nullptr, copy_stream = nullptr;
     // side streams: the independent per-class extension kernels of one round run concurrently (fork/join by events)
     cudaStream_t side[12] = {};

@@ -16,8 +16,8 @@
 namespace {
 
 constexpr uint64_t kNoKey = ~0ull;
-constexpr uint32_t kNoEnd = 0xffffffffu;                 // end code of a missing end in qm_dup_key
-constexpr int kCoordBias = 4096;                 // unclipped coordinates can be negative (clipped bases before the contig)
+constexpr uint32_t kNoEnd = QM_DUP_NO_END;
+constexpr int kCoordBias = QM_DUP_COORD_BIAS;
 
 // {contig, unclipped 5' coordinate} of a placed record as a 30-bit code, and its strand
 // (26 bits of coordinate, 4 of contig: a contig of >= 2^26 - 4096 bases or a 17th contig does not fit; *bad is raised then
@@ -59,26 +59,10 @@ dup_keys_kernel(const qm_aln *__restrict__ alns, const uint8_t *__restrict__ qua
         for (int j = 0; j < L; ++j) { const int v = q[j]; s += v >= 15 ? v : 0; }
         sc[e] = s;
     }
-    qm_dup_key t;
-    t.pair_id = pair_id0 + i;
-    t.end0 = t.end1 = kNoEnd;
-    t.pad = 0;
-    int bad = 0;
-    if (pa && pb) {
-        int ra, rb;
-        uint32_t ca = end_code(a, &ra, &bad), cb = end_code(b, &rb, &bad);
-        if (cb < ca || (cb == ca && rb < ra)) { const uint32_t u = ca; ca = cb; cb = u; const int v = ra; ra = rb; rb = v; }
-        t.key = ((uint64_t)ca << 32) | ((uint64_t)cb << 2) | (uint64_t)(ra << 1 | rb);
-        t.end0 = ca << 1 | (uint32_t)ra; t.end1 = cb << 1 | (uint32_t)rb;
-        t.score = sc[0] + sc[1];
-    } else {
-        int r;
-        const uint32_t c = end_code(pa ? a : b, &r, &bad);
-        t.key = (1ull << 63) | ((uint64_t)c << 1) | (uint64_t)r;
-        t.score = pa ? sc[0] : sc[1];
-    }
+    int bad = 0, ra = 0, rb = 0;
+    const uint32_t ca = pa ? end_code(a, &ra, &bad) : 0, cb = pb ? end_code(b, &rb, &bad) : 0;
     if (bad) atomicAdd(cnt + 1, 1ull);
-    out[atomicAdd(cnt, 1ull)] = t;
+    out[atomicAdd(cnt, 1ull)] = qm_dup_tuple(pair_id0 + i, pa, ca << 1 | (uint32_t)ra, sc[0], pb, cb << 1 | (uint32_t)rb, sc[1]);
 }
 
 // the union in pair-id order: ids[] sorted, perm[] their input positions.  Scatters key, score and end codes into sorted order and
@@ -187,17 +171,17 @@ int qm_dup_keys(qm_ctx *ctx, int n_chunks, const qm_aln *const *d_alns, const ui
     return QM_OK;
 }
 
-// the decision over the union of every rank's tuples, applied to this rank's chunks.  Synchronous.
-int qm_mark_duplicates_keys(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all, int n_chunks, qm_aln *const *d_alns,
-                            const int64_t *n_pairs, const int64_t *pair_id0, int64_t *h_n_dup_all, void *stream)
+}  // extern "C"
+
+// the decision over a union of tuples: *d_ids = the pair ids sorted, (*d_dup)[k] = 1 when pair (*d_ids)[k] is a duplicate (scratch 15,
+// valid until the next decision on the context).  A repeated id is QM_EINVAL.  Synchronous.
+int qm_dup_decide(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all, const uint64_t **d_ids, const uint8_t **d_dup, int64_t *h_n_dup,
+                  cudaStream_t st)
 {
-    if (!ctx || n_all < 0 || (n_all > 0 && !d_all) || n_chunks < 0 || (n_chunks > 0 && (!d_alns || !n_pairs || !pair_id0))) return QM_EINVAL;
-    for (int c = 0; c < n_chunks; ++c) if (n_pairs[c] < 0 || pair_id0[c] < 0) return QM_EINVAL;
-    if (h_n_dup_all) *h_n_dup_all = 0;
+    *d_ids = nullptr; *d_dup = nullptr; *h_n_dup = 0;
     if (n_all == 0) return QM_OK;
     if (2 * n_all > 0xffffffffll) return qm_fail(ctx, QM_ELIMIT, "qm_mark_duplicates: more than 2^31 pairs");
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = (cudaStream_t)stream;
     const int64_t N = n_all;
     // scratch 15: ids | id perm | keys | ends | scores | perm | end perm | dup flags | counters
     auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
@@ -231,12 +215,33 @@ int qm_mark_duplicates_keys(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all,
     if (rc) return rc;
     dup_mark_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(keys, perm, scores, N, ends, 2 * N, dup);
     dup_count_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(dup, N, cnt);
-    for (int c = 0; c < n_chunks; ++c)
-        if (n_pairs[c]) dup_apply_kernel<<<(unsigned)((n_pairs[c] + 127) / 128), 128, 0, st>>>(d_alns[c], n_pairs[c], pair_id0[c], ids, N, dup);
     QM_CUDA(ctx, cudaGetLastError());
     QM_CUDA(ctx, cudaMemcpyAsync(h, cnt, 8, cudaMemcpyDeviceToHost, st));
     QM_CUDA(ctx, cudaStreamSynchronize(st));
-    if (h_n_dup_all) *h_n_dup_all = (int64_t)h[0];
+    *d_ids = ids; *d_dup = dup; *h_n_dup = (int64_t)h[0];
+    return QM_OK;
+}
+
+extern "C" {
+
+// the decision over the union of every rank's tuples, applied to this rank's chunks.  Synchronous.
+int qm_mark_duplicates_keys(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all, int n_chunks, qm_aln *const *d_alns,
+                            const int64_t *n_pairs, const int64_t *pair_id0, int64_t *h_n_dup_all, void *stream)
+{
+    if (!ctx || n_all < 0 || (n_all > 0 && !d_all) || n_chunks < 0 || (n_chunks > 0 && (!d_alns || !n_pairs || !pair_id0))) return QM_EINVAL;
+    for (int c = 0; c < n_chunks; ++c) if (n_pairs[c] < 0 || pair_id0[c] < 0) return QM_EINVAL;
+    if (h_n_dup_all) *h_n_dup_all = 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    const uint64_t *ids = nullptr;
+    const uint8_t *dup = nullptr;
+    int64_t n_dup = 0;
+    const int rc = qm_dup_decide(ctx, d_all, n_all, &ids, &dup, &n_dup, st);
+    if (rc || n_all == 0) return rc;
+    for (int c = 0; c < n_chunks; ++c)
+        if (n_pairs[c]) dup_apply_kernel<<<(unsigned)((n_pairs[c] + 127) / 128), 128, 0, st>>>(d_alns[c], n_pairs[c], pair_id0[c], ids, n_all, dup);
+    QM_CUDA(ctx, cudaGetLastError());
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    if (h_n_dup_all) *h_n_dup_all = n_dup;
     return QM_OK;
 }
 

@@ -36,6 +36,11 @@
 //          the same defaults (BAQ off, no depth cap); the BAM of `sample` read back gives `sample`'s bytes.  The file is inflated
 //          and validated on the host before a CUDA context exists (a bad file exits 2 with or without a GPU); the records are
 //          decoded and paired on the device (qm_bam_to_pairs); the depth cap follows the file's order of the reads.
+//   qm_driver rmdup    --bam IN.bam --rmdup-bam OUT.bam [--metrics FILE] [--sample LIB] [--gpu I] [-t THREADS] [--stage-ms 1]
+//        = rules/rmdup.smk:13-16 (`picard MarkDuplicates REMOVE_DUPLICATES=true` on {sample}.{ref_name}.bam): the records of an
+//          existing coordinate-sorted BAM without its duplicates, byte for byte (0x400 cleared), the input's header plus one @PG
+//          line, the .bai and the duplication metrics.  Inflated and validated on the host before a CUDA context exists; the
+//          decision runs on the device (qm_bam_mark_duplicates), ties going to the file order of the sorted BAM as in picard
 //   qm_driver bam-from-records --ref .. --r1 .. --r2 .. --alns ALNS.bin [--perm PERM.bin] --bam OUT.bam
 //        = the BAM/BAI writer alone on given qm_aln records (test entry; with --perm no GPU is touched)
 //   qm_driver fastq-check --r1 .. --r2 .. [-t THREADS]
@@ -1066,6 +1071,17 @@ int sort_key_bits(const Genome &g, int &pos_bits)
 
 template <class T> std::vector<T> read_binary(const std::string &path);
 
+// the duplication metrics of `sample --rmdup 1 --metrics` and `rmdup --metrics` (picard's file, reduced to what is decided here)
+void write_dup_metrics(const std::string &path, const std::string &library, int64_t n_examined, int64_t n_dup)
+{
+    FILE *fm = fopen(path.c_str(), "w");
+    if (!fm) die(2, "cannot create %s", path.c_str());
+    fprintf(fm, "## METRICS CLASS\tquasimodo_b200.DuplicationMetrics\nLIBRARY\tREAD_PAIRS_EXAMINED\tREAD_PAIR_DUPLICATES\tPERCENT_DUPLICATION\n"
+                "%s\t%lld\t%lld\t%.6f\n", library.c_str(), (long long)n_examined, (long long)n_dup,
+            n_examined ? (double)n_dup / (double)n_examined : 0.0);
+    fclose(fm);
+}
+
 // wall clock of the run's phases, one line on stderr at the end (where a sample's file-level time goes)
 struct PhaseClock {
     std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now(), last = t0;
@@ -1397,14 +1413,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             for (size_t i = 0; i < bp.size(); ++i)
                 memcpy(batches[i].alns, all[(size_t)src[i].first].data() + src[i].second, (size_t)2 * bp[i] * sizeof(qm_aln));
         }
-        if (!metrics.empty()) {
-            FILE *fm = fopen(metrics.c_str(), "w");
-            if (!fm) die(2, "cannot create %s", metrics.c_str());
-            fprintf(fm, "## METRICS CLASS\tquasimodo_b200.DuplicationMetrics\nLIBRARY\tREAD_PAIRS_EXAMINED\tREAD_PAIR_DUPLICATES\tPERCENT_DUPLICATION\n"
-                        "%s\t%lld\t%lld\t%.6f\n", a.get("sample", "sample").c_str(), (long long)n_pairs, (long long)n_dup,
-                    n_pairs ? (double)n_dup / (double)n_pairs : 0.0);
-            fclose(fm);
-        }
+        if (!metrics.empty()) write_dup_metrics(metrics, a.get("sample", "sample"), n_pairs, n_dup);
     }
 
     pc.mark("merge / deferred counting");
@@ -1547,6 +1556,8 @@ int cmd_bam_from_records(const Args &a, const std::string &cmdline)
 
 
 // ------------------------------------------------------------------------------------------------
+constexpr int QM_DUP_COORD_BIAS = 4096;          // the end code's coordinate bias (qm_bam_mark_duplicates: -4095 .. 2^26 - 4096)
+
 // BAM reader (`pileup`): the input of the reference's rules `mpileup` and `bcftools` (rules/vcfcall.smk:39,115 read
 // {sample}.{ref_name}.rmdup.bam).  Everything here runs before a CUDA context exists, so a bad file fails the same way with
 // or without a GPU.
@@ -1799,6 +1810,219 @@ int cmd_pileup(const Args &a)
     pc.report();
     return 0;
 }
+
+// what `rmdup`'s validation walk leaves: the header and the offset of every record in file order
+struct DupInput {
+    std::string text;                          // header text, trailing NULs dropped
+    size_t refs_begin = 0, refs_end = 0;       // the binary reference list (n_ref and its entries) in the stream
+    Genome g;                                  // contig names and lengths (no sequence): what the .bai needs
+    std::vector<int64_t> off;
+    int64_t n_primary = 0;                     // records without 0x100 / 0x800
+    std::string library;                       // the LB of the @RG lines, empty without one
+};
+
+// {reference span (M D N = X), clipped bases (S H) before the first and after the last other operation} of a CIGAR
+inline void cigar_ends(const uint8_t *cig, size_t n_cig, int64_t &span, int64_t &lead, int64_t &trail)
+{
+    span = lead = trail = 0;
+    size_t first = n_cig, last = 0;
+    for (size_t k = 0; k < n_cig; ++k) {
+        const uint32_t w = le32(cig + 4 * k), op = w & 0xf;
+        if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) span += w >> 4;
+        if (op != 4 && op != 5) { if (first == n_cig) first = k; last = k; }
+    }
+    for (size_t k = 0; k < n_cig; ++k) {
+        if (k < first) lead += le32(cig + 4 * k) >> 4;
+        else if (k > last) trail += le32(cig + 4 * k) >> 4;
+    }
+}
+
+// The header: magic, the @SQ limits of the 30-bit end code, one library at most.  Then one walk over the records: well-formed,
+// contig ids inside the header, CIGAR operations <= 8, coordinate order with the records without a contig at the end, and an
+// unclipped 5' coordinate the end code holds on every placed record.  N and P operations, long reads, many CIGAR operations and a
+// missing SEQ or QUAL are fine.  Every failure names the read or the limit and exits 2.
+DupInput scan_bam_dup(const std::string &path, const std::vector<uint8_t> &d)
+{
+    const char *fn = path.c_str();
+    DupInput in;
+    if (d.size() < 12 || memcmp(d.data(), "BAM\1", 4) != 0) die(2, "%s: bad BAM magic: not a BAM file", fn);
+    const size_t l_text = le32(d.data() + 4);
+    if (8 + l_text + 4 > d.size()) die(2, "%s: truncated BAM header", fn);
+    in.text.assign((const char *)d.data() + 8, l_text);
+    while (!in.text.empty() && in.text.back() == '\0') in.text.pop_back();
+    size_t p = 8 + l_text;
+    in.refs_begin = p;
+    const uint32_t n_ref = le32(d.data() + p);
+    p += 4;
+    for (uint32_t i = 0; i < n_ref; ++i) {
+        if (p + 4 > d.size()) die(2, "%s: truncated BAM header", fn);
+        const size_t ln = le32(d.data() + p);
+        if (ln < 1 || p + 8 + ln > d.size()) die(2, "%s: truncated BAM header", fn);
+        in.g.names.emplace_back((const char *)d.data() + p + 4, ln - 1);
+        in.g.lens.push_back((int64_t)le32(d.data() + p + 4 + ln));
+        p += 8 + ln;
+    }
+    in.refs_end = p;
+    if (n_ref > QM_MAX_CONTIGS) die(2, "%s: the header lists %u contigs (@SQ): duplicate marking supports at most %d", fn, n_ref, QM_MAX_CONTIGS);
+    for (size_t i = 0; i < in.g.names.size(); ++i)
+        if (in.g.lens[i] >= (1 << 26) - QM_DUP_COORD_BIAS)
+            die(2, "%s: @SQ %s has %lld bp: duplicate marking supports contigs under 2^26 - 4096 bases", fn, in.g.names[i].c_str(), (long long)in.g.lens[i]);
+    std::vector<std::string> libs;
+    for (size_t b = 0; b < in.text.size();) {
+        size_t e = in.text.find('\n', b);
+        if (e == std::string::npos) e = in.text.size();
+        const std::string ln = in.text.substr(b, e - b);
+        if (ln.compare(0, 4, "@RG\t") == 0) {
+            const size_t k = ln.find("\tLB:");
+            if (k != std::string::npos) {
+                const std::string lb = ln.substr(k + 4, ln.find('\t', k + 4) - (k + 4));
+                if (std::find(libs.begin(), libs.end(), lb) == libs.end()) libs.push_back(lb);
+            }
+        }
+        b = e + 1;
+    }
+    if (libs.size() > 1) die(2, "%s: the @RG lines name %zu libraries (LB): duplicate marking of one library per file is supported", fn, libs.size());
+    if (!libs.empty()) in.library = libs[0];
+    // the record offsets (a serial chain of block_size fields), contig ids and the coordinate order
+    auto rname = [](const uint8_t *r) { return std::string((const char *)r + 36, r[12] ? r[12] - 1 : 0); };
+    int32_t last_tid = -1, last_pos = -1;
+    bool no_contig_seen = false;
+    for (; p < d.size();) {
+        if (p + 36 > d.size()) die(2, "%s: truncated record at byte %zu of the BAM stream", fn, p);
+        const uint8_t *r = d.data() + p;
+        const size_t bs = le32(r);
+        if (bs < 32 || p + 4 + bs > d.size() || 32 + (size_t)r[12] > bs) die(2, "%s: malformed or truncated record at byte %zu of the BAM stream", fn, p);
+        const int32_t tid = (int32_t)le32(r + 4), pos = (int32_t)le32(r + 8);
+        if (tid < -1 || tid >= (int32_t)n_ref) die(2, "%s: read %s: contig id %d is not in the header", fn, rname(r).c_str(), tid);
+        if (tid >= 0) {
+            if (no_contig_seen) die(2, "%s: the file is not coordinate-sorted: read %s on %s comes after records without a contig", fn, rname(r).c_str(), in.g.names[(size_t)tid].c_str());
+            if (tid < last_tid || (tid == last_tid && pos < last_pos))
+                die(2, "%s: the file is not coordinate-sorted: read %s at %s:%d comes after %s:%d", fn, rname(r).c_str(), in.g.names[(size_t)tid].c_str(), pos + 1,
+                    in.g.names[(size_t)last_tid].c_str(), last_pos + 1);
+            last_tid = tid; last_pos = pos;
+        } else no_contig_seen = true;
+        in.off.push_back((int64_t)p);
+        p += 4 + bs;
+    }
+    // the per-record checks, on the -t threads; the first failure in file order is reported
+    std::vector<std::pair<size_t, std::string>> bad;
+    std::atomic<int64_t> n_primary{0};
+    std::mutex mu;
+    parallel_ranges(in.off.size(), [&](size_t b, size_t e) {
+        int64_t np = 0;
+        for (size_t i = b; i < e; ++i) {
+            const uint8_t *r = d.data() + in.off[i];
+            const size_t bs = le32(r), l_name = r[12], n_cig = le16(r + 16);
+            const int flag = (int)le16(r + 18);
+            const int32_t tid = (int32_t)le32(r + 4), pos = (int32_t)le32(r + 8), l_seq = (int32_t)le32(r + 20);
+            auto fail = [&](const std::string &why) { std::lock_guard<std::mutex> lk(mu); bad.emplace_back(i, "read " + rname(r) + ": " + why); };
+            if (l_name < 1 || l_seq < 0 || 36 + l_name + 4 * n_cig + (size_t)(l_seq + 1) / 2 + (size_t)l_seq > 4 + bs) { fail("malformed record"); continue; }
+            const uint8_t *cig = r + 36 + l_name;
+            bool ok = true;
+            for (size_t k = 0; k < n_cig && ok; ++k)
+                if ((le32(cig + 4 * k) & 0xf) > 8) { fail("invalid CIGAR operation " + std::to_string(le32(cig + 4 * k) & 0xf)); ok = false; }
+            if (!ok) continue;
+            if (!(flag & 0x900)) ++np;
+            if ((flag & 0x4) || tid < 0 || n_cig == 0) continue;
+            int64_t span, lead, trail;
+            cigar_ends(cig, n_cig, span, lead, trail);
+            const int64_t coord = (flag & 0x10) ? pos + span - 1 + trail : pos - lead;
+            if (coord + QM_DUP_COORD_BIAS < 0 || coord + QM_DUP_COORD_BIAS >= (1 << 26))
+                fail("unclipped 5' coordinate " + std::to_string(coord + 1) + " lies outside what the end code holds (-4095 .. 2^26 - 4096)");
+        }
+        n_primary += np;
+    });
+    if (!bad.empty()) {
+        auto it = std::min_element(bad.begin(), bad.end(), [](const auto &x, const auto &y) { return x.first < y.first; });
+        die(2, "%s: %s", fn, it->second.c_str());
+    }
+    in.n_primary = n_primary;
+    return in;
+}
+
+// duplicate marking of an existing coordinate-sorted BAM: rule `rmdup` (picard MarkDuplicates REMOVE_DUPLICATES=true) one for one
+int cmd_rmdup(const Args &a, const std::string &cmdline)
+{
+    PhaseClock pc;
+    require_known(a, "rmdup", {"bam", "rmdup-bam", "metrics", "sample", "gpu", "t", "threads", "stage-ms"});
+    if (!a.has("bam") || !a.has("rmdup-bam")) die(1, "--bam and --rmdup-bam are required");
+    const int threads = std::max(1, atoi(a.get("t", a.get("threads", "4")).c_str()));
+    g_threads = threads;
+    const std::string path = a.get("bam"), out = a.get("rmdup-bam");
+    const std::vector<uint8_t> data = inflate_bgzf(path);
+    pc.mark("BGZF inflate");
+    const DupInput in = scan_bam_dup(path, data);
+    pc.mark("validation walk");
+    const int64_t n = (int64_t)in.off.size();
+    fprintf(stderr, "[qm_driver] %s: %lld records\n", path.c_str(), (long long)n);
+    Lib L;
+    const int dev = atoi(a.get("gpu", "0").c_str());
+    const int rc = qm_ctx_create(dev, &L.ctx);
+    if (rc != QM_OK) die(3, "qm_ctx_create(%d) failed (%d): no usable B200 (there is no CPU fallback)", dev, rc);
+    const bool stage_ms = atoi(a.get("stage-ms", "0").c_str()) != 0;
+    if (stage_ms) L.check(qm_profile_enable(L.ctx, 1), "qm_profile_enable");
+    pc.mark("context");
+    std::vector<uint8_t> dup((size_t)n);
+    int64_t n_units = 0, n_dup = 0;
+    L.check(qm_bam_mark_duplicates_host(L.ctx, data.data(), (int64_t)data.size(), in.off.data(), n, dup.data(), &n_units, &n_dup),
+            "qm_bam_mark_duplicates_host");
+    pc.mark("H2D + decision");
+    int64_t n_removed = 0;
+    for (uint8_t v : dup) n_removed += v;
+    fprintf(stderr, "[qm_driver] rmdup: %lld of %lld units are duplicates (%lld lone records among the units); %lld records removed\n",
+            (long long)n_dup, (long long)n_units, (long long)(2 * n_units - in.n_primary), (long long)n_removed);
+    // the input's header plus one @PG line (an ID of its own, PP = the last @PG), then the kept records byte for byte with 0x400 cleared
+    std::vector<std::string> pg_ids;
+    for (size_t b = 0; b < in.text.size();) {
+        size_t e = in.text.find('\n', b);
+        if (e == std::string::npos) e = in.text.size();
+        const std::string ln = in.text.substr(b, e - b);
+        const size_t k = ln.find("\tID:");
+        if (ln.compare(0, 4, "@PG\t") == 0 && k != std::string::npos) pg_ids.push_back(ln.substr(k + 4, ln.find('\t', k + 4) - (k + 4)));
+        b = e + 1;
+    }
+    std::string id = "quasimodo_b200.rmdup";
+    for (int i = 1; std::find(pg_ids.begin(), pg_ids.end(), id) != pg_ids.end(); ++i) id = "quasimodo_b200.rmdup." + std::to_string(i);
+    std::string text = in.text;
+    if (!text.empty() && text.back() != '\n') text += '\n';
+    text += "@PG\tID:" + id + "\tPN:quasimodo_b200" + (pg_ids.empty() ? "" : "\tPP:" + pg_ids.back()) + "\tVN:0.1\tCL:" + cmdline + "\n";
+    BgzfWriter bw(out, threads, 1);
+    std::vector<uint8_t> hdr = {'B', 'A', 'M', 1};
+    put32(hdr, (uint32_t)text.size());
+    hdr.insert(hdr.end(), text.begin(), text.end());
+    hdr.insert(hdr.end(), data.begin() + (ptrdiff_t)in.refs_begin, data.begin() + (ptrdiff_t)in.refs_end);
+    bw.write(hdr.data(), hdr.size());
+    bw.close_block();                                  // records start on a block boundary, as samtools writes them
+    std::vector<BamIndexEntry> ents;
+    ents.reserve((size_t)(n - n_removed));
+    for (int64_t i = 0; i < n; ++i) {
+        if (dup[(size_t)i]) continue;
+        const uint8_t *r = data.data() + in.off[(size_t)i];
+        const size_t bs = le32(r);
+        const uint16_t flag = (uint16_t)(le16(r + 18) & ~0x400u);
+        BamIndexEntry ie;
+        ie.rid = (int32_t)le32(r + 4); ie.beg = (int32_t)le32(r + 8); ie.mapped = !(flag & 0x4);
+        int64_t span = 0, lead, trail;
+        if (ie.mapped) cigar_ends(r + 36 + r[12], le16(r + 16), span, lead, trail);
+        ie.end = (int32_t)(ie.beg + (span > 0 ? span : 1));
+        ie.bin = (uint16_t)reg2bin(ie.beg, ie.end);
+        bw.reserve(bs + 4);
+        bw.tell(ie.blk0, ie.off0);
+        bw.write(r, 18);
+        bw.write(&flag, 2);
+        bw.write(r + 20, bs + 4 - 20);
+        bw.tell(ie.blk1, ie.off1);
+        ents.push_back(ie);
+    }
+    bw.finish();
+    write_bai(out + ".bai", in.g, ents, bw);
+    pc.mark("BAM + BAI");
+    if (a.has("metrics")) write_dup_metrics(a.get("metrics"), a.get("sample", in.library.empty() ? "sample" : in.library), n_units, n_dup);
+    if (stage_ms) print_stage_ms(L, dev);
+    qm_ctx_destroy(L.ctx);
+    pc.report();
+    return 0;
+}
 }  // namespace
 
 // --benchmark FILE (any command): the job's resources in the shape of a Snakemake `benchmark:` file (one header line, one row:
@@ -1841,7 +2065,7 @@ int main(int argc, char **argv)
 {
     g_benchmark_t0 = std::chrono::steady_clock::now();
     g_benchmark_cpu0 = clock();
-    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
+    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|rmdup|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
     std::string cmdline;
     for (int i = 0; i < argc; ++i) { if (i) cmdline += ' '; cmdline += argv[i]; }
     const std::string cmd = argv[1];
@@ -1855,6 +2079,7 @@ int main(int argc, char **argv)
     if (cmd == "decontam") return cmd_sample(a, cmdline, true);
     if (cmd == "bam-from-records") return cmd_bam_from_records(a, cmdline);
     if (cmd == "pileup") return cmd_pileup(a);
+    if (cmd == "rmdup") return cmd_rmdup(a, cmdline);
     if (cmd == "fastq-check") {                        // host only: parse the two mate files as `sample` would, report what is there
         require_known(a, "fastq-check", {"r1", "r2", "t", "threads"});
         if (!a.has("r1") || !a.has("r2")) die(1, "--r1 --r2 are required");

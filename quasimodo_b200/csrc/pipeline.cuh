@@ -196,10 +196,41 @@ int qm_ext_launch_classes(qm_ctx *ctx, const ExtParams &P, const IndexView &V, c
 // QM_EINVAL on a negative id.  Synchronous.
 int qm_sort_ids(qm_ctx *ctx, uint64_t *d_ids, uint32_t *d_perm, int64_t n, const char *who, cudaStream_t st);
 
+// duplicate marking (dedup.cu, bamdup.cu).  An end is {contig, unclipped 5' coordinate + QM_DUP_COORD_BIAS} as a 30-bit code
+// (4 bits of contig, 26 of coordinate; the bias admits clipped bases before the contig's start), times 2, plus 1 for the reverse
+// strand; QM_DUP_NO_END = no placed end.  qm_dup_tuple: the tuple of a unit with placed ends e0 (score s0) and / or e1 (score s1)
+#define QM_DUP_NO_END 0xffffffffu
+#define QM_DUP_COORD_BIAS 4096
+__device__ __forceinline__ qm_dup_key qm_dup_tuple(int64_t id, bool p0, uint32_t e0, int s0, bool p1, uint32_t e1, int s1)
+{
+    qm_dup_key t;
+    t.pair_id = id;
+    t.end0 = t.end1 = QM_DUP_NO_END;
+    t.pad = 0;
+    if (p0 && p1) {
+        if (e1 < e0) { const uint32_t u = e0; e0 = e1; e1 = u; }
+        t.key = ((uint64_t)(e0 >> 1) << 32) | ((uint64_t)(e1 >> 1) << 2) | (uint64_t)((e0 & 1) << 1 | (e1 & 1));
+        t.end0 = e0; t.end1 = e1;
+        t.score = s0 + s1;
+    } else {
+        t.key = (1ull << 63) | (uint64_t)(p0 ? e0 : e1);
+        t.score = p0 ? s0 : s1;
+    }
+    return t;
+}
+// dedup.cu: the decision over a union of tuples.  *d_ids = the ids sorted, (*d_dup)[k] = 1 when the unit of id (*d_ids)[k] is a
+// duplicate (scratch 15, valid until the next decision on the context); a repeated id is QM_EINVAL.  Synchronous.
+int qm_dup_decide(qm_ctx *ctx, const qm_dup_key *d_all, int64_t n_all, const uint64_t **d_ids, const uint8_t **d_dup, int64_t *h_n_dup,
+                  cudaStream_t st);
+
 // bamin.cu: qm_bam_to_pairs with the name hash cut to hash_bits bits (tests: pairing through colliding hashes)
 extern "C" int qm_bam_to_pairs_hashbits(qm_ctx *ctx, const qm_index *idx, const uint8_t *d_bytes, const int64_t *d_rec_off, int64_t n_recs,
                                         int32_t stride, const qm_pileup_opt *po, int baq, int max_depth, int hash_bits, qm_bam_pairs *out,
                                         void *stream);
+
+// bamdup.cu: qm_bam_mark_duplicates with the name hash cut to hash_bits bits (tests: pairing through colliding hashes)
+extern "C" int qm_bam_mark_duplicates_hashbits(qm_ctx *ctx, const uint8_t *d_bytes, const int64_t *d_rec_off, int64_t n_recs, int hash_bits,
+                                               uint8_t *d_dup, int64_t *h_n_units, int64_t *h_n_dup_units, void *stream);
 
 // sample.cu: packed reads (2 bits per base + N flags) -> one code byte per base, rows [0, n_reads)
 cudaError_t qm_unpack_reads_launch(const uint8_t *d_bases2, const uint8_t *d_nmask, int stride, int stride_p, int stride_m, int64_t n_reads,

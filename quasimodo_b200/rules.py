@@ -3,7 +3,8 @@ paths of rules `bwa` (rules/bwa.smk:1-19), `rmdup` (rules/rmdup.smk:1-18), `mpil
 (rules/vcfcall.smk:101-120), and the ONE `qm_driver sample` invocation that produces all of them.  Snakemake deletes a job
 whose declared output is missing, so tests/test_rules_cpu.py checks these tables against the reference's rule files and
 tests/test_driver_gpu.py checks that the command really writes every path.  pileup_commands gives rules `mpileup` and
-`bcftools` one `qm_driver pileup` job each, on the .rmdup.bam a separate alignment step left."""
+`bcftools` one `qm_driver pileup` job each, on the .rmdup.bam a separate alignment step left; rmdup_command gives rule `rmdup`
+one `qm_driver rmdup` job on the sorted BAM of any aligner."""
 import os
 
 # rule -> {output name ("" = the rule's single unnamed output): (directory variable, path pattern)}
@@ -62,6 +63,21 @@ def sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads=4, ex
         b = benchmark_path(dirs, "bcftools", sample, ref_name)
         os.makedirs(os.path.dirname(b), exist_ok=True)
         argv += ["--benchmark", b]
+    return argv + list(extra), paths
+
+
+def rmdup_command(driver, dirs, sample, ref_name, threads=4, extra=()):
+    """-> (argv, [the .rmdup.bam, its .bai, the metrics log]) of the per-rule replacement of `rmdup`: `qm_driver rmdup` on the
+    rule's input, the {sample}.{ref_name}.bam of rule `bwa` (rules/rmdup.smk:8), with picard's library name --sample"""
+    argv = [driver, "rmdup", "--bam", expand(dirs, "bwa", "sortedbam", sample, ref_name), "--sample", sample, "-t", str(threads)]
+    paths = []
+    for name in ("rmdupbam", "log"):
+        p = expand(dirs, "rmdup", name, sample, ref_name)
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+        argv += [DRIVER_OPTION[("rmdup", name)], p]
+        paths.append(p)
+        if ("rmdup", name) in SIDE_FILES:
+            paths.append(p + SIDE_FILES[("rmdup", name)])
     return argv + list(extra), paths
 
 
