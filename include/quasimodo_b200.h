@@ -113,8 +113,10 @@ int64_t qm_index_lpac(const qm_index *idx);
  * are bwa-mem's -- the three rounds of mem_collect_intv (SMEMs, re-seeding, the LAST-like round) and the suffix-array walk of
  * mem_chain, at most QM_MAX_SEEDS per read in bwa's order -- instead of all exact matches of the k-mer hash index.
  * qm_index_attach_bwa takes the bytes of the index files `bwa index` wrote (rules/index.smk:13: X.bwt and X.sa; the reference
- * ships them as ref/X.bwt, ref/X.sa); qm_index_build_fm rebuilds the same bytes from the genome given to qm_index_build;
- * qm_index_fm_export returns them (pass NULL buffers for the sizes).  Host work, once per genome. */
+ * ships them as ref/X.bwt, ref/X.sa); qm_index_build_fm rebuilds the same bytes from the genome given to qm_index_build, on the
+ * device (suffix array of forward + reverse complement by prefix doubling, BWT, checkpoints and samples; about 58 bytes of
+ * device memory per suffix while it runs, QM_ELIMIT past 2^31 - 1 suffixes); qm_index_fm_export copies them back as the two
+ * files (pass NULL buffers for the sizes).  Once per genome; the index stays in device memory. */
 int qm_index_attach_bwa(qm_ctx *ctx, qm_index *idx, const uint8_t *h_bwt, int64_t bwt_bytes, const uint8_t *h_sa, int64_t sa_bytes);
 int qm_index_build_fm(qm_ctx *ctx, qm_index *idx, const uint8_t *h_codes);
 int qm_index_fm_export(const qm_index *idx, uint8_t *h_bwt, int64_t *bwt_bytes, uint8_t *h_sa, int64_t *sa_bytes);

@@ -41,6 +41,11 @@
 //          existing coordinate-sorted BAM without its duplicates, byte for byte (0x400 cleared), the input's header plus one @PG
 //          line, the .bai and the duplication metrics.  Inflated and validated on the host before a CUDA context exists; the
 //          decision runs on the device (qm_bam_mark_duplicates), ties going to the file order of the sorted BAM as in picard
+//   qm_driver index    --ref X.fa [--prefix P] [--gpu I] [-t THREADS]
+//        = rules/index.smk:12-14 (`bwa index` + `samtools faidx`): bwa's five index files P.bwt, P.sa (suffix array, BWT,
+//          checkpoints and samples built on the device, qm_index_build_fm), P.pac, P.ann, P.amb, and X.fa.fai; --prefix defaults
+//          to the FASTA path, as in bwa.  The FASTA is read and validated on the host before a CUDA context exists (A/C/G/T only,
+//          line lengths samtools faidx accepts, at most QM_MAX_CONTIGS contigs, 2 x length < 2^31)
 //   qm_driver bam-from-records --ref .. --r1 .. --r2 .. --alns ALNS.bin [--perm PERM.bin] --bam OUT.bam
 //        = the BAM/BAI writer alone on given qm_aln records (test entry; with --perm no GPU is touched)
 //   qm_driver fastq-check --r1 .. --r2 .. [-t THREADS]
@@ -2023,6 +2028,165 @@ int cmd_rmdup(const Args &a, const std::string &cmdline)
     pc.report();
     return 0;
 }
+// ------------------------------------------------------------------------------------------------
+// `qm_driver index`: rule build_idx (`bwa index X.fa` + `samtools faidx X.fa`) one for one
+struct FaiRow { int64_t offset = 0, line_bases = 0, line_bytes = 0; };
+
+// the FASTA as both tools read it; every refusal exits 2 naming the contig, the line or the limit.  A line is counted in bytes with
+// its terminator ("\n" or "\r\n"), as the .fai records it; within a contig every line but the last has the first line's length
+// and the last is not longer (samtools faidx refuses anything else, a blank line followed by more sequence included).
+void read_fasta_for_index(const std::string &path, Genome &g, std::vector<std::string> &annos, std::vector<FaiRow> &fai)
+{
+    std::string d;
+    {
+        FILE *fp = fopen(path.c_str(), "rb");
+        if (!fp) die(2, "cannot open %s", path.c_str());
+        char buf[1 << 16];
+        size_t k;
+        while ((k = fread(buf, 1, sizeof buf, fp)) > 0) d.append(buf, k);
+        const bool bad = ferror(fp) != 0;
+        fclose(fp);
+        if (bad) die(2, "read error in %s", path.c_str());
+    }
+    const char *fn = path.c_str();
+    if (d.size() >= 2 && (uint8_t)d[0] == 0x1f && (uint8_t)d[1] == 0x8b) die(2, "%s: compressed FASTA: index the plain file", fn);
+    int8_t lut[256];
+    memset(lut, -1, sizeof lut);
+    lut['A'] = lut['a'] = 0; lut['C'] = lut['c'] = 1; lut['G'] = lut['g'] = 2; lut['T'] = lut['t'] = 3;
+    int64_t line_no = 0, short_line = 0;              // short_line: the line of this contig that was shorter than the first (0: none)
+    bool open = false;
+    auto close_contig = [&]() {
+        if (!open) return;
+        g.lens.back() = (int64_t)g.codes.size() - g.offs.back();
+        if (g.lens.back() == 0) die(2, "%s: contig %s has no bases", fn, g.names.back().c_str());
+    };
+    for (size_t p = 0; p < d.size();) {
+        size_t e = d.find('\n', p);
+        const bool terminated = e != std::string::npos;
+        if (!terminated) e = d.size();
+        const int64_t bytes = (int64_t)(e - p) + (terminated ? 1 : 0);
+        size_t len = e - p;
+        if (len && d[p + len - 1] == '\r') --len;
+        ++line_no;
+        const char *ln = d.data() + p;
+        if (len && ln[0] == '>') {
+            close_contig();
+            size_t a = 1;
+            while (a < len && !isspace((unsigned char)ln[a])) ++a;
+            std::string name(ln + 1, a - 1), anno = a < len ? std::string(ln + a + 1, len - a - 1) : std::string();
+            if (name.empty()) die(2, "%s: line %lld: a '>' line without a name", fn, (long long)line_no);
+            for (auto &other : g.names) if (other == name) die(2, "%s: line %lld: contig name %s occurs twice", fn, (long long)line_no, name.c_str());
+            if (g.names.size() == QM_MAX_CONTIGS) die(2, "%s: line %lld: more than %d contigs: at most %d are supported", fn, (long long)line_no, QM_MAX_CONTIGS, QM_MAX_CONTIGS);
+            g.names.push_back(name);
+            annos.push_back(anno);
+            g.offs.push_back((int64_t)g.codes.size());
+            g.lens.push_back(0);
+            FaiRow r;
+            r.offset = (int64_t)(e + (terminated ? 1 : 0));
+            fai.push_back(r);
+            open = true;
+            short_line = 0;
+        } else {
+            if (!open) {
+                if (len == 0) { p = e + 1; continue; }         // blank lines before the first header
+                die(2, "%s: line %lld: sequence before the first '>' line", fn, (long long)line_no);
+            }
+            FaiRow &r = fai.back();
+            if (len > 0) {
+                if (short_line) die(2, "%s: contig %s: line %lld is shorter than the contig's first line and more sequence follows it (samtools faidx refuses different line lengths)",
+                                    fn, g.names.back().c_str(), (long long)short_line);
+                if (r.line_bases == 0) { r.line_bases = (int64_t)len; r.line_bytes = terminated ? bytes : (int64_t)len + 1; }
+                else if ((int64_t)len > r.line_bases || (terminated && bytes - (int64_t)len != r.line_bytes - r.line_bases))
+                    die(2, "%s: contig %s: line %lld has %lld bases, the contig's first line %lld (samtools faidx refuses different line lengths)",
+                        fn, g.names.back().c_str(), (long long)line_no, (long long)len, (long long)r.line_bases);
+                for (size_t i = 0; i < len; ++i) {
+                    const int8_t v = lut[(unsigned char)ln[i]];
+                    if (v < 0) die(2, "%s: line %lld: base '%c' in contig %s: only A/C/G/T references are supported (bwa index would draw a random base)",
+                                   fn, (long long)line_no, ln[i], g.names.back().c_str());
+                    g.codes.push_back((uint8_t)v);
+                }
+                if ((int64_t)len < r.line_bases) short_line = line_no;
+            } else if (r.line_bases > 0 && !short_line) short_line = line_no;
+        }
+        if ((int64_t)g.codes.size() >= (1ll << 30))
+            die(2, "%s: more than 2^30 - 1 bases: the suffix array of both strands holds at most 2^31 - 1 suffixes", fn);
+        p = e + 1;
+    }
+    close_contig();
+    if (g.names.empty()) die(2, "%s: no contigs", fn);
+}
+
+void write_file(const std::string &path, const void *data, size_t bytes)
+{
+    FILE *fp = fopen(path.c_str(), "wb");
+    if (!fp || (bytes && fwrite(data, 1, bytes, fp) != bytes) || fclose(fp) != 0) die(2, "cannot write %s", path.c_str());
+}
+
+// .pac (bwa bntseq.c): the forward strand, base i in byte i >> 2 at shift ((~i) & 3) << 1, then one zero byte when l_pac % 4 == 0,
+// then one byte holding l_pac % 4
+std::vector<uint8_t> pack_pac(const std::vector<uint8_t> &codes)
+{
+    const int64_t l = (int64_t)codes.size();
+    std::vector<uint8_t> pac((size_t)((l >> 2) + ((l & 3) ? 1 : 0)), 0);
+    for (int64_t i = 0; i < l; ++i) pac[(size_t)(i >> 2)] |= (uint8_t)(codes[(size_t)i] << ((~i & 3) << 1));
+    if (l % 4 == 0) pac.push_back(0);
+    pac.push_back((uint8_t)(l % 4));
+    return pac;
+}
+
+int cmd_index(const Args &a)
+{
+    PhaseClock pc;
+    require_known(a, "index", {"ref", "prefix", "t", "threads", "gpu"});
+    if (!a.has("ref")) die(1, "--ref is required");
+    g_threads = std::max(1, atoi(a.get("t", a.get("threads", "4")).c_str()));
+    const std::string fa = a.get("ref"), prefix = a.get("prefix", fa);
+    if (prefix.empty()) die(1, "--prefix: empty");
+    Genome g;
+    std::vector<std::string> annos;
+    std::vector<FaiRow> fai;
+    read_fasta_for_index(fa, g, annos, fai);
+    const int64_t l_pac = (int64_t)g.codes.size();
+    pc.mark("FASTA");
+    fprintf(stderr, "[qm_driver] %s: %zu contigs, %lld bases\n", fa.c_str(), g.names.size(), (long long)l_pac);
+    Lib L;
+    const int dev = atoi(a.get("gpu", "0").c_str());
+    const int rc = qm_ctx_create(dev, &L.ctx);
+    if (rc != QM_OK) die(3, "qm_ctx_create(%d) failed (%d): no usable B200 (there is no CPU fallback)", dev, rc);
+    pc.mark("context");
+    qm_index *idx = nullptr;
+    L.check(qm_index_build(L.ctx, g.codes.data(), (int)g.names.size(), g.lens.data(), 31, &idx), "qm_index_build");
+    pc.mark("reference on the device");
+    L.check(qm_index_build_fm(L.ctx, idx, g.codes.data()), "qm_index_build_fm");
+    pc.mark("suffix array + BWT");
+    int64_t nb = 0, ns = 0;
+    L.check(qm_index_fm_export(idx, nullptr, &nb, nullptr, &ns), "qm_index_fm_export");
+    std::vector<uint8_t> bwt((size_t)nb), sa((size_t)ns);
+    L.check(qm_index_fm_export(idx, bwt.data(), &nb, sa.data(), &ns), "qm_index_fm_export");
+    qm_index_destroy(L.ctx, idx);
+    qm_ctx_destroy(L.ctx);
+    write_file(prefix + ".bwt", bwt.data(), bwt.size());
+    write_file(prefix + ".sa", sa.data(), sa.size());
+    const std::vector<uint8_t> pac = pack_pac(g.codes);
+    write_file(prefix + ".pac", pac.data(), pac.size());
+    std::string ann = std::to_string(l_pac) + " " + std::to_string(g.names.size()) + " 11\n";
+    for (size_t c = 0; c < g.names.size(); ++c) {
+        ann += "0 " + g.names[c] + " " + (annos[c].empty() ? std::string("(null)") : annos[c]) + "\n";
+        ann += std::to_string(g.offs[c]) + " " + std::to_string(g.lens[c]) + " 0\n";
+    }
+    write_file(prefix + ".ann", ann.data(), ann.size());
+    const std::string amb = std::to_string(l_pac) + " " + std::to_string(g.names.size()) + " 0\n";
+    write_file(prefix + ".amb", amb.data(), amb.size());
+    std::string fx;
+    for (size_t c = 0; c < g.names.size(); ++c)
+        fx += g.names[c] + "\t" + std::to_string(g.lens[c]) + "\t" + std::to_string(fai[c].offset) + "\t" + std::to_string(fai[c].line_bases) + "\t" +
+              std::to_string(fai[c].line_bytes) + "\n";
+    write_file(fa + ".fai", fx.data(), fx.size());
+    pc.mark("files");
+    pc.report();
+    return 0;
+}
+
 }  // namespace
 
 // --benchmark FILE (any command): the job's resources in the shape of a Snakemake `benchmark:` file (one header line, one row:
@@ -2065,7 +2229,7 @@ int main(int argc, char **argv)
 {
     g_benchmark_t0 = std::chrono::steady_clock::now();
     g_benchmark_cpu0 = clock();
-    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|rmdup|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
+    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|rmdup|index|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
     std::string cmdline;
     for (int i = 0; i < argc; ++i) { if (i) cmdline += ' '; cmdline += argv[i]; }
     const std::string cmd = argv[1];
@@ -2080,6 +2244,7 @@ int main(int argc, char **argv)
     if (cmd == "bam-from-records") return cmd_bam_from_records(a, cmdline);
     if (cmd == "pileup") return cmd_pileup(a);
     if (cmd == "rmdup") return cmd_rmdup(a, cmdline);
+    if (cmd == "index") return cmd_index(a);
     if (cmd == "fastq-check") {                        // host only: parse the two mate files as `sample` would, report what is there
         require_known(a, "fastq-check", {"r1", "r2", "t", "threads"});
         if (!a.has("r1") || !a.has("r2")) die(1, "--r1 --r2 are required");

@@ -37,7 +37,8 @@ struct qm_index {
     bool have_fm = false;
     FmView fm = {};
     void *d_fm_bwt = nullptr, *d_fm_sa = nullptr;
-    std::vector<uint8_t> fm_bwt_bytes, fm_sa_bytes;       // the index as bwa's two files (qm_index_fm_export)
+    int64_t fm_words = 0;                                 // uint32 words of the .bwt behind its 40-byte header (qm_index_fm_export)
+    int fm_device = -1;
 };
 
 static __device__ __forceinline__ int qm_ref_base(const IndexView &V, int64_t x)

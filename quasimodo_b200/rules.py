@@ -4,7 +4,8 @@ paths of rules `bwa` (rules/bwa.smk:1-19), `rmdup` (rules/rmdup.smk:1-18), `mpil
 whose declared output is missing, so tests/test_rules_cpu.py checks these tables against the reference's rule files and
 tests/test_driver_gpu.py checks that the command really writes every path.  pileup_commands gives rules `mpileup` and
 `bcftools` one `qm_driver pileup` job each, on the .rmdup.bam a separate alignment step left; rmdup_command gives rule `rmdup`
-one `qm_driver rmdup` job on the sorted BAM of any aligner."""
+one `qm_driver rmdup` job on the sorted BAM of any aligner; index_command gives rule `build_idx` (rules/index.smk:12-14) one
+`qm_driver index` job in place of `bwa index` + `samtools faidx`."""
 import os
 
 # rule -> {output name ("" = the rule's single unnamed output): (directory variable, path pattern)}
@@ -106,3 +107,20 @@ def pileup_commands(driver, dirs, sample, ref_name, ref_fa, threads=4, extra=(),
             argv += ["--benchmark", b]
         out[rule] = (argv + list(extra), paths)
     return out
+
+
+# the files rule `build_idx` (rules/index.smk:12-14) leaves next to a genome X.fa: `bwa index X.fa` writes X.fa.{amb,ann,bwt,pac,sa}
+# (its prefix defaults to the FASTA path), `samtools faidx X.fa` writes X.fa.fai
+BWA_INDEX_SUFFIXES = (".amb", ".ann", ".bwt", ".pac", ".sa")
+FAIDX_SUFFIX = ".fai"
+
+
+def index_command(driver, ref_fa, threads=4, extra=(), benchmark=None):
+    """-> (argv, [the five bwa index files and the .fai]) of the per-rule replacement of `build_idx`: `qm_driver index` on one
+    genome, writing what `bwa index` and `samtools faidx` write, under the names they use (the sample commands' --bwa-index
+    takes ref_fa as its prefix); benchmark=PATH adds `--benchmark PATH`"""
+    argv = [driver, "index", "--ref", ref_fa, "-t", str(threads)]
+    if benchmark:
+        os.makedirs(os.path.dirname(os.path.abspath(benchmark)), exist_ok=True)
+        argv += ["--benchmark", benchmark]
+    return argv + list(extra), [ref_fa + s for s in BWA_INDEX_SUFFIXES] + [ref_fa + FAIDX_SUFFIX]
