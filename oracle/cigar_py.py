@@ -42,9 +42,10 @@ def hit_to_record(doubled, l_pac, offs, read, hit, a=1, b=4, o_del=6, e_del=1, o
         tries += 1
         if not (tries < 3 and score < hit["truesc"] - a):
             break
-    # edit distance over the whole path, before anything is trimmed
+    # edit distance over the whole path, before anything is trimmed; a leading or trailing deletion is not counted (bwa_gen_cigar2
+    # leaves it out of NM and MD, and mem_reg2aln then squeezes it out of the CIGAR)
     nm, i, k = 0, 0, 0
-    for op, ln in ops:
+    for x, (op, ln) in enumerate(ops):
         if op == 0:
             nm += sum(1 for j in range(ln) if q[k + j] != t[i + j] or q[k + j] > 3 or t[i + j] > 3)
             i += ln
@@ -53,7 +54,7 @@ def hit_to_record(doubled, l_pac, offs, read, hit, a=1, b=4, o_del=6, e_del=1, o
             nm += ln
             k += ln
         else:
-            nm += ln
+            nm += ln if 0 < x < len(ops) - 1 else 0
             i += ln
     # (both sequences were turned round for a reverse-strand hit, so the path already reads along the forward strand, as a BAM
     # record wants it: bwa turns only the query back afterwards.  SURVEY.md A.4's "reverse the CIGAR after" is not what happens --

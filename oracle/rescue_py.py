@@ -70,10 +70,12 @@ def rescue_from(doubled, l_pac, offs, clens, pes, anchor, mate_seq, mate_hits, o
             if rev:
                 cb, ce = 2 * l_pac - ce, 2 * l_pac - cb
             rb, re = max(rb, cb), min(re, ce)
+        counters.setdefault("windows", []).append(re - rb if anchor["rid"] == rid else -1)     # (what the tests show they reach)
         if anchor["rid"] == rid and opt.min_seed_len <= re - rb <= MAX_WINDOW:
             seq = [(3 - int(c) if int(c) < 4 else 4) for c in mate_seq[::-1]] if opposite else [int(c) for c in mate_seq]
             (score, te, qe, score2, _, tb, qb), cells = qmo_py.ksw_align2(seq, doubled[rb:re], opt.min_seed_len * opt.a, opt)
             counters["cells"] += cells
+            counters.setdefault("scores", []).append(score)
             if score >= opt.min_seed_len and qb >= 0:
                 new = dict(rid=anchor["rid"], score=score, csub=score2,
                            qb=L - (qe + 1) if opposite else qb, qe=L - qb if opposite else qe + 1,

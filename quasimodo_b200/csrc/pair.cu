@@ -255,14 +255,30 @@ __device__ __forceinline__ int cig_band(const qm_opt &o, int w2, int lq, int rle
     const int min_w = abs(rlen - lq) + 3;
     return w < min_w ? min_w : w;
 }
+// The thread-per-task kernels keep eh[] in 16 bits with -20000 as minus infinity.  That orders like the reference's -2^30 only
+// while every real DP value stays well above -20000 and minus infinity less one cell's penalties stays above -32768.  Every
+// in-band cell (i, j) is reached by at most min(lq, rlen) diagonal steps and one gap of |i - j|, so no real H, E or F is below
+// -(max(b, 1) min(lq, rlen) + the longest gap + one gap opening).  With the default scores that is about -3,100 for 512 bases;
+// large penalties (b = 100, gaps 100 + 60 k on a 400-base read: below -24,000) break it, and such tasks go to the warp kernel,
+// whose cells are 32-bit.  kCig16Bound leaves room on both sides: NEG16 + a stays below every real value and NEG16 - (b + gap
+// opening) above -32768.
+constexpr int kCig16Bound = 12000;
+__device__ __forceinline__ bool cig_fits16(const qm_opt &o, int lq, int rlen)
+{
+    const int64_t mb = o.b > 1 ? o.b : 1;
+    const int64_t gd = o.o_del + (int64_t)o.e_del * rlen, gi = o.o_ins + (int64_t)o.e_ins * lq;
+    const int64_t oe = o.o_del + o.e_del > o.o_ins + o.e_ins ? o.o_del + o.e_del : o.o_ins + o.e_ins;
+    return mb * (lq < rlen ? lq : rlen) + (gd > gi ? gd : gi) + oe <= kCig16Bound;
+}
+
 // which kernel takes a CIGAR task first: 0 / 1 / 2 = score-only thread-per-task pass with 32 / 48 / 72 circular slots
 // (equal lengths, band <= 15 / 23 / 35 -- 35 is the most bwa_gen_cigar2 allows for equal lengths up to 140 bp),
 // 3 / 4 / 5 = thread-per-task pass with traceback and 32 / 64 / 128 slots (length difference, band <= 15 / 31 / 63),
-// 6 = the warp-per-task kernel with traceback
+// 6 = the warp-per-task kernel with traceback (also every task whose DP values 16-bit cells cannot hold: cig_fits16)
 __device__ __forceinline__ int cig_class(const IndexView &V, const qm_opt &o, const CigTask &t, int lq)
 {
     const int rlen = (int)(t.re - t.rb);
-    if (t.rb < V.l_pac && t.re > V.l_pac) return 6;
+    if ((t.rb < V.l_pac && t.re > V.l_pac) || !cig_fits16(o, lq, rlen)) return 6;
     int w = cig_band(o, t.w2, lq, rlen);
     if (lq != rlen) return w <= 15 ? 3 : w <= 31 ? 4 : w <= 63 ? 5 : 6;     // traceback needed: thread-per-task kernels by band, else warp
     w = w < t.wcap ? w : t.wcap;            // the score-only pass may narrow its band (cig_gain_cap)
@@ -758,9 +774,8 @@ cig_trace_kernel(IndexView V, qm_opt o, const uint8_t *__restrict__ codes, int s
                  const CigTask *__restrict__ tasks, const int *__restrict__ mine, const int *__restrict__ n_mine, int wmax,
                  uint8_t *__restrict__ slab, qm_aln *__restrict__ alns, int *__restrict__ next, int *__restrict__ n_next)
 {
-    // eh[] in 16 bits: every real score of a <= 500-base global alignment is above -4000 and the "minus infinity" of
-    // cells outside the band only ever loses a few hundred more, so -20000 orders exactly like the reference's
-    // -2^30 in every comparison.  Slots (2s, 2s+1) of a thread share one 32-bit word: lane t always hits bank t.
+    // eh[] in 16 bits: cig_class sends a task here only when every real DP value of it is above -kCig16Bound (cig_fits16),
+    // so -20000 orders exactly like the reference's -2^30 in every comparison.  Slots (2s, 2s+1) of a thread share one 32-bit word: lane t always hits bank t.
     extern __shared__ short ct_smem[];
     constexpr int NEG16 = -20000;
     short *HS = ct_smem + 2 * threadIdx.x;
