@@ -281,6 +281,18 @@ int  qm_sample_add_pairs_host(qm_sample *s, const uint8_t *h_codes, const uint8_
 int  qm_sample_add_pairs_host_packed(qm_sample *s, const uint8_t *h_bases2, const uint8_t *h_nmask, const uint8_t *h_quals, int32_t stride,
                                      const int32_t *h_lens, int64_t n_pairs, int64_t pair_id0, qm_aln *h_alns /* may be NULL */);
 int  qm_pack_reads_host(const uint8_t *h_codes, int32_t stride, int64_t n_reads, uint8_t *h_bases2, uint8_t *h_nmask);
+/* ---- contaminant passes (replaces rules `rm_phix` / `rm_human_ecoli`, rules/decontamination.smk:15-17,43-48: `bwa mem` against
+ * the contaminants | `samtools view -f 12 -F 256` | `sort -n` | `bedtools bamtofastq`) ----
+ * qm_sample_set_filter(on) before the first pairs (QM_EINVAL after them, or on a sample in rmdup / depth-cap mode, which in turn
+ * refuse a filter-mode sample): the sample aligns and finishes its pairs as usual, the CIGAR stage included (a CIGAR overflow
+ * unmaps a read), and its insert-size model is fixed as above; it runs no pileup, fills neither the count tensor (which stays
+ * zero) nor the indel table, ignores qm_sample_set_baq and keeps no records across batches.  A kernel applies the rule's keep
+ * test to each pair of every batch on the device: keep = (flag & 12) == 12 && !(flag & 256) on both records.
+ * qm_sample_keep_host: h_keep[p] = 1 for each kept pair p of the LAST batch handed in (any entry above; n_pairs must be that
+ * batch's pair count, QM_EINVAL otherwise), *h_n_kept (may be NULL) = their number.  n_pairs bytes come back, not the records.
+ * Synchronous.  QM_EINVAL when the sample is not in filter mode. */
+int  qm_sample_set_filter(qm_sample *s, int on);
+int  qm_sample_keep_host(qm_sample *s, uint8_t *h_keep, int64_t n_pairs, int64_t *h_n_kept);
 int32_t *qm_sample_counts(qm_sample *s);                          /* device pointer, planes [QM_NCH][l_pac] */
 int  qm_sample_stats_sync(qm_sample *s, int64_t *n_pairs, int64_t *cells, void *stream);
 int  qm_sample_counts_host(qm_sample *s, int32_t *h_rows /* [l_pac][QM_NCH] */);

@@ -113,6 +113,8 @@ SIGNATURES = {
     "qm_sample_add_pairs_host": (C.c_int, [_P, _P, _P, _I, _P, _L, _L, _P]),
     "qm_sample_add_pairs_host_packed": (C.c_int, [_P, _P, _P, _P, _I, _P, _L, _L, _P]),
     "qm_pack_reads_host": (C.c_int, [_P, _I, _L, _P, _P]),
+    "qm_sample_set_filter": (C.c_int, [_P, C.c_int]),
+    "qm_sample_keep_host": (C.c_int, [_P, _P, _L, C.POINTER(C.c_int64)]),
     "qm_sample_counts": (_P, [_P]),
     "qm_sample_stats_sync": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), _P]),
     "qm_sample_counts_host": (C.c_int, [_P, _P]),

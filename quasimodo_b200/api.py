@@ -211,6 +211,18 @@ class Sample:
         """bcftools mpileup -d: htslib's depth cap (0 = off); counting is deferred to finish()"""
         _check(self.ctx._h, _lib.lib().qm_sample_set_max_depth(self._h, int(max_depth)), "qm_sample_set_max_depth")
 
+    def set_filter(self, on=True):
+        """filter mode (a contaminant pass): align and finish pairs, count nothing, leave one keep byte per pair of each batch"""
+        _check(self.ctx._h, _lib.lib().qm_sample_set_filter(self._h, 1 if on else 0), "qm_sample_set_filter")
+
+    def keep(self, n_pairs):
+        """filter mode: -> uint8 [n_pairs], 1 for each pair of the last batch whose records both pass `samtools view -f 12 -F 256`"""
+        k = np.zeros(n_pairs, dtype=np.uint8)
+        n = C.c_int64()
+        _check(self.ctx._h, _lib.lib().qm_sample_keep_host(self._h, k.ctypes.data, int(n_pairs), C.byref(n)), "qm_sample_keep_host")
+        assert n.value == int(k.sum())
+        return k
+
     def set_baq(self, flag=3):
         """base alignment quality for the pileup: 0 off (-B, default), 3 extended BAQ (what both mpileups run), 1 plain"""
         _check(self.ctx._h, _lib.lib().qm_sample_set_baq(self._h, int(flag)), "qm_sample_set_baq")

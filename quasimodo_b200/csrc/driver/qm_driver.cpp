@@ -20,6 +20,12 @@
 //        (duplicates flagged 0x400), --rmdup-bam is the REMOVE_DUPLICATES=true file.  With --gpus the reads and records stay on
 //        their GPUs: duplicates and the --max-depth cap are decided over small per-pair / per-read tuples all-gathered over NCCL,
 //        so every output is the one-GPU output
+//        --decontam A.fa[,B.fa] [--decontam2 C.fa[,D.fa]] [--clean-r1 F --clean-r2 F]: rules rm_phix and rm_human_ecoli
+//        (rules/decontamination.smk:15-17,43-48) in the same job, in front of the target: each raw batch is aligned against pass 1's
+//        genome (its own index, filter-mode sample and insert-size model; bwa's options, not --bwa-index / --fm-seeds), the pairs
+//        whose records are both unmapped are gathered on the host, still packed, and go on to pass 2, then to the target, whose pair
+//        ids count the kept pairs.  Every output equals `decontam` (pass 1) | `decontam` (pass 2) | `sample` on the cleaned FASTQ,
+//        with --gpus too; --clean-r1/-r2 write that cleaned FASTQ.  Not with --keep-contigs
 //        = rules/bwa.smk:15-18 (bwa mem | samtools view | samtools sort | samtools index -> BAM + BAI),
 //          rules/vcfcall.smk:39 (pileup path: count TSV, SURVEY.md B.3) and rules/vcfcall.smk:115-117 (VCF)
 //   qm_driver decontam --ref CONTAMINANT.fa[,MORE.fa] --r1 .. --r2 .. --out-r1 CLEAN1.fq --out-r2 CLEAN2.fq
@@ -61,6 +67,7 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <condition_variable>
 #include <cstdarg>
 #include <ctime>
 #include <cstdint>
@@ -383,6 +390,71 @@ void free_batch(Lib &L, Batch &b)
     std::string().swap(b.names);
     std::vector<uint32_t>().swap(b.name_off);
 }
+
+// The pairs of src[k] whose byte keep[k][p] is set (keep[k] == nullptr: all of them), in order, as one batch at the largest stride
+// among the sources: packed bases, N mask, qualities, codes, lengths and names are copied as they are, the rows padded as pack_batch
+// pads them (N bases, quality 0).  A threaded host gather; the records are not carried (alns stays unset).
+void gather_pairs(Lib &L, const std::vector<const Batch *> &src, const std::vector<const uint8_t *> &keep, Batch &out)
+{
+    std::vector<std::pair<uint32_t, int64_t>> sel;            // (source, pair)
+    int32_t stride = 16;
+    for (size_t k = 0; k < src.size(); ++k) {
+        for (int64_t p = 0; p < src[k]->n_pairs; ++p) if (!keep[k] || keep[k][p]) sel.emplace_back((uint32_t)k, p);
+        if (src[k]->n_pairs) stride = std::max(stride, src[k]->stride);
+    }
+    const size_t n = sel.size(), sp = (size_t)stride / 4, sm = (size_t)stride / 8;
+    out.n_pairs = (int64_t)n;
+    out.stride = stride;
+    void *p = nullptr;
+    L.check(qm_host_alloc(L.ctx, 2 * n * stride, &p), "qm_host_alloc"); out.codes = (uint8_t *)p;
+    L.check(qm_host_alloc(L.ctx, 2 * n * stride, &p), "qm_host_alloc"); out.quals = (uint8_t *)p;
+    L.check(qm_host_alloc(L.ctx, 2 * n * sizeof(int32_t), &p), "qm_host_alloc"); out.lens = (int32_t *)p;
+    L.check(qm_host_alloc(L.ctx, 2 * n * sp, &p), "qm_host_alloc"); out.bases2 = (uint8_t *)p;
+    L.check(qm_host_alloc(L.ctx, 2 * n * sm, &p), "qm_host_alloc"); out.nmask = (uint8_t *)p;
+    auto name = [&](size_t i) { const Batch &b = *src[sel[i].first]; return b.names.data() + b.name_off[(size_t)sel[i].second]; };
+    std::vector<uint32_t> nl(n);
+    parallel_ranges(n, [&](size_t i0, size_t i1) { for (size_t i = i0; i < i1; ++i) nl[i] = (uint32_t)strlen(name(i)) + 1; });
+    out.name_off.resize(n);
+    uint32_t o = 0;
+    for (size_t i = 0; i < n; ++i) { out.name_off[i] = o; o += nl[i]; }
+    out.names.resize(o);
+    parallel_ranges(n, [&](size_t i0, size_t i1) {
+        for (size_t i = i0; i < i1; ++i) {
+            const Batch &b = *src[sel[i].first];
+            memcpy(&out.names[out.name_off[i]], name(i), nl[i]);
+            const size_t bs = (size_t)b.stride, bp = bs / 4, bm = bs / 8;
+            for (int m = 0; m < 2; ++m) {
+                const size_t r = (size_t)(2 * sel[i].second + m), w = 2 * i + m;
+                memcpy(out.codes + w * stride, b.codes + r * bs, bs); memset(out.codes + w * stride + bs, 4, stride - bs);
+                memcpy(out.quals + w * stride, b.quals + r * bs, bs); memset(out.quals + w * stride + bs, 0, stride - bs);
+                memcpy(out.bases2 + w * sp, b.bases2 + r * bp, bp); memset(out.bases2 + w * sp + bp, 0, sp - bp);
+                memcpy(out.nmask + w * sm, b.nmask + r * bm, bm); memset(out.nmask + w * sm + bm, 0xff, sm - bm);
+                out.lens[w] = b.lens[r];
+            }
+        }
+    });
+}
+
+// Pair ids of `sample --decontam` across the GPU workers.  A pair's id in a stage is its index in that stage's input (in the
+// three-job chain: its index in the FASTQ the stage reads), so batch i takes its ids of a stage once batch i - 1 has taken its own.
+// Channel s < number of stages: ids of stage s; one more channel orders the writes of the cleaned FASTQ.
+struct Ledger {
+    std::mutex m;
+    std::condition_variable cv;
+    std::vector<int64_t> turn, total;                        // per channel: the batch whose turn it is, pairs taken so far
+    int64_t begin(int ch, int64_t i)
+    {
+        std::unique_lock<std::mutex> lk(m);
+        cv.wait(lk, [&]() { return turn[(size_t)ch] == i; });
+        return total[(size_t)ch];
+    }
+    void end(int ch, int64_t n)
+    {
+        { std::lock_guard<std::mutex> lk(m); total[(size_t)ch] += n; ++turn[(size_t)ch]; }
+        cv.notify_all();
+    }
+    int64_t take(int ch, int64_t i, int64_t n) { const int64_t t = begin(ch, i); end(ch, n); return t; }
+};
 
 // ------------------------------------------------------------------------------------------------
 // BGZF writer (SURVEY.md B.7): blocks of <= 0xff00 bytes, raw deflate level 1, compressed by a thread team,
@@ -762,17 +834,26 @@ std::string trim_float3(double x)
 // --gpus: batches are dealt round-robin, batch i to GPU i % n_gpu; a GPU keeps the records of its batches in the order it got them
 int batch_gpu(int64_t batch, int n_gpu) { return (int)(batch % n_gpu); }
 
-// where each batch's records lie among those its GPU kept (qm_sample_kept_alns_host): {GPU, first record} per batch
-std::vector<std::pair<int, int64_t>> batch_sources(const std::vector<int64_t> &batch_pairs, int n_gpu)
+// where each batch's records lie among those its GPU kept (qm_sample_kept_alns_host): {GPU, first record} per batch, batch i having
+// gone to GPU batch_dev[i]
+std::vector<std::pair<int, int64_t>> batch_sources(const std::vector<int64_t> &batch_pairs, const std::vector<int> &batch_dev, int n_gpu)
 {
     std::vector<std::pair<int, int64_t>> src(batch_pairs.size());
     std::vector<int64_t> next((size_t)n_gpu, 0);
     for (size_t i = 0; i < batch_pairs.size(); ++i) {
-        const int d = batch_gpu((int64_t)i, n_gpu);
+        const int d = batch_dev[i];
         src[i] = {d, next[(size_t)d]};
         next[(size_t)d] += 2 * batch_pairs[i];
     }
     return src;
+}
+
+// the same for batches dealt round-robin
+std::vector<std::pair<int, int64_t>> batch_sources(const std::vector<int64_t> &batch_pairs, int n_gpu)
+{
+    std::vector<int> dev(batch_pairs.size());
+    for (size_t i = 0; i < dev.size(); ++i) dev[i] = batch_gpu((int64_t)i, n_gpu);
+    return batch_sources(batch_pairs, dev, n_gpu);
 }
 
 // An indel allele that passes the caller's thresholds (same rule as the SNPs: raw depth at the anchor >= min_dp, supporting
@@ -963,7 +1044,7 @@ Args parse_args(int argc, char **argv, int first)
 }
 
 // an option the command does not know is a usage error (a typo such as --min-qual must not silently run with the default)
-void require_known(const Args &a, const char *cmd, std::initializer_list<const char *> known)
+void require_known(const Args &a, const char *cmd, const std::vector<const char *> &known)
 {
     for (auto &kv : a.kv) {
         bool ok = false;
@@ -1054,9 +1135,28 @@ std::vector<std::string> split(const std::string &s, char sep)
     return out;
 }
 
+void check_refs(const Genome &g);
+
 void load_refs(const std::string &spec, Genome &g)
 {
     for (auto &p : split(spec, ',')) read_fasta(p, g);
+    check_refs(g);
+}
+
+// a contaminant pass's genome (--decontam / --decontam2): as load_refs, an empty contig named with its file and option
+void load_pass_refs(const char *opt, const std::string &spec, Genome &g)
+{
+    for (auto &p : split(spec, ',')) {
+        const size_t c0 = g.names.size();
+        read_fasta(p, g);
+        for (size_t i = c0; i < g.names.size(); ++i)
+            if (g.lens[i] <= 0) die(2, "--%s %s: contig %s is empty", opt, p.c_str(), g.names[i].c_str());
+    }
+    check_refs(g);
+}
+
+void check_refs(const Genome &g)
+{
     if (g.names.size() > QM_MAX_CONTIGS) die(2, "%zu contigs: at most %d are supported", g.names.size(), QM_MAX_CONTIGS);
     for (size_t i = 0; i < g.names.size(); ++i) {
         if (g.lens[i] <= 0) die(2, "contig %s is empty", g.names[i].c_str());
@@ -1200,14 +1300,30 @@ void write_outputs(const Args &a, const Genome &g, std::vector<Lib> &Ls, const s
     }
 }
 
+// one contaminant pass of `sample --decontam` (rule rm_phix) or `--decontam2` (rule rm_human_ecoli): its genome and, per GPU, its
+// index and filter-mode sample
+struct Pass {
+    Genome g;
+    std::vector<qm_index *> idxs;
+    std::vector<qm_sample *> smps;
+};
+
 int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
 {
     PhaseClock pc;
-    require_known(a, decontam ? "decontam" : "sample",
-                  {"ref", "r1", "r2", "sample", "bam", "counts", "vcf", "vcf-gz", "out-r1", "out-r2", "keep-contigs", "gpu", "gpus", "t", "threads",
-                   "batch-pairs", "rmdup", "rmdup-bam", "metrics", "no-rescue", "mpileup", "bwa-index", "fm-seeds", "indels", "max-depth", "baq",
-                   "min-mapq", "q", "min-bq", "Q", "count-orphans", "ignore-overlaps", "min-dp", "min-alt", "min-af", "print-options", "stage-ms",
-                   "w", "k", "c", "W", "D", "A", "B", "O", "E", "L", "U", "T", "d"});
+    std::vector<const char *> known = {
+        "ref", "r1", "r2", "sample", "bam", "counts", "vcf", "vcf-gz", "out-r1", "out-r2", "keep-contigs", "gpu", "gpus", "t", "threads",
+        "batch-pairs", "rmdup", "rmdup-bam", "metrics", "no-rescue", "mpileup", "bwa-index", "fm-seeds", "indels", "max-depth", "baq",
+        "min-mapq", "q", "min-bq", "Q", "count-orphans", "ignore-overlaps", "min-dp", "min-alt", "min-af", "print-options", "stage-ms",
+        "w", "k", "c", "W", "D", "A", "B", "O", "E", "L", "U", "T", "d"};
+    if (!decontam) known.insert(known.end(), {"decontam", "decontam2", "clean-r1", "clean-r2"});
+    require_known(a, decontam ? "decontam" : "sample", known);
+    // --decontam A.fa[,B.fa] [--decontam2 C.fa[,D.fa]]: rules rm_phix and rm_human_ecoli in this job, in front of the target
+    // (--clean-r1 / --clean-r2: what the last pass keeps, as FASTQ)
+    if (a.has("decontam2") && !a.has("decontam")) die(1, "--decontam2 needs --decontam (it is the second pass)");
+    if (a.has("clean-r1") != a.has("clean-r2")) die(1, "--clean-r1 and --clean-r2 go together");
+    if (a.has("clean-r1") && !a.has("decontam")) die(1, "--clean-r1 / --clean-r2 need --decontam");
+    if (a.has("decontam") && a.has("keep-contigs")) die(1, "--decontam and --keep-contigs exclude each other (exact passes or the fused approximation)");
     if (atoi(a.get("print-options", "0").c_str())) {   // host only: the alignment options this command line resolves to
         qm_opt o; qm_opt_default(&o);
         apply_bwa_options(a, o);
@@ -1229,6 +1345,9 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     const int keep_contigs = atoi(a.get("keep-contigs", "0").c_str());
     Genome g;
     load_refs(a.get("ref"), g);
+    std::vector<Pass> passes;
+    for (const char *k : {"decontam", "decontam2"})
+        if (a.has(k)) { passes.emplace_back(); load_pass_refs(k, a.get(k), passes.back().g); }
     // --gpus A,B,C or A-B: one context, index and sample per GPU in this one process; batches are dealt round-robin, the
     // count tensors merged with one NCCL all-reduce (north_star).  --gpu I: the single-GPU form.
     std::vector<int> devs;
@@ -1270,6 +1389,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         bwt_file = read_binary<uint8_t>(a.get("bwa-index") + ".bwt");
         sa_file = read_binary<uint8_t>(a.get("bwa-index") + ".sa");
     }
+    const qm_opt pass_opt = opt;                       // the passes take bwa's options, not the target's seeding through bwa's index
     if (a.has("bwa-index") || fm_build) opt.flags |= QM_F_FM_SEEDS;
     std::vector<qm_index *> idxs((size_t)n_gpu, nullptr);
     std::vector<qm_sample *> smps((size_t)n_gpu, nullptr);
@@ -1279,6 +1399,16 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             Ls[d].check(qm_index_attach_bwa(Ls[d].ctx, idxs[d], bwt_file.data(), (int64_t)bwt_file.size(), sa_file.data(), (int64_t)sa_file.size()), "qm_index_attach_bwa");
         else if (fm_build) Ls[d].check(qm_index_build_fm(Ls[d].ctx, idxs[d], g.codes.data()), "qm_index_build_fm");
         Ls[d].check(qm_sample_begin(Ls[d].ctx, idxs[d], &opt, &popt, &smps[d]), "qm_sample_begin");
+    }
+    for (auto &ps : passes) {
+        ps.idxs.assign((size_t)n_gpu, nullptr);
+        ps.smps.assign((size_t)n_gpu, nullptr);
+        for (int d = 0; d < n_gpu; ++d) {
+            Ls[d].check(qm_index_build(Ls[d].ctx, ps.g.codes.data(), (int)ps.g.names.size(), ps.g.lens.data(), pass_opt.min_seed_len, &ps.idxs[d]),
+                        "qm_index_build");
+            Ls[d].check(qm_sample_begin(Ls[d].ctx, ps.idxs[d], &pass_opt, &popt, &ps.smps[d]), "qm_sample_begin");
+            Ls[d].check(qm_sample_set_filter(ps.smps[d], 1), "qm_sample_set_filter");
+        }
     }
     qm_index *idx = idxs[0];
     pc.mark("context + reference + index");
@@ -1303,6 +1433,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     const bool keep = want_batches || decontam;       // records / reads needed after the batch loop
     FastqPairReader fr(a.get("r1"), a.get("r2"));
     std::deque<Batch> batches;                        // (a deque: the workers hold references while more batches arrive)
+    std::vector<int> batch_dev;                       // the GPU each of them went to
     std::vector<int64_t> first_read;
     RawBatch raw;
     int64_t n_pairs = 0, kept = 0;
@@ -1321,10 +1452,144 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     };
     int64_t n_batches = 0;
     const auto t_loop = std::chrono::steady_clock::now();
-    while (read_batch(fr, batch_pairs, raw)) {
+    if (!passes.empty()) {
+        // Stage s < P is contaminant pass s + 1, stage P the target.  Each stage fixes its insert-size model from the first batch it
+        // gets, which must hold QM_PESTAT_PAIRS pairs or the whole rest of its input, as the stage's first FASTQ batch in the chain
+        // does.  Until every stage has had such a batch the raw batches run here on GPU 0, and what a stage still without a model
+        // receives waits in pend[s] (carried over to the next raw batch); then the models go to every GPU and each raw batch runs all
+        // stages on its own GPU's worker while the next one is read.
+        const int P = (int)passes.size();
+        std::vector<std::vector<Batch>> pend((size_t)P + 1);
+        std::vector<int64_t> pend_n((size_t)P + 1, 0), n_in((size_t)P + 1, 0);
+        std::vector<bool> fixed((size_t)P + 1, false);
+        const std::string c1 = a.get("clean-r1"), c2 = a.get("clean-r2");
+        FILE *fc1 = nullptr, *fc2 = nullptr;
+        if (!c1.empty()) {
+            fc1 = fopen(c1.c_str(), "w"); fc2 = fopen(c2.c_str(), "w");
+            if (!fc1 || !fc2) die(2, "cannot create %s / %s", c1.c_str(), c2.c_str());
+        }
+        // a pass on GPU d: `in` aligned with pair ids from id0, its kept pairs gathered into `out`, `in` released
+        auto run_pass = [&](int d, int s, Batch &in, int64_t id0, Batch &out) {
+            std::vector<uint8_t> kb((size_t)in.n_pairs);
+            if (in.n_pairs > 0) {
+                qm_sample *ps = passes[(size_t)s].smps[(size_t)d];
+                Ls[d].check(qm_sample_add_pairs_host_packed(ps, in.bases2, in.nmask, in.quals, in.stride, in.lens, in.n_pairs, id0, nullptr),
+                            "qm_sample_add_pairs_host_packed");
+                Ls[d].check(qm_sample_keep_host(ps, kb.data(), in.n_pairs, nullptr), "qm_sample_keep_host");
+            }
+            gather_pairs(Ls[d], {&in}, {kb.data()}, out);
+            free_batch(Ls[d], in);
+        };
+        // the target on GPU d: records as `sample` keeps them; the batch is then stored (BAM / text pileup) or released
+        auto run_target = [&](int d, Batch &b, int64_t id0) {
+            void *p = nullptr;
+            if (keep) { Ls[d].check(qm_host_alloc(Ls[d].ctx, (size_t)2 * b.n_pairs * sizeof(qm_aln), &p), "qm_host_alloc"); b.alns = (qm_aln *)p; }
+            if (b.n_pairs > 0)
+                Ls[d].check(qm_sample_add_pairs_host_packed(smps[d], b.bases2, b.nmask, b.quals, b.stride, b.lens, b.n_pairs, id0, b.alns),
+                            "qm_sample_add_pairs_host_packed");
+        };
+        auto write_clean = [&](const Batch &b) { if (fc1) for (int64_t p = 0; p < b.n_pairs; ++p) write_fastq_pair(fc1, fc2, b, p); };
+        auto store = [&](int d, Batch &b, Batch *slot) {
+            if (slot) *slot = std::move(b);
+            else free_batch(Ls[d], b);
+        };
+        // startup (GPU 0): `cur` enters stage s (eof: no more input, a stage without a model takes what it has)
+        auto advance = [&](int s, Batch cur, bool has, bool eof) {
+            for (; s <= P; ++s) {
+                if (!fixed[(size_t)s]) {
+                    if (has) { pend_n[(size_t)s] += cur.n_pairs; pend[(size_t)s].push_back(std::move(cur)); }
+                    if (pend_n[(size_t)s] < QM_PESTAT_PAIRS && !eof) return;
+                    std::vector<Batch> &q = pend[(size_t)s];
+                    if (q.empty()) return;
+                    if (q.size() == 1) cur = std::move(q[0]);
+                    else {
+                        std::vector<const Batch *> src;
+                        for (auto &x : q) src.push_back(&x);
+                        Batch m;
+                        gather_pairs(L, src, std::vector<const uint8_t *>(q.size(), nullptr), m);
+                        for (auto &x : q) free_batch(L, x);
+                        cur = std::move(m);
+                        const std::string stage = s < P ? "pass " + std::to_string(s + 1) : std::string("the target");
+                        fprintf(stderr, "[qm_driver] decontam: the first batch of %s (%lld pairs) carries over the pairs of %zu raw batches\n",
+                                stage.c_str(), (long long)cur.n_pairs, q.size());
+                    }
+                    q.clear();
+                    pend_n[(size_t)s] = 0;
+                    fixed[(size_t)s] = true;
+                    has = true;
+                }
+                const int64_t id0 = n_in[(size_t)s];
+                n_in[(size_t)s] += cur.n_pairs;
+                if (s < P) {
+                    Batch out;
+                    run_pass(0, s, cur, id0, out);
+                    cur = std::move(out);
+                } else {
+                    Batch *slot = nullptr;
+                    if (want_batches) { batches.emplace_back(); batch_dev.push_back(0); slot = &batches.back(); }
+                    run_target(0, cur, id0);
+                    write_clean(cur);
+                    store(0, cur, slot);
+                }
+            }
+        };
+        Ledger ledger;
+        int64_t n_par = 0;                              // raw batches run by the workers
+        while (read_batch(fr, batch_pairs, raw)) {
+            const bool startup = !std::all_of(fixed.begin(), fixed.end(), [](bool f) { return f; });
+            const int d = startup ? 0 : batch_gpu(n_batches, n_gpu);
+            join_worker(d);
+            Batch b;
+            pack_batch(Ls[d], raw, false, b);
+            ++n_batches;
+            if (startup) {
+                advance(0, std::move(b), true, false);
+                if (std::all_of(fixed.begin(), fixed.end(), [](bool f) { return f; })) {
+                    // every stage has its model: every GPU gets it, the ledger starts where the startup left off
+                    for (int s = 0; s <= P && n_gpu > 1; ++s) {
+                        qm_sample *s0 = s < P ? passes[(size_t)s].smps[0] : smp;
+                        qm_pestat pes[4];
+                        L.check(qm_sample_get_pestat(s0, pes), "qm_sample_get_pestat");
+                        for (int e = 1; e < n_gpu; ++e)
+                            Ls[e].check(qm_sample_set_pestat(s < P ? passes[(size_t)s].smps[(size_t)e] : smps[e], pes), "qm_sample_set_pestat");
+                    }
+                    ledger.turn.assign((size_t)P + 2, 0);
+                    ledger.total = n_in;
+                    ledger.total.push_back(0);
+                }
+                continue;
+            }
+            Batch *slot = nullptr;
+            if (want_batches) { batches.emplace_back(); batch_dev.push_back(d); slot = &batches.back(); }
+            const int64_t j = n_par++;
+            workers[d] = std::thread([&, d, j, slot, cur = std::move(b)]() mutable {
+                for (int s = 0; s < P; ++s) {
+                    const int64_t id0 = ledger.take(s, j, cur.n_pairs);
+                    Batch out;
+                    run_pass(d, s, cur, id0, out);
+                    cur = std::move(out);
+                }
+                run_target(d, cur, ledger.take(P, j, cur.n_pairs));
+                ledger.begin(P + 1, j);
+                write_clean(cur);
+                ledger.end(P + 1, 0);
+                store(d, cur, slot);
+            });
+        }
+        for (int d = 0; d < n_gpu; ++d) join_worker(d);
+        if (n_par > 0) n_in.assign(ledger.total.begin(), ledger.total.begin() + P + 1);
+        else for (int s = 0; s <= P; ++s) if (!fixed[(size_t)s]) { advance(s, Batch(), false, true); break; }
+        if (fc1 && (fclose(fc1) != 0 || fclose(fc2) != 0)) die(2, "write error on %s / %s", c1.c_str(), c2.c_str());
+        for (int s = 0; s < P; ++s)
+            fprintf(stderr, "[qm_driver] decontam pass %d: %lld of %lld pairs kept\n", s + 1, (long long)n_in[(size_t)s + 1], (long long)n_in[(size_t)s]);
+        n_pairs = n_in[(size_t)P];
+        int64_t r0 = 0;
+        for (auto &b : batches) { first_read.push_back(r0); r0 += 2 * b.n_pairs; }
+    } else while (read_batch(fr, batch_pairs, raw)) {
         const int d = batch_gpu(n_batches, n_gpu);
         join_worker(d);
         batches.emplace_back();
+        batch_dev.push_back(d);
         Batch &b = batches.back();
         pack_batch(Ls[d], raw, keep, b);
         const int64_t pair0 = n_pairs;
@@ -1359,7 +1624,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         n_pairs += b.n_pairs;
         ++n_batches;
         if (!want_batches && in_flight[d] == nullptr) { free_batch(Ls[d], b); }
-        if (!want_batches && n_gpu == 1 && in_flight[d] == nullptr) batches.pop_back();
+        if (!want_batches && n_gpu == 1 && in_flight[d] == nullptr) { batches.pop_back(); batch_dev.pop_back(); }
     }
     for (int d = 0; d < n_gpu; ++d) join_worker(d);
     const double loop_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_loop).count();
@@ -1410,7 +1675,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         if (want_batches) {                            // final flags of every record, batch by batch, from the GPU that held the batch
             std::vector<int64_t> bp;
             for (auto &b : batches) bp.push_back(b.n_pairs);
-            const auto src = batch_sources(bp, n_gpu);
+            const auto src = batch_sources(bp, batch_dev, n_gpu);
             std::vector<std::vector<qm_aln>> all((size_t)n_gpu);
             for (size_t i = 0; i < bp.size(); ++i) all[(size_t)src[i].first].resize((size_t)(src[i].second + 2 * bp[i]));
             for (int d = 0; d < n_gpu; ++d)
@@ -1479,6 +1744,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     }
     for (auto &b : batches) free_batch(L, b);
     for (int d = 0; d < n_gpu; ++d) {
+        for (auto &ps : passes) { qm_sample_destroy(ps.smps[(size_t)d]); qm_index_destroy(Ls[d].ctx, ps.idxs[(size_t)d]); }
         qm_sample_destroy(smps[d]);
         qm_index_destroy(Ls[d].ctx, idxs[d]);
         qm_ctx_destroy(Ls[d].ctx);

@@ -46,6 +46,12 @@ struct qm_sample {
     int max_depth = 0;                            // > 0: `bcftools mpileup -d` depth cap (qm_sample_set_max_depth): deferred counting too
     int baq = 0;                                  // 1 / 3: base alignment quality (plain / extended) caps the qualities the pileup sees (qm_sample_set_baq)
     bool rmdup_finished = false;                  // qm_sample_rmdup_finish has run: no more pairs, no second finish until a reset
+    // filter mode (qm_sample_set_filter): align and finish pairs, count nothing; the keep rule's byte per pair of the last batch
+    // (qm_sample_keep_host) lands in d_keep, the number of kept pairs in d_n_kept
+    bool filter = false;
+    uint8_t *d_keep = nullptr;
+    unsigned long long *d_n_kept = nullptr;
+    int64_t keep_cap = 0, last_n = -1;
     struct Kept { uint8_t *codes, *quals; int32_t *lens; qm_aln *alns; int64_t n; int32_t stride; int64_t pair0; };   // pair0: id of the first pair
     std::vector<Kept> kept;
 };
@@ -86,6 +92,40 @@ cudaError_t qm_unpack_reads_launch(const uint8_t *d_bases2, const uint8_t *d_nma
 
 namespace {
 
+// rules/decontamination.smk:15-17,43-48 (`samtools view -f 12 -F 256` on the records of a pair, then `bedtools bamtofastq`, which
+// re-emits a pair only when both of its records passed): keep[p] = 1 iff both records are unmapped with an unmapped mate and neither
+// is secondary.  One thread per pair; the warp's kept pairs go to *n_kept in one atomic.
+__global__ void __launch_bounds__(256)
+keep_pairs_kernel(const qm_aln *__restrict__ alns, int64_t n_pairs, uint8_t *__restrict__ keep, unsigned long long *__restrict__ n_kept)
+{
+    const int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    bool k = false;
+    if (p < n_pairs) {
+        const unsigned f0 = alns[2 * p].flag, f1 = alns[2 * p + 1].flag;
+        k = (f0 & 12u) == 12u && !(f0 & 256u) && (f1 & 12u) == 12u && !(f1 & 256u);
+        keep[p] = (uint8_t)k;
+    }
+    const unsigned b = __ballot_sync(0xffffffffu, k);
+    if ((threadIdx.x & 31) == 0 && b) atomicAdd(n_kept, (unsigned long long)__popc(b));
+}
+
+// start of a batch in filter mode: room for its keep bytes, the kept count zeroed on the batch's stream
+int filter_begin(qm_sample *s, int64_t n_pairs, cudaStream_t st)
+{
+    if (!s->filter) return QM_OK;
+    qm_ctx *ctx = s->ctx;
+    if (n_pairs > s->keep_cap) {
+        QM_CUDA(ctx, cudaDeviceSynchronize());      // the last batch may still be writing the old buffer on another stream
+        QM_CUDA(ctx, cudaFree(s->d_keep));
+        s->d_keep = nullptr; s->keep_cap = 0;
+        QM_CUDA(ctx, cudaMalloc(&s->d_keep, (size_t)n_pairs));
+        s->keep_cap = n_pairs;
+    }
+    QM_CUDA(ctx, cudaMemsetAsync(s->d_n_kept, 0, sizeof(unsigned long long), st));
+    s->last_n = n_pairs;
+    return QM_OK;
+}
+
 // the qualities the pileup sees: the reads' own, or (qm_sample_set_baq) capped by their base alignment quality
 int sample_pileup_quals(qm_sample *s, const qm_aln *alns, const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
                         int64_t n_reads, cudaStream_t st, const uint8_t **out)
@@ -103,8 +143,9 @@ int sample_pileup_quals(qm_sample *s, const qm_aln *alns, const uint8_t *d_codes
 
 // quals_ready (may be NULL): event after which d_quals is valid; only the pileup reads the qualities, so their copy
 // may still be in flight while the reads are being aligned
+// keep_off: the chunk's first pair within its batch (filter mode: where its keep bytes go)
 int sample_chunk(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
-                 int64_t n, int64_t pair_id0, qm_aln *d_alns_out, cudaStream_t st, cudaEvent_t quals_ready = nullptr)
+                 int64_t n, int64_t pair_id0, int64_t keep_off, qm_aln *d_alns_out, cudaStream_t st, cudaEvent_t quals_ready = nullptr)
 {
     qm_ctx *ctx = s->ctx;
     // the pileup stages a pair's reads in 512-byte rows and would leave longer reads out of the counts without a word
@@ -130,6 +171,12 @@ int sample_chunk(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_quals, i
     qm_aln *alns = d_alns_out ? d_alns_out : s->d_alns;
     rc = qm_pair_finish(ctx, s->idx, &s->opt, d_codes, stride, d_lens, n, pair_id0, s->d_regs, s->d_n_regs, s->pes, alns, st);
     if (rc) return rc;
+    if (s->filter) {
+        keep_pairs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(alns, n, s->d_keep + keep_off, s->d_n_kept);
+        QM_CUDA(ctx, cudaGetLastError());
+        s->n_pairs += n;
+        return QM_OK;
+    }
     if (s->rmdup || s->max_depth > 0) {
         // keep the chunk for qm_sample_rmdup_finish: duplicates are a property of the whole sample
         qm_sample::Kept k = {nullptr, nullptr, nullptr, nullptr, n, stride, pair_id0};
@@ -174,6 +221,7 @@ int qm_sample_begin(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const q
     cudaError_t e;
     if ((e = cudaMalloc(&s->d_counts, (size_t)QM_NCH * idx->v.l_pac * sizeof(int32_t))) != cudaSuccess ||
         (e = cudaMalloc(&s->d_cells, 8)) != cudaSuccess ||
+        (e = cudaMalloc(&s->d_n_kept, sizeof(unsigned long long))) != cudaSuccess ||
         (e = cudaMalloc(&s->d_regs, (size_t)2 * kChunkPairs * QM_MAX_REGS * sizeof(qm_reg))) != cudaSuccess ||
         (e = cudaMalloc(&s->d_n_regs, (size_t)2 * kChunkPairs * sizeof(int32_t))) != cudaSuccess ||
         (e = cudaMalloc(&s->d_alns, (size_t)2 * kChunkPairs * sizeof(qm_aln))) != cudaSuccess ||
@@ -207,6 +255,7 @@ void qm_sample_destroy(qm_sample *s)
     free_kept(s);
     qm_indel_table_destroy(s->indels);
     cudaFree(s->d_counts); cudaFree(s->d_cells); cudaFree(s->d_regs); cudaFree(s->d_n_regs); cudaFree(s->d_alns);
+    cudaFree(s->d_keep); cudaFree(s->d_n_kept);
     for (int i = 0; i < 2; ++i) {
         cudaFree(s->d_stage[i]);
         if (s->ev_copied[i]) cudaEventDestroy(s->ev_copied[i]);
@@ -226,7 +275,7 @@ int qm_sample_reset(qm_sample *s, void *stream)
     QM_CUDA(ctx, cudaMemsetAsync(s->d_counts, 0, (size_t)QM_NCH * s->idx->v.l_pac * sizeof(int32_t), (cudaStream_t)stream));
     QM_CUDA(ctx, cudaMemsetAsync(s->d_cells, 0, 8, (cudaStream_t)stream));
     { const int rc = qm_indel_table_reset(s->indels, stream); if (rc) return rc; }
-    s->have_pes = false; s->n_pairs = 0; s->rmdup_finished = false;
+    s->have_pes = false; s->n_pairs = 0; s->rmdup_finished = false; s->last_n = -1;
     if (!s->kept.empty()) { QM_CUDA(ctx, cudaStreamSynchronize((cudaStream_t)stream)); free_kept(s); }
     return QM_OK;
 }
@@ -236,6 +285,7 @@ int qm_sample_set_rmdup(qm_sample *s, int on)
 {
     if (!s) return QM_EINVAL;
     if (s->n_pairs != 0) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_rmdup: pairs were already added; reset the sample first");
+    if (on && s->filter) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_rmdup: the sample is in filter mode");
     s->rmdup = on != 0;
     return QM_OK;
 }
@@ -245,7 +295,35 @@ int qm_sample_set_max_depth(qm_sample *s, int max_depth)
 {
     if (!s || max_depth < 0) return QM_EINVAL;
     if (s->n_pairs != 0) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_max_depth: pairs were already added; reset the sample first");
+    if (max_depth > 0 && s->filter) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_max_depth: the sample is in filter mode");
     s->max_depth = max_depth;
+    return QM_OK;
+}
+
+// Filter mode (a contaminant pass of `sample --decontam`): pairs are aligned and finished as usual, CIGAR stage included (a CIGAR
+// overflow unmaps a read), but nothing is counted and nothing is kept across batches; each batch leaves one keep byte per pair.
+int qm_sample_set_filter(qm_sample *s, int on)
+{
+    if (!s) return QM_EINVAL;
+    if (s->n_pairs != 0) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_filter: pairs were already added; reset the sample first");
+    if (on && (s->rmdup || s->max_depth > 0)) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_filter: the sample defers its counting (rmdup / depth cap)");
+    s->filter = on != 0;
+    return QM_OK;
+}
+
+// the keep bytes of the last batch a filter-mode sample was given, and how many pairs they keep; synchronous
+int qm_sample_keep_host(qm_sample *s, uint8_t *h_keep, int64_t n_pairs, int64_t *h_n_kept)
+{
+    if (!s || n_pairs < 0 || (n_pairs > 0 && !h_keep)) return QM_EINVAL;
+    qm_ctx *ctx = s->ctx;
+    if (!s->filter) return qm_fail(ctx, QM_EINVAL, "qm_sample_keep_host: the sample is not in filter mode (qm_sample_set_filter)");
+    if (n_pairs != s->last_n) return qm_fail(ctx, QM_EINVAL, "qm_sample_keep_host: the last batch had %lld pairs, not %lld", (long long)s->last_n, (long long)n_pairs);
+    QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    QM_CUDA(ctx, cudaDeviceSynchronize());          // the batch may have been added on any stream
+    unsigned long long nk = 0;
+    if (n_pairs > 0) QM_CUDA(ctx, cudaMemcpy(h_keep, s->d_keep, (size_t)n_pairs, cudaMemcpyDeviceToHost));
+    QM_CUDA(ctx, cudaMemcpy(&nk, s->d_n_kept, sizeof nk, cudaMemcpyDeviceToHost));
+    if (h_n_kept) *h_n_kept = (int64_t)nk;
     return QM_OK;
 }
 
@@ -526,9 +604,10 @@ int qm_sample_add_pairs(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_q
 {
     if (!s || n_pairs < 0 || (n_pairs > 0 && (!d_codes || !d_quals || !d_lens)) || stride <= 0) return QM_EINVAL;
     QM_CUDA(s->ctx, cudaSetDevice(s->ctx->device));
+    { const int rc = filter_begin(s, n_pairs, (cudaStream_t)stream); if (rc) return rc; }
     for (int64_t p0 = 0; p0 < n_pairs; p0 += kChunkPairs) {
         const int64_t n = n_pairs - p0 < kChunkPairs ? n_pairs - p0 : kChunkPairs;
-        int rc = sample_chunk(s, d_codes + 2 * p0 * stride, d_quals + 2 * p0 * stride, stride, d_lens + 2 * p0, n, pair_id0 + p0,
+        int rc = sample_chunk(s, d_codes + 2 * p0 * stride, d_quals + 2 * p0 * stride, stride, d_lens + 2 * p0, n, pair_id0 + p0, p0,
                               d_alns ? d_alns + 2 * p0 : nullptr, (cudaStream_t)stream);
         if (rc) return rc;
     }
@@ -543,9 +622,10 @@ static int add_pairs_host_impl(qm_sample *s, const uint8_t *h_codes, const uint8
 {
     const bool packed = h_codes == nullptr;
     if (!s || n_pairs < 0 || (n_pairs > 0 && ((packed ? (!h_bases2 || !h_nmask) : false) || !h_quals || !h_lens)) || stride <= 0) return QM_EINVAL;
-    if (n_pairs == 0) return QM_OK;
     qm_ctx *ctx = s->ctx;
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    { const int rc = filter_begin(s, n_pairs, ctx->own_stream); if (rc) return rc; }
+    if (n_pairs == 0) return QM_OK;
     const int stride_p = (stride + 3) >> 2, stride_m = (stride + 7) >> 3;
     const size_t seq_bytes = (size_t)2 * kChunkPairs * stride;
     const size_t seq_al = (seq_bytes + 255) & ~(size_t)255;
@@ -640,7 +720,7 @@ static int add_pairs_host_impl(qm_sample *s, const uint8_t *h_codes, const uint8
         if (packed) { ctx->se_pk = s->d_stage[b] + o_pk; ctx->se_mk = s->d_stage[b] + o_mk; ctx->se_sp = stride_p; ctx->se_sm = stride_m; }
         for (int pt = 0; pt < n_parts; ++pt) { ctx->se_part_end[pt] = 2 * n * (pt + 1) / n_parts; ctx->se_part_ev[pt] = s->ev_part[b][pt]; }
         int rc = sample_chunk(s, s->d_stage[b], s->d_stage[b] + seq_al, stride, (const int32_t *)(s->d_stage[b] + 2 * seq_al), n,
-                              pair_id0 + p0, nullptr, ks, s->ev_quals[b]);
+                              pair_id0 + p0, p0, nullptr, ks, s->ev_quals[b]);
         ctx->se_n_parts = 0; ctx->se_pk = ctx->se_mk = nullptr;
         if (rc) return rc;
         if (h_alns) QM_CUDA(ctx, cudaMemcpyAsync(h_alns + 2 * p0, s->d_alns, (size_t)2 * n * sizeof(qm_aln), cudaMemcpyDeviceToHost, ks));

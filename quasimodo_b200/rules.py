@@ -5,7 +5,8 @@ whose declared output is missing, so tests/test_rules_cpu.py checks these tables
 tests/test_driver_gpu.py checks that the command really writes every path.  pileup_commands gives rules `mpileup` and
 `bcftools` one `qm_driver pileup` job each, on the .rmdup.bam a separate alignment step left; rmdup_command gives rule `rmdup`
 one `qm_driver rmdup` job on the sorted BAM of any aligner; index_command gives rule `build_idx` (rules/index.smk:12-14) one
-`qm_driver index` job in place of `bwa index` + `samtools faidx`."""
+`qm_driver index` job in place of `bwa index` + `samtools faidx`; decontam_sample_command puts the decontamination rules
+`rm_phix` and `rm_human_ecoli` (rules/decontamination.smk) in front of the four in the same job."""
 import os
 
 # rule -> {output name ("" = the rule's single unnamed output): (directory variable, path pattern)}
@@ -107,6 +108,31 @@ def pileup_commands(driver, dirs, sample, ref_name, ref_fa, threads=4, extra=(),
             argv += ["--benchmark", b]
         out[rule] = (argv + list(extra), paths)
     return out
+
+
+# the cleaned FASTQ of the decontamination rules (rules/decontamination.smk:8-9,36-37): rm_phix writes the reads without PhiX,
+# rm_human_ecoli those without human and E. coli either; rule `bwa` reads the last
+CLEAN_FASTQ = {"rm_phix": ("seq_dir", "/cl_fq/{sample}.qc.nophix.r{mate}.fq"), "rm_human_ecoli": ("seq_dir", "/cl_fq/{sample}.qc.cl.r{mate}.fq")}
+
+
+def decontam_sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, phix_fa, human_ecoli_fa=(), threads=4, extra=(), benchmark=False):
+    """-> (argv, [every path the job writes]) of rules rm_phix [+ rm_human_ecoli] + bwa + rmdup + mpileup + bcftools as ONE
+    `qm_driver sample --decontam` job on the raw reads r1 / r2: sample_command's outputs plus the last pass's cleaned FASTQ (rule
+    rm_human_ecoli's when human_ecoli_fa names its genomes, else rule rm_phix's), the FASTQ the assemblers read.  With both passes
+    rule rm_phix's intermediate FASTQ is not written."""
+    argv, paths = sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads, benchmark=benchmark)
+    argv += ["--decontam", phix_fa]
+    last = "rm_phix"
+    if human_ecoli_fa:
+        argv += ["--decontam2", ",".join(human_ecoli_fa)]
+        last = "rm_human_ecoli"
+    var, pat = CLEAN_FASTQ[last]
+    for mate in (1, 2):
+        p = dirs[var] + pat.format(sample=sample, mate=mate)
+        os.makedirs(os.path.dirname(p), exist_ok=True)
+        argv += [f"--clean-r{mate}", p]
+        paths.append(p)
+    return argv + list(extra), paths
 
 
 # the files rule `build_idx` (rules/index.smk:12-14) leaves next to a genome X.fa: `bwa index X.fa` writes X.fa.{amb,ann,bwt,pac,sa}
