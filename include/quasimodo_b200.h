@@ -251,15 +251,25 @@ int qm_counts_to_rows(qm_ctx *ctx, const qm_index *idx, const int32_t *d_planes,
  * batch by batch, from device memory (qm_sample_add_pairs, asynchronous on `stream` except for the small
  * per-round read-backs) or from host memory (qm_sample_add_pairs_host: chunked, the next chunk's copy overlaps
  * the current chunk's kernels when the host buffers are page-locked; synchronous).
- * bwa estimates its insert-size model per input chunk (mem_pestat); here it is fixed ONCE per sample, from
+ * bwa estimates its insert-size model per input chunk (mem_pestat); by default it is fixed ONCE per sample, from
  * the first min(n, QM_PESTAT_PAIRS) pairs handed in, or from that prefix of the sample given explicitly
  * (qm_sample_estimate_pestat: a shard that does not start at pair 0 passes the sample's first pairs; every
  * GPU derives the same model, no collective), or set directly, so that the records do not depend on batching
  * or sharding.
+ * Per-chunk mode reproduces bwa instead: qm_sample_set_chunks(s, h_chunk_pairs, n_chunks) gives the sizes in pairs of the
+ * chunks of the NEXT add call (in order; they must add up to its n_pairs, QM_EINVAL there otherwise, so no chunk straddles two
+ * calls) and puts the sample in that mode for good (before its first pairs: QM_EINVAL after them; a reset keeps the mode).
+ * Each chunk's pairs are paired against mem_pestat over ALL of that chunk's pairs, estimated on the device; a chunk with too few
+ * pairs for an orientation fails it, as in bwa.  A chunk holds 1 .. QM_CHUNK_MAX_PAIRS pairs (QM_ELIMIT above).  Where chunks
+ * end is the caller's rule (bwa mem: bseq_read's running base count, -K); the records then depend neither on the batching nor on
+ * the GPUs, and no model crosses between GPUs.  qm_sample_set_pestat (bwa mem -I) still replaces every chunk's model.
+ * qm_sample_chunk_pestat: the models of the last add call's chunks, 4 per chunk, in order (*n_chunks of them; none when a model
+ * was set); with h_pes NULL and max_chunks 0 only *n_chunks.
  * Contract of the read arrays (every entry below): read r occupies row r of `stride` bytes, its length lens[r] lies in
  * [0, stride], stride <= 512 (QM_ELIMIT otherwise); the lengths are the caller's word -- the device entry cannot check them
  * without a pass over the data, the driver checks them while it parses FASTQ. */
 #define QM_PESTAT_PAIRS 65536
+#define QM_CHUNK_MAX_PAIRS (1 << 21)
 typedef struct qm_sample qm_sample;
 int  qm_sample_begin(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const qm_pileup_opt *popt, qm_sample **out);
 void qm_sample_destroy(qm_sample *s);
@@ -268,6 +278,8 @@ int  qm_sample_set_pestat(qm_sample *s, const qm_pestat pes[4]);
 int  qm_sample_get_pestat(const qm_sample *s, qm_pestat pes[4]);
 int  qm_sample_estimate_pestat(qm_sample *s, const uint8_t *d_codes, int32_t stride, const int32_t *d_lens, int64_t n_pairs,
                                void *stream);
+int  qm_sample_set_chunks(qm_sample *s, const int64_t *h_chunk_pairs, int64_t n_chunks);
+int  qm_sample_chunk_pestat(const qm_sample *s, qm_pestat *h_pes, int64_t max_chunks, int64_t *n_chunks);
 int  qm_sample_add_pairs(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride,
                          const int32_t *d_lens, int64_t n_pairs, int64_t pair_id0, qm_aln *d_alns /* may be NULL */,
                          void *stream);

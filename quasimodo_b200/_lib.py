@@ -109,6 +109,8 @@ SIGNATURES = {
     "qm_sample_set_pestat": (C.c_int, [_P, _P]),
     "qm_sample_get_pestat": (C.c_int, [_P, _P]),
     "qm_sample_estimate_pestat": (C.c_int, [_P, _P, _I, _P, _L, _P]),
+    "qm_sample_set_chunks": (C.c_int, [_P, _P, _L]),
+    "qm_sample_chunk_pestat": (C.c_int, [_P, _P, _L, C.POINTER(C.c_int64)]),
     "qm_sample_add_pairs": (C.c_int, [_P, _P, _P, _I, _P, _L, _L, _P, _P]),
     "qm_sample_add_pairs_host": (C.c_int, [_P, _P, _P, _I, _P, _L, _L, _P]),
     "qm_sample_add_pairs_host_packed": (C.c_int, [_P, _P, _P, _P, _I, _P, _L, _L, _P]),

@@ -178,6 +178,20 @@ class Sample:
         rc = _lib.lib().qm_sample_estimate_pestat(self._h, _ptr(d_codes), stride, _ptr(d_lens), n // 2, C.c_void_p(stream))
         _check(self.ctx._h, rc, "qm_sample_estimate_pestat")
 
+    def set_chunks(self, chunk_pairs):
+        """per-chunk mode (bwa mem's model per input chunk): the sizes in pairs of the next add call's chunks, which must add up
+        to its pairs; see qm_sample_set_chunks"""
+        c = np.ascontiguousarray(chunk_pairs, dtype=np.int64)
+        _check(self.ctx._h, _lib.lib().qm_sample_set_chunks(self._h, c.ctypes.data if len(c) else None, len(c)), "qm_sample_set_chunks")
+
+    def chunk_pestat(self):
+        """per-chunk mode: the models of the last add call's chunks, [n_chunks, 4] of PESTAT_DTYPE"""
+        n = C.c_int64()
+        _check(self.ctx._h, _lib.lib().qm_sample_chunk_pestat(self._h, None, 0, C.byref(n)), "qm_sample_chunk_pestat")
+        buf = np.zeros(4 * max(n.value, 1), dtype=_lib.PESTAT_DTYPE)
+        _check(self.ctx._h, _lib.lib().qm_sample_chunk_pestat(self._h, buf.ctypes.data, n.value, C.byref(n)), "qm_sample_chunk_pestat")
+        return buf[:4 * n.value].reshape(-1, 4)
+
     def add_pairs(self, d_codes, d_quals, d_lens, pair_id0=0, d_alns=None, stream=0):
         """device-resident batch: torch uint8 [2n, stride] codes / quals, int32 [2n] lens"""
         n, stride = d_codes.shape

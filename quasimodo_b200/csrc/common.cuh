@@ -25,8 +25,10 @@ struct qm_ctx {
     // scratch arenas grown on demand (never shrunk); index = purpose.  32-36: the tuples of duplicate marking and the depth cap
     // (dedup.cu, depthcap.cu, sort.cu, sample.cu);
     // 37-39: BAM records in (bamin.cu: staged record stream, file-order rows and pairing state, pair layout);
-    // 40-41: duplicate marking of a BAM (bamdup.cu: staged record stream and verdicts, per-record state and tuples)
-    qm_scratch scratch[42];
+    // 40-41: duplicate marking of a BAM (bamdup.cu: staged record stream and verdicts, per-record state and tuples);
+    // 42-43: per-chunk insert-size models (pair.cu qm_pestat_chunks: chunk starts, pair -> chunk map and models, read by
+    // qm_pair_finish_models after it; the histograms)
+    qm_scratch scratch[44];
     cudaStream_t own_stream = nullptr, copy_stream = nullptr;
     // side streams: the independent per-class extension kernels of one round run concurrently (fork/join by events)
     cudaStream_t side[12] = {};

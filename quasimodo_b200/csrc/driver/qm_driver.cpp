@@ -10,6 +10,9 @@
 //                      [-q / --min-mapq N] [-Q / --min-bq N] [--count-orphans 1] [--ignore-overlaps 1]: the mpileups' -q -Q -A -x
 //                      [--stage-ms 1: per-stage device time (CUDA events) of every GPU in the log]
 //                      [--benchmark FILE (every command): wall time, peak memory, I/O and CPU load as a Snakemake benchmark TSV]
+//                      [-K INT: bwa mem -K, input chunks of INT bases, each paired against its own insert-size model (mem_pestat over
+//                       all of its pairs), as bwa does; the default is one model per sample from its first QM_PESTAT_PAIRS pairs (DESIGN.md 5.3)]
+//                      [-I mean[,std[,max[,min]]]: bwa mem -I, the FR insert-size model given instead of estimated]
 //                      [--print-options 1: print the alignment options the command line resolves to and exit (host only)]
 //        an option the command does not know is a usage error
 //        --mpileup: the text pileup of `samtools mpileup -f ref bam` (rules/vcfcall.smk:39, input of the VarScan rule) with -B
@@ -25,7 +28,8 @@
 //        genome (its own index, filter-mode sample and insert-size model; bwa's options, not --bwa-index / --fm-seeds), the pairs
 //        whose records are both unmapped are gathered on the host, still packed, and go on to pass 2, then to the target, whose pair
 //        ids count the kept pairs.  Every output equals `decontam` (pass 1) | `decontam` (pass 2) | `sample` on the cleaned FASTQ,
-//        with --gpus too; --clean-r1/-r2 write that cleaned FASTQ.  Not with --keep-contigs
+//        with --gpus too; --clean-r1/-r2 write that cleaned FASTQ.  Not with --keep-contigs.  With -K every stage cuts bwa's chunks
+//        over its own input (pass 2 over pass 1's survivors, the target over pass 2's), on one GPU
 //        = rules/bwa.smk:15-18 (bwa mem | samtools view | samtools sort | samtools index -> BAM + BAI),
 //          rules/vcfcall.smk:39 (pileup path: count TSV, SURVEY.md B.3) and rules/vcfcall.smk:115-117 (VCF)
 //   qm_driver decontam --ref CONTAMINANT.fa[,MORE.fa] --r1 .. --r2 .. --out-r1 CLEAN1.fq --out-r2 CLEAN2.fq
@@ -54,8 +58,9 @@
 //          line lengths samtools faidx accepts, at most QM_MAX_CONTIGS contigs, 2 x length < 2^31)
 //   qm_driver bam-from-records --ref .. --r1 .. --r2 .. --alns ALNS.bin [--perm PERM.bin] --bam OUT.bam
 //        = the BAM/BAI writer alone on given qm_aln records (test entry; with --perm no GPU is touched)
-//   qm_driver fastq-check --r1 .. --r2 .. [-t THREADS]
-//        = the FASTQ side alone (host only): the two mate files parsed and validated as `sample` would, pairs / bases / parse rate
+//   qm_driver fastq-check --r1 .. --r2 .. [-t THREADS] [-K N [--batch-pairs M]]
+//        = the FASTQ side alone (host only): the two mate files parsed and validated as `sample` would, pairs / bases / parse rate;
+//          with -K the sizes in pairs of bwa mem's input chunks of N bases, cut as `sample -K N` cuts them
 //
 // Exit status: 0 ok, 1 usage, 2 I/O or format error, 3 library/CUDA error (message on stderr), so a failing job
 // fails its Snakemake rule exactly like a failing `bwa`.
@@ -220,6 +225,7 @@ struct Batch {
     qm_aln *alns = nullptr;
     std::string names;                                // NUL-separated, one per pair
     std::vector<uint32_t> name_off;
+    std::vector<int64_t> chunks;                      // -K: the sizes in pairs of bwa's input chunks the batch consists of
 };
 
 struct FastqPairReader {
@@ -263,39 +269,64 @@ template <class F> void parallel_ranges(size_t n, F fn)
     for (auto &th : pool) th.join();
 }
 
+// one FASTQ record appended to a side; false at the end of the file
+bool read_record(LineReader &r, Side &v)
+{
+    const char *p = nullptr;
+    size_t n = 0;
+    if (!r.next_view(p, n)) return false;
+    while (n == 0) if (!r.next_view(p, n)) return false;                // blank lines between records
+    if (p[0] != '@') die(2, "%s: FASTQ header expected, got '%.*s'", r.path.c_str(), (int)std::min<size_t>(n, 40), p);
+    // bwa: the name up to the first whitespace, a trailing /<digit> dropped (bwa.c trim_readno; SURVEY.md B.8)
+    size_t e = 1;
+    while (e < n && !isspace((unsigned char)p[e])) ++e;
+    if (e > 3 && p[e - 2] == '/' && isdigit((unsigned char)p[e - 1])) e -= 2;
+    v.noff.push_back((uint32_t)v.names.size());
+    v.names.insert(v.names.end(), p + 1, p + e);
+    v.names.push_back('\0');
+    if (!r.next_view(p, n)) die(2, "%s: truncated FASTQ record", r.path.c_str());
+    const size_t sl = n;
+    v.seq.insert(v.seq.end(), p, p + n);
+    if (!r.next_view(p, n)) die(2, "%s: truncated FASTQ record", r.path.c_str());
+    if (n == 0 || p[0] != '+') die(2, "%s: '+' line expected", r.path.c_str());
+    if (!r.next_view(p, n)) die(2, "%s: truncated FASTQ record", r.path.c_str());
+    if (n != sl) die(2, "%s: sequence and quality lengths differ in @%s", r.path.c_str(), v.names.data() + v.noff.back());
+    v.qual.insert(v.qual.end(), p, p + n);
+    v.soff.push_back((uint64_t)v.seq.size());
+    ++v.n;
+    return true;
+}
+
+// bwa mem's input chunks (-K): bseq_read (bwa.c, bwa 0.7.17 as recalled) reads pairs in order and adds both mates' lengths to a
+// running sum; a chunk ends after the first pair at which the sum reaches K, and the next one starts from zero.  *sum carries an
+// open chunk's sum into the next call; chunks gets the sizes (in pairs) of the chunks that end among pairs [from, n).
+void cut_chunks(const RawBatch &b, size_t from, int64_t K, int64_t *sum, int64_t *open, std::vector<int64_t> &chunks)
+{
+    for (size_t i = from; i < b.a.n; ++i) {
+        *sum += (int64_t)(b.a.len(i) + b.b.len(i));
+        ++*open;
+        if (*sum >= K) { chunks.push_back(*open); *sum = 0; *open = 0; }
+        else if (*open >= QM_CHUNK_MAX_PAIRS)
+            die(1, "option -K: a chunk of %lld bases runs past %d pairs, the most one chunk may hold (QM_CHUNK_MAX_PAIRS); choose a smaller -K",
+                (long long)K, QM_CHUNK_MAX_PAIRS);
+    }
+}
+
 // reads up to max_pairs pairs; mates are matched by file order (bwa's rule), not by name.  The two files are read (and
-// inflated) side by side: the second mate's file has a thread of its own.
-bool read_batch(FastqPairReader &fr, int64_t max_pairs, RawBatch &out)
+// inflated) side by side: the second mate's file has a thread of its own.  With K > 0 (bwa mem -K) the batch is then read on,
+// pair by pair, to the end of bwa's chunk it stops in, so that it holds whole chunks; *chunks gets their sizes in pairs (the
+// last one of the input is whatever remains).
+bool read_batch(FastqPairReader &fr, int64_t max_pairs, RawBatch &out, int64_t K = 0, std::vector<int64_t> *chunks = nullptr)
 {
     // a record's four lines are consumed as they are read (a view dies with the next read): one copy from the file buffer into the
     // side's arrays, no string per line
     auto side = [max_pairs](LineReader &r, Side &v) {
         v.clear();
-        const char *p = nullptr;
-        size_t n = 0;
         while ((int64_t)v.n < max_pairs) {
-            if (!r.next_view(p, n)) return;
-            while (n == 0) if (!r.next_view(p, n)) return;              // blank lines between records
-            if (p[0] != '@') die(2, "%s: FASTQ header expected, got '%.*s'", r.path.c_str(), (int)std::min<size_t>(n, 40), p);
-            // bwa: the name up to the first whitespace, a trailing /<digit> dropped (bwa.c trim_readno; SURVEY.md B.8)
-            size_t e = 1;
-            while (e < n && !isspace((unsigned char)p[e])) ++e;
-            if (e > 3 && p[e - 2] == '/' && isdigit((unsigned char)p[e - 1])) e -= 2;
-            v.noff.push_back((uint32_t)v.names.size());
-            v.names.insert(v.names.end(), p + 1, p + e);
-            v.names.push_back('\0');
-            if (!r.next_view(p, n)) die(2, "%s: truncated FASTQ record", r.path.c_str());
-            const size_t sl = n;
-            v.seq.insert(v.seq.end(), p, p + n);
-            if (!r.next_view(p, n)) die(2, "%s: truncated FASTQ record", r.path.c_str());
-            if (n == 0 || p[0] != '+') die(2, "%s: '+' line expected", r.path.c_str());
-            if (!r.next_view(p, n)) die(2, "%s: truncated FASTQ record", r.path.c_str());
-            if (n != sl) die(2, "%s: sequence and quality lengths differ in @%s", r.path.c_str(), v.names.data() + v.noff.back());
-            v.qual.insert(v.qual.end(), p, p + n);
-            v.soff.push_back((uint64_t)v.seq.size());
-            if (++v.n == 1 && max_pairs <= ((int64_t)1 << 23)) {
+            if (!read_record(r, v)) return;
+            if (v.n == 1 && max_pairs <= ((int64_t)1 << 23)) {
                 // the first record sizes the batch's arrays (address space only: no growth by doubling, no copies of what was read)
-                const size_t m = (size_t)max_pairs;
+                const size_t m = (size_t)max_pairs, sl = v.len(0);
                 v.seq.reserve(m * (sl + 1)); v.qual.reserve(m * (sl + 1));
                 v.names.reserve(m * (v.names.size() + 2)); v.soff.reserve(m + 1); v.noff.reserve(m);
             }
@@ -306,6 +337,17 @@ bool read_batch(FastqPairReader &fr, int64_t max_pairs, RawBatch &out)
     t2.join();
     if (out.a.n < out.b.n) die(2, "%s has more records than %s", fr.r2.path.c_str(), fr.r1.path.c_str());
     if (out.a.n > out.b.n) die(2, "%s has fewer records than %s", fr.r2.path.c_str(), fr.r1.path.c_str());
+    if (K > 0) {
+        chunks->clear();
+        int64_t sum = 0, open = 0;
+        cut_chunks(out, 0, K, &sum, &open, *chunks);
+        while (open > 0) {
+            const bool g1 = read_record(fr.r1, out.a), g2 = read_record(fr.r2, out.b);
+            if (g1 != g2) die(2, "%s has %s records than %s", fr.r2.path.c_str(), g1 ? "fewer" : "more", fr.r1.path.c_str());
+            if (!g1) { chunks->push_back(open); break; }
+            cut_chunks(out, out.a.n - 1, K, &sum, &open, *chunks);
+        }
+    }
     // bwa refuses mates whose names differ once /1 and /2 are dropped (bwamem_pair.c mem_sam_pe: "paired reads have different
     // names"): files that went out of step pair every read with a stranger and still align -- fail like bwa instead
     std::atomic<size_t> first_bad{out.a.n};
@@ -1104,6 +1146,48 @@ void apply_bwa_options(const Args &a, qm_opt &o)
     if (o.min_seed_len < 8 || o.min_seed_len > 31) die(1, "option -k: 8 <= k <= 31 (the k-mer index packs a seed into 62 bits)");
 }
 
+// bwa mem -K INT and -I mean[,std[,max[,min]]] (fastmap.c, bwa 0.7.17 as recalled).  -K: bwa's input chunks hold K bases
+// instead of 10^7 x threads, and each is paired against its own insert-size model (0: the driver's default, one model per sample
+// from its first QM_PESTAT_PAIRS pairs).  -I: the model is given, not estimated: only FR (pes[1]) is set, std defaults to
+// 0.1 x mean, high = (int)(mean + 4 std + .499), low = (int)(mean - 4 std + .499) clamped to >= 1 (bwa's rounding idiom), and an
+// explicit max and min replace them; the other three orientations fail.  bwa reads the fields with strtod and takes any
+// punctuation followed by a digit as the separator; what bwa would silently ignore (trailing text, a mean <= 0, min > max) is a
+// usage error here.
+struct PairOptions { int64_t K = 0; bool has_I = false; qm_pestat pes[4]; };
+
+PairOptions parse_pair_options(const Args &a)
+{
+    PairOptions r;
+    if (a.has("K")) {
+        const std::string v = a.get("K");
+        if (v.empty() || v.size() > 15 || v.find_first_not_of("0123456789") != std::string::npos || atoll(v.c_str()) < 1)
+            die(1, "option -K: '%s' is not a positive integer (bases per input chunk)", v.c_str());
+        r.K = atoll(v.c_str());
+    }
+    for (auto &pe : r.pes) { memset(&pe, 0, sizeof pe); pe.failed = 1; }
+    if (a.has("I")) {
+        const std::string v = a.get("I");
+        const char *q = v.c_str();
+        char *p = nullptr;
+        qm_pestat &f = r.pes[1];
+        auto bad = [&]() { die(1, "option -I: '%s' is not mean[,std[,max[,min]]]", v.c_str()); };
+        auto next_field = [&]() { return *p != 0 && ispunct((unsigned char)*p) && isdigit((unsigned char)p[1]); };
+        f.failed = 0;
+        f.avg = strtod(q, &p);
+        if (p == q || !(f.avg > 0) || !std::isfinite(f.avg)) bad();
+        f.std = f.avg * .1;
+        if (next_field()) f.std = strtod(p + 1, &p);
+        f.high = (int)(f.avg + 4. * f.std + .499);
+        f.low = (int)(f.avg - 4. * f.std + .499);
+        if (f.low < 1) f.low = 1;
+        if (next_field()) f.high = (int)(strtod(p + 1, &p) + .499);
+        if (next_field()) f.low = (int)(strtod(p + 1, &p) + .499);
+        if (*p != 0 || !(f.std >= 0) || !std::isfinite(f.std) || f.high < f.low || f.low < 0) bad();
+        r.has_I = true;
+    }
+    return r;
+}
+
 // the admission options of both mpileups (rules/vcfcall.smk:39,115 pass none: the defaults), under the tools' names:
 // -q / --min-mapq, -Q / --min-bq, --count-orphans 1 (-A), --ignore-overlaps 1 (-x)
 void apply_mpileup_options(const Args &a, qm_pileup_opt &p)
@@ -1115,11 +1199,14 @@ void apply_mpileup_options(const Args &a, qm_pileup_opt &p)
     if (p.min_mapq > 255 || p.min_bq > 93) die(1, "option -q is at most 255 and option -Q at most 93");
 }
 
-void print_options(const qm_opt &o, const qm_pileup_opt &p)
+void print_options(const qm_opt &o, const qm_pileup_opt &p, const PairOptions &po)
 {
     printf("q=%d Q=%d count-orphans=%d ignore-overlaps=%d ", p.min_mapq, p.min_bq, p.count_orphans, p.ignore_overlaps);
-    printf("A=%d B=%d O=%d,%d E=%d,%d L=%d,%d U=%d T=%d d=%d w=%d k=%d c=%d D=%g W=%d flags=%d\n", o.a, o.b, o.o_del, o.o_ins, o.e_del, o.e_ins,
+    printf("A=%d B=%d O=%d,%d E=%d,%d L=%d,%d U=%d T=%d d=%d w=%d k=%d c=%d D=%g W=%d flags=%d", o.a, o.b, o.o_del, o.o_ins, o.e_del, o.e_ins,
            o.pen_clip5, o.pen_clip3, o.pen_unpaired, o.T, o.zdrop, o.w, o.min_seed_len, o.max_occ, (double)o.drop_ratio, o.min_chain_weight, o.flags);
+    if (po.K) printf(" K=%lld", (long long)po.K);                     // -K / -I only when given
+    if (po.has_I) printf(" I=%.17g,%.17g,%d,%d", po.pes[1].avg, po.pes[1].std, po.pes[1].high, po.pes[1].low);
+    printf("\n");
 }
 
 std::vector<std::string> split(const std::string &s, char sep)
@@ -1315,7 +1402,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         "ref", "r1", "r2", "sample", "bam", "counts", "vcf", "vcf-gz", "out-r1", "out-r2", "keep-contigs", "gpu", "gpus", "t", "threads",
         "batch-pairs", "rmdup", "rmdup-bam", "metrics", "no-rescue", "mpileup", "bwa-index", "fm-seeds", "indels", "max-depth", "baq",
         "min-mapq", "q", "min-bq", "Q", "count-orphans", "ignore-overlaps", "min-dp", "min-alt", "min-af", "print-options", "stage-ms",
-        "w", "k", "c", "W", "D", "A", "B", "O", "E", "L", "U", "T", "d"};
+        "w", "k", "c", "W", "D", "A", "B", "O", "E", "L", "U", "T", "d", "K", "I"};
     if (!decontam) known.insert(known.end(), {"decontam", "decontam2", "clean-r1", "clean-r2"});
     require_known(a, decontam ? "decontam" : "sample", known);
     // --decontam A.fa[,B.fa] [--decontam2 C.fa[,D.fa]]: rules rm_phix and rm_human_ecoli in this job, in front of the target
@@ -1324,6 +1411,8 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     if (a.has("clean-r1") != a.has("clean-r2")) die(1, "--clean-r1 and --clean-r2 go together");
     if (a.has("clean-r1") && !a.has("decontam")) die(1, "--clean-r1 / --clean-r2 need --decontam");
     if (a.has("decontam") && a.has("keep-contigs")) die(1, "--decontam and --keep-contigs exclude each other (exact passes or the fused approximation)");
+    const PairOptions pair_opts = parse_pair_options(a);
+    const int64_t K = pair_opts.K;
     if (atoi(a.get("print-options", "0").c_str())) {   // host only: the alignment options this command line resolves to
         qm_opt o; qm_opt_default(&o);
         apply_bwa_options(a, o);
@@ -1331,7 +1420,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         if (a.has("bwa-index") || atoi(a.get("fm-seeds", "0").c_str())) o.flags |= QM_F_FM_SEEDS;
         qm_pileup_opt po; qm_pileup_opt_default(&po);
         apply_mpileup_options(a, po);
-        print_options(o, po);
+        print_options(o, po, pair_opts);
         return 0;
     }
     if (!a.has("ref") || !a.has("r1") || !a.has("r2")) die(1, "--ref, --r1 and --r2 are required");
@@ -1363,6 +1452,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             for (size_t j = 0; j < i; ++j) if (devs[j] == devs[i]) die(1, "--gpus: device %d is listed twice", devs[i]);
         }
         if (decontam && devs.size() > 1) die(1, "decontam runs on one GPU (--gpu I)");
+        if (K && a.has("decontam") && devs.size() > 1) die(1, "sample --decontam with -K runs on one GPU (--gpu I)");
     } else devs.push_back(atoi(a.get("gpu", "0").c_str()));
     const int n_gpu = (int)devs.size();
     std::vector<Lib> Ls((size_t)n_gpu);
@@ -1399,6 +1489,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             Ls[d].check(qm_index_attach_bwa(Ls[d].ctx, idxs[d], bwt_file.data(), (int64_t)bwt_file.size(), sa_file.data(), (int64_t)sa_file.size()), "qm_index_attach_bwa");
         else if (fm_build) Ls[d].check(qm_index_build_fm(Ls[d].ctx, idxs[d], g.codes.data()), "qm_index_build_fm");
         Ls[d].check(qm_sample_begin(Ls[d].ctx, idxs[d], &opt, &popt, &smps[d]), "qm_sample_begin");
+        if (pair_opts.has_I) Ls[d].check(qm_sample_set_pestat(smps[d], pair_opts.pes), "qm_sample_set_pestat");    // bwa mem -I
     }
     for (auto &ps : passes) {
         ps.idxs.assign((size_t)n_gpu, nullptr);
@@ -1408,6 +1499,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
                         "qm_index_build");
             Ls[d].check(qm_sample_begin(Ls[d].ctx, ps.idxs[d], &pass_opt, &popt, &ps.smps[d]), "qm_sample_begin");
             Ls[d].check(qm_sample_set_filter(ps.smps[d], 1), "qm_sample_set_filter");
+            if (pair_opts.has_I) Ls[d].check(qm_sample_set_pestat(ps.smps[d], pair_opts.pes), "qm_sample_set_pestat");
         }
     }
     qm_index *idx = idxs[0];
@@ -1436,6 +1528,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
     std::vector<int> batch_dev;                       // the GPU each of them went to
     std::vector<int64_t> first_read;
     RawBatch raw;
+    std::vector<int64_t> chunks;                      // -K: the chunks of the batch read last
     int64_t n_pairs = 0, kept = 0;
     FILE *f1 = nullptr, *f2 = nullptr;
     if (decontam) {
@@ -1473,6 +1566,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             std::vector<uint8_t> kb((size_t)in.n_pairs);
             if (in.n_pairs > 0) {
                 qm_sample *ps = passes[(size_t)s].smps[(size_t)d];
+                if (K) Ls[d].check(qm_sample_set_chunks(ps, in.chunks.data(), (int64_t)in.chunks.size()), "qm_sample_set_chunks");
                 Ls[d].check(qm_sample_add_pairs_host_packed(ps, in.bases2, in.nmask, in.quals, in.stride, in.lens, in.n_pairs, id0, nullptr),
                             "qm_sample_add_pairs_host_packed");
                 Ls[d].check(qm_sample_keep_host(ps, kb.data(), in.n_pairs, nullptr), "qm_sample_keep_host");
@@ -1484,6 +1578,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         auto run_target = [&](int d, Batch &b, int64_t id0) {
             void *p = nullptr;
             if (keep) { Ls[d].check(qm_host_alloc(Ls[d].ctx, (size_t)2 * b.n_pairs * sizeof(qm_aln), &p), "qm_host_alloc"); b.alns = (qm_aln *)p; }
+            if (b.n_pairs > 0 && K) Ls[d].check(qm_sample_set_chunks(smps[d], b.chunks.data(), (int64_t)b.chunks.size()), "qm_sample_set_chunks");
             if (b.n_pairs > 0)
                 Ls[d].check(qm_sample_add_pairs_host_packed(smps[d], b.bases2, b.nmask, b.quals, b.stride, b.lens, b.n_pairs, id0, b.alns),
                             "qm_sample_add_pairs_host_packed");
@@ -1533,6 +1628,65 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
                 }
             }
         };
+        // -K (GPU 0): every stage cuts bwa's chunks over its own input stream -- pass 1 over the FASTQ, pass 2 over pass 1's survivors,
+        // the target over pass 2's -- as the chain `decontam -K | decontam -K | sample -K` does.  What a stage receives waits in
+        // pend[s] (which always starts at a chunk start) until chunks close; the closed chunks run as one add call, the open one's
+        // pairs stay for the next batch; eof: the rest is the stage's last chunk.
+        auto advance_k = [&](int s, Batch cur, bool has, bool eof) {
+            for (; s <= P; ++s) {
+                std::vector<Batch> &q = pend[(size_t)s];
+                if (has && cur.n_pairs > 0) q.push_back(std::move(cur));
+                else if (has) free_batch(L, cur);
+                has = false;
+                std::vector<int64_t> chunks;
+                int64_t sum = 0, open = 0, done = 0;
+                for (const Batch &x : q)
+                    for (int64_t p = 0; p < x.n_pairs; ++p) {
+                        sum += x.lens[2 * p] + x.lens[2 * p + 1];
+                        ++open;
+                        if (sum >= K) { chunks.push_back(open); done += open; sum = 0; open = 0; }
+                        else if (open >= QM_CHUNK_MAX_PAIRS)
+                            die(1, "option -K: a chunk of %lld bases runs past %d pairs, the most one chunk may hold (QM_CHUNK_MAX_PAIRS); "
+                                   "choose a smaller -K", (long long)K, QM_CHUNK_MAX_PAIRS);
+                    }
+                if (eof && open) { chunks.push_back(open); done += open; open = 0; }
+                if (done == 0) { if (eof) continue; return; }
+                // the closed chunks' pairs as one batch, the open chunk's pairs as the new pend[s]
+                std::vector<const Batch *> src;
+                std::vector<std::vector<uint8_t>> head_mask(q.size()), rest_mask(q.size());
+                std::vector<const uint8_t *> hm, rm;
+                int64_t left = done;
+                for (size_t k = 0; k < q.size(); ++k) {
+                    src.push_back(&q[k]);
+                    head_mask[k].assign((size_t)q[k].n_pairs, 0);
+                    rest_mask[k].assign((size_t)q[k].n_pairs, 1);
+                    for (int64_t p = 0; p < q[k].n_pairs && left > 0; ++p, --left) { head_mask[k][(size_t)p] = 1; rest_mask[k][(size_t)p] = 0; }
+                    hm.push_back(head_mask[k].data()); rm.push_back(rest_mask[k].data());
+                }
+                Batch head, rest;
+                gather_pairs(L, src, hm, head);
+                if (open > 0) gather_pairs(L, src, rm, rest);
+                for (auto &x : q) free_batch(L, x);
+                q.clear();
+                pend_n[(size_t)s] = rest.n_pairs;
+                if (rest.n_pairs > 0) q.push_back(std::move(rest));
+                head.chunks = std::move(chunks);
+                const int64_t id0 = n_in[(size_t)s];
+                n_in[(size_t)s] += head.n_pairs;
+                if (s < P) {
+                    Batch out;
+                    run_pass(0, s, head, id0, out);
+                    cur = std::move(out);
+                    has = true;
+                } else {
+                    Batch *slot = nullptr;
+                    if (want_batches) { batches.emplace_back(); batch_dev.push_back(0); slot = &batches.back(); }
+                    run_target(0, head, id0);
+                    write_clean(head);
+                    store(0, head, slot);
+                }
+            }
+        };
         Ledger ledger;
         int64_t n_par = 0;                              // raw batches run by the workers
         while (read_batch(fr, batch_pairs, raw)) {
@@ -1542,6 +1696,7 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             Batch b;
             pack_batch(Ls[d], raw, false, b);
             ++n_batches;
+            if (K) { advance_k(0, std::move(b), true, false); continue; }
             if (startup) {
                 advance(0, std::move(b), true, false);
                 if (std::all_of(fixed.begin(), fixed.end(), [](bool f) { return f; })) {
@@ -1577,7 +1732,8 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
             });
         }
         for (int d = 0; d < n_gpu; ++d) join_worker(d);
-        if (n_par > 0) n_in.assign(ledger.total.begin(), ledger.total.begin() + P + 1);
+        if (K) advance_k(0, Batch(), false, true);
+        else if (n_par > 0) n_in.assign(ledger.total.begin(), ledger.total.begin() + P + 1);
         else for (int s = 0; s <= P; ++s) if (!fixed[(size_t)s]) { advance(s, Batch(), false, true); break; }
         if (fc1 && (fclose(fc1) != 0 || fclose(fc2) != 0)) die(2, "write error on %s / %s", c1.c_str(), c2.c_str());
         for (int s = 0; s < P; ++s)
@@ -1585,27 +1741,32 @@ int cmd_sample(const Args &a, const std::string &cmdline, bool decontam)
         n_pairs = n_in[(size_t)P];
         int64_t r0 = 0;
         for (auto &b : batches) { first_read.push_back(r0); r0 += 2 * b.n_pairs; }
-    } else while (read_batch(fr, batch_pairs, raw)) {
+    } else while (read_batch(fr, batch_pairs, raw, K, &chunks)) {
         const int d = batch_gpu(n_batches, n_gpu);
         join_worker(d);
         batches.emplace_back();
         batch_dev.push_back(d);
         Batch &b = batches.back();
         pack_batch(Ls[d], raw, keep, b);
+        // -K: the batch holds whole chunks of bwa's (read_batch), so whole chunks are dealt to the GPUs; each GPU estimates the
+        // models of its own chunks and none is broadcast
+        if (K) b.chunks = chunks;
         const int64_t pair0 = n_pairs;
         if (n_batches == 0 || decontam) {
             // (later batches go to a worker thread, also with one GPU: the next batch is read and packed while this one is on the device)
             // the first batch fixes the sample's insert-size model (its first QM_PESTAT_PAIRS pairs): every GPU gets that model
             // before it sees a batch of its own, so the records do not depend on the number of GPUs
+            if (K) L.check(qm_sample_set_chunks(smp, b.chunks.data(), (int64_t)b.chunks.size()), "qm_sample_set_chunks");
             L.check(qm_sample_add_pairs_host_packed(smp, b.bases2, b.nmask, b.quals, b.stride, b.lens, b.n_pairs, pair0, b.alns), "qm_sample_add_pairs_host_packed");
-            if (n_gpu > 1) {
+            if (n_gpu > 1 && !K) {
                 qm_pestat pes[4];
                 L.check(qm_sample_get_pestat(smp, pes), "qm_sample_get_pestat");
                 for (int e = 1; e < n_gpu; ++e) Ls[e].check(qm_sample_set_pestat(smps[e], pes), "qm_sample_set_pestat");
             }
         } else {
             in_flight[d] = &b;
-            workers[d] = std::thread([&Ls, &smps, d, &b, pair0]() {
+            workers[d] = std::thread([&Ls, &smps, d, &b, pair0, K]() {
+                if (K) Ls[d].check(qm_sample_set_chunks(smps[d], b.chunks.data(), (int64_t)b.chunks.size()), "qm_sample_set_chunks");
                 Ls[d].check(qm_sample_add_pairs_host_packed(smps[d], b.bases2, b.nmask, b.quals, b.stride, b.lens, b.n_pairs, pair0, b.alns), "qm_sample_add_pairs_host_packed");
             });
         }
@@ -2512,15 +2673,20 @@ int main(int argc, char **argv)
     if (cmd == "rmdup") return cmd_rmdup(a, cmdline);
     if (cmd == "index") return cmd_index(a);
     if (cmd == "fastq-check") {                        // host only: parse the two mate files as `sample` would, report what is there
-        require_known(a, "fastq-check", {"r1", "r2", "t", "threads"});
+        // -K N: bwa mem's input chunks of N bases as `sample -K N` cuts them, one line "chunks: size size ..." (pairs per chunk)
+        require_known(a, "fastq-check", {"r1", "r2", "t", "threads", "K", "batch-pairs"});
         if (!a.has("r1") || !a.has("r2")) die(1, "--r1 --r2 are required");
         g_threads = std::max(1, atoi(a.get("t", a.get("threads", "4")).c_str()));
+        const int64_t K = parse_pair_options(a).K;
+        const int64_t batch = std::max<int64_t>(1, atoll(a.get("batch-pairs", "2000000").c_str()));
         FastqPairReader fr(a.get("r1"), a.get("r2"));
         RawBatch raw;
         int64_t n_pairs = 0, bases = 0;
         size_t mx = 0;
+        std::vector<int64_t> chunks, all_chunks;
         const auto t0 = std::chrono::steady_clock::now();
-        while (read_batch(fr, 2000000, raw)) {
+        while (read_batch(fr, batch, raw, K, &chunks)) {
+            all_chunks.insert(all_chunks.end(), chunks.begin(), chunks.end());
             n_pairs += (int64_t)raw.size();
             bases += (int64_t)raw.a.seq.size() + (int64_t)raw.b.seq.size();
             for (const Side *sd : {&raw.a, &raw.b}) for (size_t i = 0; i < sd->n; ++i) mx = std::max(mx, sd->len(i));
@@ -2528,6 +2694,11 @@ int main(int argc, char **argv)
         const double dt = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         printf("%lld pairs, %lld bases, longest read %zu, parsed in %.2f s (%.3f M pairs/s)\n", (long long)n_pairs, (long long)bases, mx, dt,
                dt > 0 ? (double)n_pairs / dt / 1e6 : 0.0);
+        if (K) {
+            printf("chunks:");
+            for (int64_t c : all_chunks) printf(" %lld", (long long)c);
+            printf("\n");
+        }
         return 0;
     }
     if (cmd == "vcf-index") {                          // bgzip -c X > X.gz; tabix -p vcf X.gz  (host only: rules/vcfcall.smk:118-119, rules/genome_diff.smk:24-25)

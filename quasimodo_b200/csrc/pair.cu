@@ -18,9 +18,15 @@ constexpr int kSubnTabLen = 256;
 struct PairTables {
     const double *mapq_l;        // [kMapqTabLen]: l < coef_len ? 1 : log(coef_len)/log(l)
     const int *subn;             // [kSubnTabLen]: (int)(4.343*log(n+1)+.499)
-    const double *pair_term[4];  // per orientation: .721*log(2*erfc(|ns|/sqrt2))*a for dist = low..high
-    qm_pestat pes[4];
+    // insert-size models, 4 per model (FF FR RF RR); pair p uses model model_of[p] (model 0 when model_of is NULL: one model
+    // for the whole batch).  term + term_off[4 m + d]: .721*log(2*erfc(|ns|/sqrt2))*a of model m, orientation d, dist = low..high
+    const qm_pestat *pes;
+    const double *term;
+    const int64_t *term_off;
+    const int32_t *model_of;
 };
+
+__device__ __forceinline__ int pair_model(const PairTables &T, int64_t pi) { return T.model_of ? T.model_of[pi] : 0; }
 
 
 __device__ __forceinline__ uint64_t hash64(uint64_t key)
@@ -45,19 +51,88 @@ __device__ int cal_sub(const qm_opt &o, const qm_reg *a, int n)
     return j < n ? a[j].score : o.min_seed_len * o.a;
 }
 
-// insert-size histogram for mem_pestat: hist[dir][isize] += 1 for every qualifying pair
+// insert-size histogram for mem_pestat: hist[chunk][dir][isize] += 1 for every qualifying pair.  model_of (may be NULL: one
+// histogram) gives each pair's chunk; the launch covers the pairs of chunks c0.. and hist starts at chunk c0's.
 __global__ void pestat_hist_kernel(IndexView V, qm_opt o, const qm_reg *__restrict__ regs, const int32_t *__restrict__ n_regs,
-                                   int64_t n_pairs, unsigned *__restrict__ hist)
+                                   int64_t p0, int64_t n_pairs, const int32_t *__restrict__ model_of, int c0, unsigned *__restrict__ hist)
 {
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i >= n_pairs) return;
+    const int64_t i = p0 + blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= p0 + n_pairs) return;
     const qm_reg *r0 = regs + (2 * i) * QM_MAX_REGS, *r1 = regs + (2 * i + 1) * QM_MAX_REGS;
     const int n0 = n_regs[2 * i], n1 = n_regs[2 * i + 1];
     if (n0 && n1 && !(cal_sub(o, r0, n0) > 0.8 * r0[0].score) && !(cal_sub(o, r1, n1) > 0.8 * r1[0].score) &&
         r0[0].rid == r1[0].rid) {
         int64_t is;
         const int dir = qm_infer_dir(V.l_pac, r0[0].rb, r1[0].rb, &is);
-        if (is && is <= o.max_ins) atomicAdd(&hist[(int64_t)dir * (o.max_ins + 1) + is], 1u);
+        const int64_t c = model_of ? model_of[i] - c0 : 0;
+        if (is && is <= o.max_ins) atomicAdd(&hist[(c * 4 + dir) * (o.max_ins + 1) + is], 1u);
+    }
+}
+
+// pair p -> the chunk it belongs to (chunk c holds pairs start[c] .. start[c + 1] - 1)
+__global__ void chunk_of_kernel(const int64_t *__restrict__ start, int n_chunks, int64_t n_pairs, int32_t *__restrict__ model_of)
+{
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n_pairs) return;
+    int lo = 0, hi = n_chunks - 1;
+    while (lo < hi) { const int m = (lo + hi + 1) >> 1; if (start[m] <= i) lo = m; else hi = m - 1; }
+    model_of[i] = lo;
+}
+
+// mem_pestat over one histogram per chunk (bwamem_pair.c, bwa 0.7.17 as recalled): block = chunk, thread = orientation.
+// Each thread walks its bins in ascending order, the operation order of mem_pestat over its sorted list and of the host
+// replay in qm_pestat_sync.  The average's sum is a sum of integers (exact in any order); the variance's sum is not, so it
+// is added one pair at a time, as bwa adds it.  Then the orientations with fewer than 5 % of the best one's pairs fail.
+__global__ void __launch_bounds__(32)
+pestat_model_kernel(const unsigned *__restrict__ hist, int max_ins, int c0, qm_pestat *__restrict__ pes)
+{
+    __shared__ int64_t s_cnt[4];
+    const int d = threadIdx.x;
+    const int64_t bins = (int64_t)max_ins + 1;
+    qm_pestat r;
+    r.low = r.high = r.failed = r.pad = 0; r.avg = r.std = 0;
+    if (d < 4) {
+        const unsigned *q = hist + ((int64_t)blockIdx.x * 4 + d) * bins;
+        int64_t n = 0;
+        for (int64_t v = 0; v < bins; ++v) n += q[v];
+        s_cnt[d] = n;
+        if (n < 10) r.failed = 1;
+        else {
+            const int64_t k25 = (int)(.25 * n + .499), k75 = (int)(.75 * n + .499);
+            int p25 = (int)bins - 1, p75 = (int)bins - 1;
+            {
+                int64_t c = 0;
+                bool h25 = false;
+                for (int64_t v = 0; v < bins; ++v) {
+                    c += q[v];
+                    if (!h25 && c > k25) { p25 = (int)v; h25 = true; }
+                    if (c > k75) { p75 = (int)v; break; }
+                }
+            }
+            r.low = (int)(p25 - 2.0 * (p75 - p25) + .499);
+            if (r.low < 1) r.low = 1;
+            r.high = (int)(p75 + 2.0 * (p75 - p25) + .499);
+            int64_t x = 0, sum = 0;
+            for (int64_t v = r.low; v <= r.high && v < bins; ++v) { sum += (int64_t)q[v] * v; x += q[v]; }
+            r.avg = (double)sum / x;
+            for (int64_t v = r.low; v <= r.high && v < bins; ++v) {
+                const double dlt = ((double)v - r.avg) * ((double)v - r.avg);
+                for (unsigned c = 0; c < q[v]; ++c) r.std = __dadd_rn(r.std, dlt);
+            }
+            r.std = sqrt(r.std / x);
+            r.low = (int)(p25 - 3.0 * (p75 - p25) + .499);
+            r.high = (int)(p75 + 3.0 * (p75 - p25) + .499);
+            if (r.low > r.avg - 4.0 * r.std) r.low = (int)(r.avg - 4.0 * r.std + .499);
+            if (r.high < r.avg + 4.0 * r.std) r.high = (int)(r.avg + 4.0 * r.std + .499);
+            if (r.low < 1) r.low = 1;
+        }
+    }
+    __syncthreads();
+    if (d < 4) {
+        int64_t mx = 0;
+        for (int e = 0; e < 4; ++e) mx = s_cnt[e] > mx ? s_cnt[e] : mx;
+        if (!r.failed && s_cnt[d] < mx * 0.05) r.failed = 1;
+        pes[((int64_t)c0 + blockIdx.x) * 4 + d] = r;
     }
 }
 
@@ -126,9 +201,11 @@ __device__ __forceinline__ bool p128_gt(const P128 &a, const P128 &b) { return a
 
 // mem_pair.  Instead of materialising and sorting every candidate pair, keep the best two by (score, hash)
 // and count the near-best ones in a second pass over the same enumeration.
-__device__ int pair_up(const IndexView &V, const qm_opt &o, const PairTables &T, qm_reg *const a[2], const int n_pri[2],
+__device__ int pair_up(const IndexView &V, const qm_opt &o, const PairTables &T, int model, qm_reg *const a[2], const int n_pri[2],
                        uint64_t id, int *sub, int *n_sub, int z[2])
 {
+    const qm_pestat *pes = T.pes + 4 * model;
+    const int64_t *toff = T.term_off + 4 * model;
     P128 v[2 * QM_MAX_REGS];
     int nv = 0;
     const int64_t l_pac = V.l_pac;
@@ -152,15 +229,15 @@ __device__ int pair_up(const IndexView &V, const qm_opt &o, const PairTables &T,
         for (int i = 0; i < nv; ++i) {
             for (int r = 0; r < 2; ++r) {
                 const int dir = r << 1 | (int)(v[i].y >> 1 & 1);
-                if (T.pes[dir].failed) continue;
+                if (pes[dir].failed) continue;
                 const int which = r << 1 | ((int)(v[i].y & 1) ^ 1);
                 if (y[which] < 0) continue;
                 for (int k = y[which]; k >= 0; --k) {
                     if ((int)(v[k].y & 3) != which) continue;
                     const int64_t dist = (int64_t)v[i].x - (int64_t)v[k].x;
-                    if (dist > T.pes[dir].high) break;
-                    if (dist < T.pes[dir].low) continue;
-                    const double term = T.pair_term[dir][dist - T.pes[dir].low];
+                    if (dist > pes[dir].high) break;
+                    if (dist < pes[dir].low) continue;
+                    const double term = T.term[toff[dir] + (dist - pes[dir].low)];
                     int q = (int)((double)((v[i].y >> 32) + (v[k].y >> 32)) + term + .499);
                     if (q < 0) q = 0;
                     P128 u;
@@ -593,7 +670,7 @@ pair_decide_kernel(IndexView V, qm_opt o, PairTables T, const uint8_t *__restric
     mark_primary(o, n[0], a[0], id << 1 | 0);
     mark_primary(o, n[1], a[1], id << 1 | 1);
     n_pri[0] = n[0]; n_pri[1] = n[1];
-    if (n_pri[0] && n_pri[1] && (o_sc = pair_up(V, o, T, a, n_pri, id, &subo, &n_sub, z)) > 0) {
+    if (n_pri[0] && n_pri[1] && (o_sc = pair_up(V, o, T, pair_model(T, pi), a, n_pri, id, &subo, &n_sub, z)) > 0) {
         bool is_multi[2];
         for (int i = 0; i < 2; ++i) {
             int j;
@@ -1027,7 +1104,8 @@ pair_finish_kernel(IndexView V, PairTables T, int64_t n_pairs, const qm_reg *__r
         if (!paired_done && h0->rid == h1->rid && h0->rid >= 0) {
             int64_t dist;
             const int d = qm_infer_dir(V.l_pac, regs[(2 * pi) * QM_MAX_REGS].rb, regs[(2 * pi + 1) * QM_MAX_REGS].rb, &dist);
-            if (!T.pes[d].failed && dist >= T.pes[d].low && dist <= T.pes[d].high) extra_flag |= 2;
+            const qm_pestat &pe = T.pes[4 * pair_model(T, pi) + d];
+            if (!pe.failed && dist >= pe.low && dist <= pe.high) extra_flag |= 2;
         }
         finish_pair(h0, h1, extra_flag);
     }
@@ -1057,7 +1135,7 @@ int qm_pestat_sync(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const qm
         QM_CUDA(ctx, cudaMemsetAsync(p, 0, 4 * bins * sizeof(unsigned), st));
         const int tpb = 128;
         const int sp = qm_prof_begin(ctx, QM_ST_PAIR, st);
-        pestat_hist_kernel<<<(unsigned)((n_pairs + tpb - 1) / tpb), tpb, 0, st>>>(idx->v, *opt, d_regs, d_n_regs, n_pairs, (unsigned *)p);
+        pestat_hist_kernel<<<(unsigned)((n_pairs + tpb - 1) / tpb), tpb, 0, st>>>(idx->v, *opt, d_regs, d_n_regs, 0, n_pairs, nullptr, 0, (unsigned *)p);
         qm_prof_end(ctx, QM_ST_PAIR, sp, st, 1);
         QM_CUDA(ctx, cudaMemcpyAsync(h.data(), p, 4 * bins * sizeof(unsigned), cudaMemcpyDeviceToHost, st));
         QM_CUDA(ctx, cudaStreamSynchronize(st));
@@ -1099,18 +1177,68 @@ int qm_pestat_sync(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const qm
     return QM_OK;
 }
 
-int qm_pair_finish(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride,
-                   const int32_t *d_lens, int64_t n_pairs, int64_t pair_id0, qm_reg *d_regs, int32_t *d_n_regs,
-                   const qm_pestat pes[4], qm_aln *d_alns, void *stream)
+// Insert-size models of the chunks of a batch (bwa's mem_process_seqs: one mem_pestat per input chunk, over all of the chunk's
+// pairs).  Chunk c holds pairs h_start[c] .. h_start[c + 1] - 1.  Leaves the pair -> chunk map and the models on the device
+// (scratch 42: *d_model_of, *d_pes, valid until the next call) and the models in h_pes[4 n_chunks]; synchronous.
+int qm_pestat_chunks(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const qm_reg *d_regs, const int32_t *d_n_regs,
+                     const int64_t *h_start, int n_chunks, const int32_t **d_model_of, const qm_pestat **d_pes, qm_pestat *h_pes, void *stream)
 {
-    if (!ctx || !idx || !opt || !pes || n_pairs < 0 || (n_pairs > 0 && (!d_codes || !d_lens || !d_regs || !d_n_regs || !d_alns)))
+    if (!ctx || !idx || !opt || !h_start || n_chunks < 1 || !d_model_of || !d_pes || !h_pes) return QM_EINVAL;
+    if (opt->max_ins < 1 || opt->max_ins > (1 << 20)) return qm_fail(ctx, QM_ELIMIT, "qm_pestat_chunks: max_ins must be in [1, 2^20]");
+    QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t n_pairs = h_start[n_chunks];
+    // scratch 42: chunk starts | pair -> chunk | models
+    const size_t o_map = ((size_t)(n_chunks + 1) * 8 + 255) & ~(size_t)255;
+    const size_t o_pes = (o_map + (size_t)(n_pairs > 0 ? n_pairs : 1) * 4 + 255) & ~(size_t)255;
+    void *p = nullptr;
+    int rc = qm_scratch_reserve(ctx, 42, o_pes + (size_t)n_chunks * 4 * sizeof(qm_pestat), &p);
+    if (rc) return rc;
+    char *b = (char *)p;
+    int64_t *starts = (int64_t *)b;
+    int32_t *map = (int32_t *)(b + o_map);
+    qm_pestat *pes = (qm_pestat *)(b + o_pes);
+    QM_CUDA(ctx, cudaMemcpyAsync(starts, h_start, (size_t)(n_chunks + 1) * 8, cudaMemcpyHostToDevice, st));
+    const int tpb = 128;
+    const int sp = qm_prof_begin(ctx, QM_ST_PAIR, st);
+    if (n_pairs > 0) chunk_of_kernel<<<(unsigned)((n_pairs + 255) / 256), 256, 0, st>>>(starts, n_chunks, n_pairs, map);
+    // the histograms of up to 256 MB of chunks at a time ([chunk][4][max_ins + 1] counters)
+    const size_t per_chunk = (size_t)4 * (opt->max_ins + 1) * sizeof(unsigned);
+    const int group = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_chunks, ((size_t)256 << 20) / per_chunk));
+    void *h = nullptr;
+    rc = qm_scratch_reserve(ctx, 43, (size_t)group * per_chunk, &h);
+    if (rc) return rc;
+    for (int c0 = 0; c0 < n_chunks; c0 += group) {
+        const int c1 = std::min(n_chunks, c0 + group);
+        const int64_t p0 = h_start[c0], np = h_start[c1] - h_start[c0];
+        QM_CUDA(ctx, cudaMemsetAsync(h, 0, (size_t)(c1 - c0) * per_chunk, st));
+        if (np > 0)
+            pestat_hist_kernel<<<(unsigned)((np + tpb - 1) / tpb), tpb, 0, st>>>(idx->v, *opt, d_regs, d_n_regs, p0, np, map, c0, (unsigned *)h);
+        pestat_model_kernel<<<(unsigned)(c1 - c0), 32, 0, st>>>((const unsigned *)h, opt->max_ins, c0, pes);
+    }
+    qm_prof_end(ctx, QM_ST_PAIR, sp, st, 1 + 3 * ((n_chunks + group - 1) / group));
+    QM_CUDA(ctx, cudaGetLastError());
+    QM_CUDA(ctx, cudaMemcpyAsync(h_pes, pes, (size_t)n_chunks * 4 * sizeof(qm_pestat), cudaMemcpyDeviceToHost, st));
+    QM_CUDA(ctx, cudaStreamSynchronize(st));
+    *d_model_of = map; *d_pes = pes;
+    return QM_OK;
+}
+
+// qm_pair_finish with one insert-size model per chunk of the batch: h_pes[4 n_models] on the host (the pairing terms are
+// evaluated there), d_pes the same models on the device (NULL: uploaded here), d_model_of each pair's model (NULL: model 0)
+int qm_pair_finish_models(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride,
+                          const int32_t *d_lens, int64_t n_pairs, int64_t pair_id0, qm_reg *d_regs, int32_t *d_n_regs,
+                          const qm_pestat *h_pes, int n_models, const qm_pestat *d_pes, const int32_t *d_model_of, qm_aln *d_alns, void *stream)
+{
+    if (!ctx || !idx || !opt || !h_pes || n_models < 1 || n_pairs < 0 || (n_pairs > 0 && (!d_codes || !d_lens || !d_regs || !d_n_regs || !d_alns)))
         return QM_EINVAL;
     if (n_pairs == 0) return QM_OK;
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (!(opt->flags & QM_F_NO_RESCUE)) {
         const int sr = qm_prof_begin(ctx, QM_ST_RESCUE, st);
-        const int rr = qm_mate_rescue(ctx, idx, opt, d_codes, stride, d_lens, n_pairs, d_regs, d_n_regs, pes, nullptr, stream);
+        const int rr = qm_mate_rescue_models(ctx, idx, opt, d_codes, stride, d_lens, n_pairs, d_regs, d_n_regs, h_pes, n_models, d_pes, d_model_of,
+                                             nullptr, stream);
         qm_prof_end(ctx, QM_ST_RESCUE, sr, st, 3);
         if (rr) return rr;
     }
@@ -1120,22 +1248,26 @@ int qm_pair_finish(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
         tab[l] = l < opt->mapq_coef_len ? 1. : log((double)opt->mapq_coef_len) / log((double)l);
     std::vector<int> subn(kSubnTabLen);
     for (int n = 0; n < kSubnTabLen; ++n) subn[n] = (int)(4.343 * log((double)(n + 1)) + .499);
-    size_t term_off[4], n_term = 0;
-    for (int d = 0; d < 4; ++d) {
-        term_off[d] = n_term;
-        if (!pes[d].failed && pes[d].high >= pes[d].low) n_term += (size_t)(pes[d].high - pes[d].low + 1);
+    const int n_pes = 4 * n_models;
+    std::vector<int64_t> term_off((size_t)n_pes);
+    size_t n_term = 0;
+    for (int d = 0; d < n_pes; ++d) {
+        term_off[(size_t)d] = (int64_t)n_term;
+        if (!h_pes[d].failed && h_pes[d].high >= h_pes[d].low) n_term += (size_t)(h_pes[d].high - h_pes[d].low + 1);
     }
     std::vector<double> term(n_term + 1);
-    for (int d = 0; d < 4; ++d) {
-        if (pes[d].failed || pes[d].high < pes[d].low) continue;
-        for (int64_t dist = pes[d].low; dist <= pes[d].high; ++dist) {
-            const double ns = (dist - pes[d].avg) / pes[d].std;
-            term[term_off[d] + (size_t)(dist - pes[d].low)] = .721 * log(2. * erfc(fabs(ns) * M_SQRT1_2)) * opt->a;
+    for (int d = 0; d < n_pes; ++d) {
+        const qm_pestat &pe = h_pes[d];
+        if (pe.failed || pe.high < pe.low) continue;
+        for (int64_t dist = pe.low; dist <= pe.high; ++dist) {
+            const double ns = (dist - pe.avg) / pe.std;
+            term[term_off[(size_t)d] + (size_t)(dist - pe.low)] = .721 * log(2. * erfc(fabs(ns) * M_SQRT1_2)) * opt->a;
         }
     }
     // scratch 5: tables | counters | task list | per-warp global fallback for oversized direction matrices
     const int cig_blocks = ctx->sm_count * 3;                      // persistent: 3 blocks x 4 warps x 14 KB per SM
-    const size_t o_tab = 0, o_subn = o_tab + kMapqTabLen * 8, o_term = o_subn + kSubnTabLen * 4;
+    const size_t o_tab = 0, o_subn = o_tab + kMapqTabLen * 8, o_pes = o_subn + kSubnTabLen * 4;
+    const size_t o_toff = o_pes + (size_t)n_pes * sizeof(qm_pestat), o_term = o_toff + (size_t)n_pes * 8;
     const size_t o_misc = (o_term + term.size() * 8 + 255) & ~(size_t)255;
     const size_t o_tasks = o_misc + 256;
     const size_t o_left = (o_tasks + (size_t)2 * n_pairs * sizeof(CigTask) + 255) & ~(size_t)255;
@@ -1149,12 +1281,15 @@ int qm_pair_finish(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
     char *b = (char *)p;
     QM_CUDA(ctx, cudaMemcpyAsync(b + o_tab, tab.data(), kMapqTabLen * 8, cudaMemcpyHostToDevice, st));
     QM_CUDA(ctx, cudaMemcpyAsync(b + o_subn, subn.data(), kSubnTabLen * 4, cudaMemcpyHostToDevice, st));
+    QM_CUDA(ctx, cudaMemcpyAsync(b + o_pes, h_pes, (size_t)n_pes * sizeof(qm_pestat), cudaMemcpyHostToDevice, st));
+    QM_CUDA(ctx, cudaMemcpyAsync(b + o_toff, term_off.data(), (size_t)n_pes * 8, cudaMemcpyHostToDevice, st));
     QM_CUDA(ctx, cudaMemcpyAsync(b + o_term, term.data(), term.size() * 8, cudaMemcpyHostToDevice, st));
     QM_CUDA(ctx, cudaMemsetAsync(b + o_misc, 0, 256, st));
     QM_CUDA(ctx, cudaStreamSynchronize(st));      // the host vectors above go out of scope
     PairTables T;
     T.mapq_l = (const double *)(b + o_tab); T.subn = (const int *)(b + o_subn);
-    for (int d = 0; d < 4; ++d) { T.pair_term[d] = (const double *)(b + o_term) + term_off[d]; T.pes[d] = pes[d]; }
+    T.pes = (const qm_pestat *)(b + o_pes); T.term_off = (const int64_t *)(b + o_toff); T.term = (const double *)(b + o_term);
+    T.model_of = d_model_of;
     int *n_tasks = (int *)(b + o_misc), *cursor = (int *)(b + o_misc + 8), *err = (int *)(b + o_misc + 16);
     // task lists of 2 n_pairs slots each, see the launches below; counters n_list[0..8]
     int *n_list = (int *)(b + o_misc + 32), *lists = (int *)(b + o_left);
@@ -1218,6 +1353,14 @@ int qm_pair_finish(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
     QM_CUDA(ctx, cudaStreamSynchronize(st));
     if (h_err) return qm_fail(ctx, QM_ELIMIT, "qm_pair_finish: traceback scratch exhausted (code %d)", h_err);
     return QM_OK;
+}
+
+int qm_pair_finish(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride,
+                   const int32_t *d_lens, int64_t n_pairs, int64_t pair_id0, qm_reg *d_regs, int32_t *d_n_regs,
+                   const qm_pestat pes[4], qm_aln *d_alns, void *stream)
+{
+    if (!pes) return QM_EINVAL;
+    return qm_pair_finish_models(ctx, idx, opt, d_codes, stride, d_lens, n_pairs, pair_id0, d_regs, d_n_regs, pes, 1, nullptr, nullptr, d_alns, stream);
 }
 
 }  // extern "C"

@@ -236,3 +236,16 @@ extern "C" int qm_bam_mark_duplicates_hashbits(qm_ctx *ctx, const uint8_t *d_byt
 // sample.cu: packed reads (2 bits per base + N flags) -> one code byte per base, rows [0, n_reads)
 cudaError_t qm_unpack_reads_launch(const uint8_t *d_bases2, const uint8_t *d_nmask, int stride, int stride_p, int stride_m, int64_t n_reads,
                                    uint8_t *d_codes, cudaStream_t st);
+
+// pair.cu / rescue.cu: the paired stage with one insert-size model per chunk of the batch (qm_sample_set_chunks).  Models are
+// 4 qm_pestat each; d_model_of[p] is pair p's model (NULL: model 0 for every pair); d_pes NULL: h_pes is uploaded.
+extern "C" int qm_pestat_chunks(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const qm_reg *d_regs, const int32_t *d_n_regs,
+                                const int64_t *h_start, int n_chunks, const int32_t **d_model_of, const qm_pestat **d_pes, qm_pestat *h_pes,
+                                void *stream);
+extern "C" int qm_mate_rescue_models(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride,
+                                     const int32_t *d_lens, int64_t n_pairs, qm_reg *d_regs, int32_t *d_n_regs, const qm_pestat *h_pes,
+                                     int n_models, const qm_pestat *d_pes, const int32_t *d_model_of, int64_t *d_stats, void *stream);
+extern "C" int qm_pair_finish_models(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride,
+                                     const int32_t *d_lens, int64_t n_pairs, int64_t pair_id0, qm_reg *d_regs, int32_t *d_n_regs,
+                                     const qm_pestat *h_pes, int n_models, const qm_pestat *d_pes, const int32_t *d_model_of, qm_aln *d_alns,
+                                     void *stream);

@@ -133,7 +133,12 @@ __device__ SwOut sw_align2_warp(const qm_opt &o, const uint8_t *seq, int l_ms, c
     return r;
 }
 
-struct PesArg { qm_pestat p[4]; };
+// insert-size models, 4 per model; pair p searches with model model_of[p] (model 0 when model_of is NULL)
+struct PesArg {
+    const qm_pestat *pes;
+    const int32_t *model_of;
+    __device__ __forceinline__ const qm_pestat *of(int64_t pi) const { return pes + 4 * (model_of ? model_of[pi] : 0); }
+};
 
 // orientations (bit r) in which the anchor at arb needs no alignment: no usable model, or a region of the mate at a proper distance
 __device__ __forceinline__ int served_dirs(const IndexView &V, const qm_pestat *pes, int64_t arb, const qm_reg *ma, int n_ma)
@@ -193,6 +198,7 @@ rescue_scan_kernel(IndexView V, qm_opt o, PesArg P, int64_t n_pairs, int max_que
 {
     const int64_t pi = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (pi >= n_pairs) return;
+    const qm_pestat *pes = P.of(pi);
     int k = 0, base = 0;
     for (int pass = 0; pass < 2; ++pass) {              // count, then write
         int w = 0;
@@ -201,12 +207,12 @@ rescue_scan_kernel(IndexView V, qm_opt o, PesArg P, int64_t n_pairs, int max_que
             const int n = n_regs[2 * pi + i], n_ma = n_regs[2 * pi + !i], l_ms = lens[2 * pi + !i];
             for (int j = 0; j < n; ++j) {
                 if (a[j].score < a[0].score - o.pen_unpaired) continue;
-                const int skip = served_dirs(V, P.p, a[j].rb, ma, n_ma);
+                const int skip = served_dirs(V, pes, a[j].rb, ma, n_ma);
                 if (skip == 15) continue;
                 for (int r = 0; r < 4; ++r) {
                     int64_t rb, re;
                     bool is_rev;
-                    if ((skip >> r & 1) || !rescue_window(V, o, P.p, a[j].rb, a[j].rid, r, l_ms, max_query, rb, re, is_rev)) continue;
+                    if ((skip >> r & 1) || !rescue_window(V, o, pes, a[j].rb, a[j].rid, r, l_ms, max_query, rb, re, is_rev)) continue;
                     if (pass && base + w < cap_tasks) { ResTask t; t.pair = k ? (int)pi : -1; t.tr = ((i << 4 | j) << 2) | r; tasks[base + w] = t; }
                     ++w;
                 }
@@ -267,7 +273,7 @@ rescue_align_kernel(IndexView V, qm_opt o, PesArg P, const uint8_t *__restrict__
         const int l_ms = lens[2 * (int64_t)t.pair + !i];
         int64_t rb, re;
         bool is_rev;
-        rescue_window(V, o, P.p, a->rb, a->rid, r, l_ms, 32 * C, rb, re, is_rev);
+        rescue_window(V, o, P.of(t.pair), a->rb, a->rid, r, l_ms, 32 * C, rb, re, is_rev);
         const ResOut res = run_alignment<C>(V, o, codes + (2 * (int64_t)t.pair + !i) * stride, l_ms, rb, re, is_rev, s_win[wib], s_seq[wib], log);
         if (lane == 0) out[item] = res;
     }
@@ -296,6 +302,7 @@ rescue_apply_kernel(IndexView V, qm_opt o, PesArg P, const uint8_t *__restrict__
         if (item >= total) break;
         const int64_t pi = list[item];
         const int2 blk = blocks[item];
+        const qm_pestat *pes = P.of(pi);
         int next = 0;                                   // first result of the pair's block not yet passed
         // anchors: lane t holds anchor j = t & 15 of end t >> 4 as the lists were BEFORE any rescue
         int64_t my_rb = 0;
@@ -317,13 +324,13 @@ rescue_apply_kernel(IndexView V, qm_opt o, PesArg P, const uint8_t *__restrict__
             const int l_ms = lens[2 * pi + !i];
             // orientations already served by a region of the mate (lanes over the mate's regions)
             int skip = 0;
-            for (int r = 0; r < 4; ++r) if (P.p[r].failed) skip |= 1 << r;
+            for (int r = 0; r < 4; ++r) if (pes[r].failed) skip |= 1 << r;
             {
                 int mine = 0;
                 if (lane < n_ma) {
                     int64_t dist;
                     const int r = qm_infer_dir(l_pac, arb, ma[lane].rb, &dist);
-                    if (dist >= P.p[r].low && dist <= P.p[r].high) mine = 1 << r;
+                    if (dist >= pes[r].low && dist <= pes[r].high) mine = 1 << r;
                 }
 #pragma unroll
                 for (int d = 16; d; d >>= 1) mine |= __shfl_xor_sync(0xffffffffu, mine, d);
@@ -335,7 +342,7 @@ rescue_apply_kernel(IndexView V, qm_opt o, PesArg P, const uint8_t *__restrict__
                 if (skip >> r & 1) continue;
                 int64_t rb, re;
                 bool is_rev;
-                if (rescue_window(V, o, P.p, arb, arid, r, l_ms, 32 * C, rb, re, is_rev)) {
+                if (rescue_window(V, o, pes, arb, arid, r, l_ms, 32 * C, rb, re, is_rev)) {
                     const int want = (t << 2) | r;
                     while (next < blk.y && tasks[blk.x + next].tr < want) ++next;       // run up front, not needed after all
                     ResOut aln;
@@ -379,16 +386,20 @@ rescue_apply_kernel(IndexView V, qm_opt o, PesArg P, const uint8_t *__restrict__
 
 extern "C" {
 
-int qm_mate_rescue(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride, const int32_t *d_lens,
-                   int64_t n_pairs, qm_reg *d_regs, int32_t *d_n_regs, const qm_pestat pes[4], int64_t *d_stats, void *stream)
+// mate rescue with one insert-size model per chunk of the batch: h_pes[4 n_models] on the host, d_pes the same on the device
+// (NULL: uploaded here), d_model_of each pair's model (NULL: model 0)
+int qm_mate_rescue_models(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride, const int32_t *d_lens,
+                          int64_t n_pairs, qm_reg *d_regs, int32_t *d_n_regs, const qm_pestat *h_pes, int n_models, const qm_pestat *d_pes,
+                          const int32_t *d_model_of, int64_t *d_stats, void *stream)
 {
-    if (!ctx || !idx || !opt || !pes || n_pairs < 0 || (n_pairs > 0 && (!d_codes || !d_lens || !d_regs || !d_n_regs))) return QM_EINVAL;
+    const qm_pestat *pes = h_pes;
+    if (!ctx || !idx || !opt || !pes || n_models < 1 || n_pairs < 0 || (n_pairs > 0 && (!d_codes || !d_lens || !d_regs || !d_n_regs))) return QM_EINVAL;
     if (n_pairs == 0) return QM_OK;
     if (n_pairs > (1ll << 24)) return qm_fail(ctx, QM_ELIMIT, "qm_mate_rescue: more than 2^24 pairs in one call");
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
     bool any = false;
-    for (int d = 0; d < 4; ++d) any |= !pes[d].failed;
+    for (int d = 0; d < 4 * n_models; ++d) any |= !pes[d].failed;
     if (!any) return QM_OK;                       // no usable insert-size model: every orientation is skipped
     if (stride > kResMaxQuery) return qm_fail(ctx, QM_ELIMIT, "qm_mate_rescue: reads longer than %d bases", kResMaxQuery);
     const int blocks = ctx->sm_count * (stride <= 160 ? 4 : stride <= 256 ? 3 : 2);
@@ -402,8 +413,9 @@ int qm_mate_rescue(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
     const size_t o_task = (o_blk + (size_t)n_pairs * sizeof(int2) + 255) & ~(size_t)255;
     const size_t o_res = (o_task + cap_tasks * sizeof(ResTask) + 255) & ~(size_t)255;
     const size_t o_log = (o_res + cap_tasks * sizeof(ResOut) + 255) & ~(size_t)255;
+    const size_t o_pes = o_log + (size_t)blocks * kResWarps * kResLog * sizeof(uint32_t);
     void *p = nullptr;
-    const int rc = qm_scratch_reserve(ctx, 14, o_log + (size_t)blocks * kResWarps * kResLog * sizeof(uint32_t), &p);
+    const int rc = qm_scratch_reserve(ctx, 14, o_pes + (d_pes ? 0 : (size_t)n_models * 4 * sizeof(qm_pestat)), &p);
     if (rc) return rc;
     char *b = (char *)p;
     int *ctr = (int *)b;                              // [0] listed pairs, [1] tasks, [2] task cursor, [3] pair cursor
@@ -415,7 +427,12 @@ int qm_mate_rescue(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
     unsigned long long *stats = (unsigned long long *)d_stats;
     QM_CUDA(ctx, cudaMemsetAsync(b, 0, 256, st));
     PesArg P;
-    for (int d = 0; d < 4; ++d) P.p[d] = pes[d];
+    P.model_of = d_model_of;
+    P.pes = d_pes;
+    if (!d_pes) {
+        QM_CUDA(ctx, cudaMemcpyAsync(b + o_pes, h_pes, (size_t)n_models * 4 * sizeof(qm_pestat), cudaMemcpyHostToDevice, st));
+        P.pes = (const qm_pestat *)(b + o_pes);
+    }
     // reads are at most `stride` long: 5 / 8 / 16 query columns per lane
     const int C = stride <= 160 ? 5 : stride <= 256 ? 8 : 16;
     rescue_scan_kernel<<<(unsigned)((n_pairs + 127) / 128), 128, 0, st>>>(idx->v, *opt, P, n_pairs, 32 * C, d_regs, d_n_regs, d_lens, list, blk, tasks, (int)cap_tasks, ctr);
@@ -429,6 +446,12 @@ int qm_mate_rescue(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const ui
 #undef QM_RES_LAUNCH
     QM_CUDA(ctx, cudaGetLastError());
     return QM_OK;
+}
+
+int qm_mate_rescue(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride, const int32_t *d_lens,
+                   int64_t n_pairs, qm_reg *d_regs, int32_t *d_n_regs, const qm_pestat pes[4], int64_t *d_stats, void *stream)
+{
+    return qm_mate_rescue_models(ctx, idx, opt, d_codes, stride, d_lens, n_pairs, d_regs, d_n_regs, pes, 1, nullptr, nullptr, d_stats, stream);
 }
 
 }  // extern "C"

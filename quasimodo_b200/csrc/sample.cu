@@ -5,10 +5,12 @@
 // A qm_sample owns the int32 count tensor [QM_NCH][l_pac] of the sample and chunk-sized scratch (regions,
 // alignment records).  Pairs are processed in chunks of kChunkPairs: seeding/chaining -> extension rounds ->
 // pairing/CIGAR -> pileup, all on the caller's stream (device entry) or on the context's compute stream with
-// the next chunk's host->device copy running on the copy stream (host entry).  The insert-size model
-// (bwa's per-chunk mem_pestat) is fixed ONCE per sample from the first min(n, 2^18) pairs handed in -- or
+// the next chunk's host->device copy running on the copy stream (host entry).  By default the insert-size model
+// (bwa's per-chunk mem_pestat) is fixed ONCE per sample from the first min(n, QM_PESTAT_PAIRS) pairs handed in -- or
 // set by the caller (multi-GPU: rank 0's model is broadcast) -- so that results do not depend on how the
-// pair stream is split into batches or across GPUs (SURVEY.md 8e).
+// pair stream is split into batches or across GPUs (SURVEY.md 8e).  In per-chunk mode (qm_sample_set_chunks) the
+// caller names bwa's input chunks instead and every chunk is paired against its own model, as bwa mem does; the
+// internal chunks are then cut at those chunks' ends, so a model never depends on the batching either.
 #include <stdlib.h>
 #include <vector>
 #include <thread>
@@ -16,7 +18,7 @@
 #include "pipeline.cuh"
 
 namespace {
-constexpr int64_t kChunkPairs = 1 << 21;
+constexpr int64_t kChunkPairs = QM_CHUNK_MAX_PAIRS;
 constexpr int64_t kPestatPairs = QM_PESTAT_PAIRS;
 constexpr int kCopyParts = 8;
 }
@@ -54,6 +56,10 @@ struct qm_sample {
     int64_t keep_cap = 0, last_n = -1;
     struct Kept { uint8_t *codes, *quals; int32_t *lens; qm_aln *alns; int64_t n; int32_t stride; int64_t pair0; };   // pair0: id of the first pair
     std::vector<Kept> kept;
+    // per-chunk mode (qm_sample_set_chunks): the next add call's chunk sizes in pairs, and the models of the last call's chunks
+    bool chunked = false;
+    std::vector<int64_t> next_chunks;
+    std::vector<qm_pestat> chunk_pes;
 };
 
 namespace {
@@ -126,6 +132,36 @@ int filter_begin(qm_sample *s, int64_t n_pairs, cudaStream_t st)
     return QM_OK;
 }
 
+// The internal chunks of an add call of n_pairs pairs: [starts[k], starts[k] + sizes[k]), at most kChunkPairs each.  In per-chunk
+// mode they hold whole bwa chunks (bwa chunks bwa0[k] .. bwa0[k + 1] - 1 of s->next_chunks), which are taken over here.
+int plan_chunks(qm_sample *s, int64_t n_pairs, std::vector<int64_t> &starts, std::vector<int64_t> &sizes, std::vector<int64_t> &bwa,
+                std::vector<int> &bwa0)
+{
+    starts.clear(); sizes.clear(); bwa.clear(); bwa0.clear();
+    if (!s->chunked) {
+        for (int64_t p0 = 0; p0 < n_pairs; p0 += kChunkPairs) { starts.push_back(p0); sizes.push_back(std::min(kChunkPairs, n_pairs - p0)); }
+        return QM_OK;
+    }
+    bwa.swap(s->next_chunks);
+    s->next_chunks.clear();
+    s->chunk_pes.clear();
+    int64_t tot = 0;
+    for (int64_t c : bwa) tot += c;
+    if (tot != n_pairs)
+        return qm_fail(s->ctx, QM_EINVAL, "per-chunk mode: the chunk sizes given (qm_sample_set_chunks) add up to %lld pairs, the call has %lld",
+                       (long long)tot, (long long)n_pairs);
+    int64_t p0 = 0;
+    for (size_t c = 0; c < bwa.size();) {
+        bwa0.push_back((int)c);
+        int64_t n = 0;
+        while (c < bwa.size() && n + bwa[c] <= kChunkPairs) n += bwa[c++];
+        starts.push_back(p0); sizes.push_back(n);
+        p0 += n;
+    }
+    bwa0.push_back((int)bwa.size());
+    return QM_OK;
+}
+
 // the qualities the pileup sees: the reads' own, or (qm_sample_set_baq) capped by their base alignment quality
 int sample_pileup_quals(qm_sample *s, const qm_aln *alns, const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
                         int64_t n_reads, cudaStream_t st, const uint8_t **out)
@@ -144,8 +180,10 @@ int sample_pileup_quals(qm_sample *s, const qm_aln *alns, const uint8_t *d_codes
 // quals_ready (may be NULL): event after which d_quals is valid; only the pileup reads the qualities, so their copy
 // may still be in flight while the reads are being aligned
 // keep_off: the chunk's first pair within its batch (filter mode: where its keep bytes go)
+// bwa_sizes (per-chunk mode, NULL otherwise): the sizes of the n_bwa bwa chunks that make up these n pairs
 int sample_chunk(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_quals, int32_t stride, const int32_t *d_lens,
-                 int64_t n, int64_t pair_id0, int64_t keep_off, qm_aln *d_alns_out, cudaStream_t st, cudaEvent_t quals_ready = nullptr)
+                 int64_t n, int64_t pair_id0, int64_t keep_off, qm_aln *d_alns_out, cudaStream_t st, cudaEvent_t quals_ready = nullptr,
+                 const int64_t *bwa_sizes = nullptr, int n_bwa = 0)
 {
     qm_ctx *ctx = s->ctx;
     // the pileup stages a pair's reads in 512-byte rows and would leave longer reads out of the counts without a word
@@ -154,23 +192,38 @@ int sample_chunk(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_quals, i
         return qm_fail(ctx, QM_EINVAL, "pairs added after qm_sample_rmdup_finish: reset the sample first");
     int rc = qm_align_se(ctx, s->idx, &s->opt, d_codes, stride, d_lens, 2 * n, s->d_regs, s->d_n_regs, s->d_cells, st);
     if (rc) return rc;
-    if (!s->have_pes) {
-        // one model per sample.  With a communicator it is rank 0's (the rank that holds the sample's first pairs), broadcast:
-        // the other ranks have aligned their own first chunk meanwhile and only wait for 128 bytes.
-        const bool root = !s->comm || qm_comm_rank(s->comm) == 0;
-        if (root) {
-            rc = qm_pestat_sync(ctx, s->idx, &s->opt, s->d_regs, s->d_n_regs, n < kPestatPairs ? n : kPestatPairs, s->pes, st);
-            if (rc) return rc;
-        }
-        if (s->comm && qm_comm_size(s->comm) > 1) {
-            rc = qm_pestat_bcast(ctx, s->comm, s->pes, 0, st);
-            if (rc) return rc;
-        }
-        s->have_pes = true;
-    }
     qm_aln *alns = d_alns_out ? d_alns_out : s->d_alns;
-    rc = qm_pair_finish(ctx, s->idx, &s->opt, d_codes, stride, d_lens, n, pair_id0, s->d_regs, s->d_n_regs, s->pes, alns, st);
-    if (rc) return rc;
+    if (bwa_sizes && !s->have_pes) {
+        // per-chunk mode without a given model (-I): mem_pestat over every pair of each chunk, each pair against its chunk's model
+        std::vector<int64_t> start((size_t)n_bwa + 1, 0);
+        for (int c = 0; c < n_bwa; ++c) start[(size_t)c + 1] = start[(size_t)c] + bwa_sizes[c];
+        std::vector<qm_pestat> pes((size_t)n_bwa * 4);
+        const int32_t *d_model_of = nullptr;
+        const qm_pestat *d_pes = nullptr;
+        rc = qm_pestat_chunks(ctx, s->idx, &s->opt, s->d_regs, s->d_n_regs, start.data(), n_bwa, &d_model_of, &d_pes, pes.data(), st);
+        if (rc) return rc;
+        s->chunk_pes.insert(s->chunk_pes.end(), pes.begin(), pes.end());
+        rc = qm_pair_finish_models(ctx, s->idx, &s->opt, d_codes, stride, d_lens, n, pair_id0, s->d_regs, s->d_n_regs, pes.data(), n_bwa, d_pes,
+                                   d_model_of, alns, st);
+        if (rc) return rc;
+    } else {
+        if (!s->have_pes) {
+            // one model per sample.  With a communicator it is rank 0's (the rank that holds the sample's first pairs), broadcast:
+            // the other ranks have aligned their own first chunk meanwhile and only wait for 128 bytes.
+            const bool root = !s->comm || qm_comm_rank(s->comm) == 0;
+            if (root) {
+                rc = qm_pestat_sync(ctx, s->idx, &s->opt, s->d_regs, s->d_n_regs, n < kPestatPairs ? n : kPestatPairs, s->pes, st);
+                if (rc) return rc;
+            }
+            if (s->comm && qm_comm_size(s->comm) > 1) {
+                rc = qm_pestat_bcast(ctx, s->comm, s->pes, 0, st);
+                if (rc) return rc;
+            }
+            s->have_pes = true;
+        }
+        rc = qm_pair_finish(ctx, s->idx, &s->opt, d_codes, stride, d_lens, n, pair_id0, s->d_regs, s->d_n_regs, s->pes, alns, st);
+        if (rc) return rc;
+    }
     if (s->filter) {
         keep_pairs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(alns, n, s->d_keep + keep_off, s->d_n_kept);
         QM_CUDA(ctx, cudaGetLastError());
@@ -276,6 +329,7 @@ int qm_sample_reset(qm_sample *s, void *stream)
     QM_CUDA(ctx, cudaMemsetAsync(s->d_cells, 0, 8, (cudaStream_t)stream));
     { const int rc = qm_indel_table_reset(s->indels, stream); if (rc) return rc; }
     s->have_pes = false; s->n_pairs = 0; s->rmdup_finished = false; s->last_n = -1;
+    s->next_chunks.clear(); s->chunk_pes.clear();
     if (!s->kept.empty()) { QM_CUDA(ctx, cudaStreamSynchronize((cudaStream_t)stream)); free_kept(s); }
     return QM_OK;
 }
@@ -581,6 +635,39 @@ int qm_sample_get_pestat(const qm_sample *s, qm_pestat pes[4])
     return QM_OK;
 }
 
+// Per-chunk mode: bwa mem's insert-size model per input chunk (bwamem.c mem_process_seqs runs mem_pestat over all pairs of
+// each chunk).  h_chunk_pairs[0 .. n_chunks) are the sizes in pairs of the chunks of the NEXT add call, in order; they must add up
+// to its n_pairs (QM_EINVAL there otherwise), so a chunk never straddles two calls.  Where the chunks end is the caller's rule (bwa:
+// bseq_read's running base count); a chunk holds at most QM_CHUNK_MAX_PAIRS pairs.  The prefix model and qm_pestat_bcast are not
+// used in this mode; a model given with qm_sample_set_pestat (bwa mem -I) still replaces every chunk's.
+int qm_sample_set_chunks(qm_sample *s, const int64_t *h_chunk_pairs, int64_t n_chunks)
+{
+    if (!s || n_chunks < 0 || (n_chunks > 0 && !h_chunk_pairs)) return QM_EINVAL;
+    if (!s->chunked && s->n_pairs != 0) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_chunks: pairs were already added; reset the sample first");
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        if (h_chunk_pairs[c] <= 0) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_set_chunks: chunk %lld has %lld pairs", (long long)c, (long long)h_chunk_pairs[c]);
+        if (h_chunk_pairs[c] > kChunkPairs)
+            return qm_fail(s->ctx, QM_ELIMIT, "qm_sample_set_chunks: chunk %lld has %lld pairs, at most %lld (QM_CHUNK_MAX_PAIRS) are supported",
+                           (long long)c, (long long)h_chunk_pairs[c], (long long)kChunkPairs);
+    }
+    s->chunked = true;
+    s->next_chunks.assign(h_chunk_pairs, h_chunk_pairs + n_chunks);
+    return QM_OK;
+}
+
+// per-chunk mode: the models of the chunks of the last add call, 4 per chunk (none when a model was given); h_pes NULL with
+// max_chunks 0: only their number
+int qm_sample_chunk_pestat(const qm_sample *s, qm_pestat *h_pes, int64_t max_chunks, int64_t *n_chunks)
+{
+    if (!s || !n_chunks || max_chunks < 0 || (max_chunks > 0 && !h_pes)) return QM_EINVAL;
+    const int64_t n = (int64_t)s->chunk_pes.size() / 4;
+    *n_chunks = n;
+    if (!h_pes) return QM_OK;
+    if (n > max_chunks) return qm_fail(s->ctx, QM_EINVAL, "qm_sample_chunk_pestat: %lld chunks, room for %lld", (long long)n, (long long)max_chunks);
+    std::copy(s->chunk_pes.begin(), s->chunk_pes.end(), h_pes);
+    return QM_OK;
+}
+
 // insert-size model from a designated prefix of the sample (the first min(n, QM_PESTAT_PAIRS) pairs given):
 // single-end alignment of the prefix + mem_pestat, nothing is counted.  A shard that does not start at pair 0
 // calls this with the sample's first pairs before adding its own (every rank gets the same model, no collective).
@@ -604,11 +691,15 @@ int qm_sample_add_pairs(qm_sample *s, const uint8_t *d_codes, const uint8_t *d_q
 {
     if (!s || n_pairs < 0 || (n_pairs > 0 && (!d_codes || !d_quals || !d_lens)) || stride <= 0) return QM_EINVAL;
     QM_CUDA(s->ctx, cudaSetDevice(s->ctx->device));
+    std::vector<int64_t> starts, sizes, bwa;
+    std::vector<int> bwa0;
+    { const int rc = plan_chunks(s, n_pairs, starts, sizes, bwa, bwa0); if (rc) return rc; }
     { const int rc = filter_begin(s, n_pairs, (cudaStream_t)stream); if (rc) return rc; }
-    for (int64_t p0 = 0; p0 < n_pairs; p0 += kChunkPairs) {
-        const int64_t n = n_pairs - p0 < kChunkPairs ? n_pairs - p0 : kChunkPairs;
+    for (size_t k = 0; k < starts.size(); ++k) {
+        const int64_t p0 = starts[k], n = sizes[k];
         int rc = sample_chunk(s, d_codes + 2 * p0 * stride, d_quals + 2 * p0 * stride, stride, d_lens + 2 * p0, n, pair_id0 + p0, p0,
-                              d_alns ? d_alns + 2 * p0 : nullptr, (cudaStream_t)stream);
+                              d_alns ? d_alns + 2 * p0 : nullptr, (cudaStream_t)stream, nullptr,
+                              s->chunked ? bwa.data() + bwa0[k] : nullptr, s->chunked ? bwa0[k + 1] - bwa0[k] : 0);
         if (rc) return rc;
     }
     return QM_OK;
@@ -624,6 +715,9 @@ static int add_pairs_host_impl(qm_sample *s, const uint8_t *h_codes, const uint8
     if (!s || n_pairs < 0 || (n_pairs > 0 && ((packed ? (!h_bases2 || !h_nmask) : false) || !h_quals || !h_lens)) || stride <= 0) return QM_EINVAL;
     qm_ctx *ctx = s->ctx;
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
+    std::vector<int64_t> starts, sizes, bwa;
+    std::vector<int> bwa0;
+    { const int rc = plan_chunks(s, n_pairs, starts, sizes, bwa, bwa0); if (rc) return rc; }
     { const int rc = filter_begin(s, n_pairs, ctx->own_stream); if (rc) return rc; }
     if (n_pairs == 0) return QM_OK;
     const int stride_p = (stride + 3) >> 2, stride_m = (stride + 7) >> 3;
@@ -646,8 +740,9 @@ static int add_pairs_host_impl(qm_sample *s, const uint8_t *h_codes, const uint8
     // Full-size chunks (large batches: fewer extension rounds, shorter tails).  A chunk's bases are copied in kCopyParts
     // pieces and seeded piece by piece, so only the first piece's copy is exposed; qualities travel behind the bases
     // (only the pileup at the end of a chunk reads them); the next chunk's copies run under this chunk's kernels.
-    std::vector<int64_t> starts, sizes;
-    {
+    // (Per-chunk mode: the chunks plan_chunks cut at bwa chunk ends.)
+    if (!s->chunked) {
+        starts.clear(); sizes.clear();
         int64_t ramp[8] = { kChunkPairs };
         int n_ramp = 1;
         if (const char *e = getenv("QM_HOST_CHUNKS")) {             // measurement knob: comma-separated chunk sizes
@@ -720,7 +815,8 @@ static int add_pairs_host_impl(qm_sample *s, const uint8_t *h_codes, const uint8
         if (packed) { ctx->se_pk = s->d_stage[b] + o_pk; ctx->se_mk = s->d_stage[b] + o_mk; ctx->se_sp = stride_p; ctx->se_sm = stride_m; }
         for (int pt = 0; pt < n_parts; ++pt) { ctx->se_part_end[pt] = 2 * n * (pt + 1) / n_parts; ctx->se_part_ev[pt] = s->ev_part[b][pt]; }
         int rc = sample_chunk(s, s->d_stage[b], s->d_stage[b] + seq_al, stride, (const int32_t *)(s->d_stage[b] + 2 * seq_al), n,
-                              pair_id0 + p0, p0, nullptr, ks, s->ev_quals[b]);
+                              pair_id0 + p0, p0, nullptr, ks, s->ev_quals[b],
+                              s->chunked ? bwa.data() + bwa0[c] : nullptr, s->chunked ? bwa0[c + 1] - bwa0[c] : 0);
         ctx->se_n_parts = 0; ctx->se_pk = ctx->se_mk = nullptr;
         if (rc) return rc;
         if (h_alns) QM_CUDA(ctx, cudaMemcpyAsync(h_alns + 2 * p0, s->d_alns, (size_t)2 * n * sizeof(qm_aln), cudaMemcpyDeviceToHost, ks));

@@ -46,11 +46,14 @@ def benchmark_path(dirs, rule, sample, ref_name):
     return dirs[var] + pat.format(sample=sample, ref_name=ref_name)
 
 
-def sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads=4, extra=(), benchmark=False):
+def sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads=4, extra=(), benchmark=False, chunk_bases=None):
     """-> (argv, [every path the four reference rules declare or leave behind]) for one {sample}.{ref_name};
     benchmark=True adds `--benchmark` at rule bcftools' benchmark path (not part of the returned list: Snakemake does not
-    fail a job over it)"""
+    fail a job over it); chunk_bases=K adds bwa mem's `-K K` (one insert-size model per input chunk of K bases, as bwa pairs;
+    `bwa mem -t T` itself is `-K 10000000*T`)"""
     argv = [driver, "sample", "--ref", ref_fa, "--r1", r1, "--r2", r2, "--sample", sample, "-t", str(threads), "--rmdup", "1"]
+    if chunk_bases is not None:
+        argv += ["-K", str(int(chunk_bases))]
     paths = []
     for key, opt in DRIVER_OPTION.items():
         p = expand(dirs, key[0], key[1], sample, ref_name)
@@ -115,12 +118,13 @@ def pileup_commands(driver, dirs, sample, ref_name, ref_fa, threads=4, extra=(),
 CLEAN_FASTQ = {"rm_phix": ("seq_dir", "/cl_fq/{sample}.qc.nophix.r{mate}.fq"), "rm_human_ecoli": ("seq_dir", "/cl_fq/{sample}.qc.cl.r{mate}.fq")}
 
 
-def decontam_sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, phix_fa, human_ecoli_fa=(), threads=4, extra=(), benchmark=False):
+def decontam_sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, phix_fa, human_ecoli_fa=(), threads=4, extra=(), benchmark=False,
+                            chunk_bases=None):
     """-> (argv, [every path the job writes]) of rules rm_phix [+ rm_human_ecoli] + bwa + rmdup + mpileup + bcftools as ONE
     `qm_driver sample --decontam` job on the raw reads r1 / r2: sample_command's outputs plus the last pass's cleaned FASTQ (rule
     rm_human_ecoli's when human_ecoli_fa names its genomes, else rule rm_phix's), the FASTQ the assemblers read.  With both passes
     rule rm_phix's intermediate FASTQ is not written."""
-    argv, paths = sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads, benchmark=benchmark)
+    argv, paths = sample_command(driver, dirs, sample, ref_name, ref_fa, r1, r2, threads, benchmark=benchmark, chunk_bases=chunk_bases)
     argv += ["--decontam", phix_fa]
     last = "rm_phix"
     if human_ecoli_fa:
