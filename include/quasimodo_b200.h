@@ -152,6 +152,8 @@ typedef struct {
 } qm_aln;                                                                     /* 128 B */
 typedef struct { int32_t low, high, failed, pad; double avg, std; } qm_pestat;  /* x4: FF FR RF RR */
 
+/* Read arrays of the two entries below: read r occupies row r of `stride` bytes, lens[r] in [0, stride], stride <= 512
+ * (QM_ELIMIT otherwise).  qm_align_se fails with QM_ECUDA should reads be left unfinished after its last round. */
 /* diagnostic / parity entry: seeds of every read, sorted by (qbeg, rbeg) (SURVEY.md 8a2) */
 int qm_collect_seeds(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8_t *d_codes, int32_t stride,
                      const int32_t *d_lens, int64_t n_reads, qm_seed *d_seeds /* [n][QM_MAX_SEEDS] */,

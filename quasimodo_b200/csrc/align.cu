@@ -1339,6 +1339,7 @@ spec_finish_kernel(IndexView V, qm_opt o, const uint8_t *__restrict__ codes, int
     }
 }
 
+constexpr int kMaxStride = 512;               // longest row the read-level entries take (the extension's queries stop at QM_EXT_MAX_QLEN)
 constexpr int64_t kSeBatch = 1 << 22;         // a round with fewer tasks hands the still-active reads to tail_kernel       // reads per internal round-trip (bounds scratch memory)
 
 struct SeScratch {
@@ -1479,6 +1480,7 @@ int qm_collect_seeds(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const 
     if (!ctx || !idx || !opt || n_reads < 0 || (n_reads > 0 && (!d_codes || !d_lens || !d_seeds || !d_n_seeds)))
         return QM_EINVAL;
     if (opt->min_seed_len != idx->v.k) return qm_fail(ctx, QM_EINVAL, "index built with k=%d but min_seed_len=%d", idx->v.k, opt->min_seed_len);
+    if (stride > kMaxStride) return qm_fail(ctx, QM_ELIMIT, "qm_collect_seeds: rows of %d bases: reads longer than %d bases are not supported", stride, kMaxStride);
     if (n_reads == 0) return QM_OK;
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
     if (opt->flags & QM_F_FM_SEEDS) {
@@ -1503,6 +1505,7 @@ int qm_align_se(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8
         return QM_EINVAL;
     if (opt->min_seed_len != idx->v.k) return qm_fail(ctx, QM_EINVAL, "index built with k=%d but min_seed_len=%d", idx->v.k, opt->min_seed_len);
     if (opt->e_ins <= 0 || opt->e_del <= 0) return qm_fail(ctx, QM_EINVAL, "gap extension penalties must be > 0");
+    if (stride > kMaxStride) return qm_fail(ctx, QM_ELIMIT, "qm_align_se: rows of %d bases: reads longer than %d bases are not supported", stride, kMaxStride);
     if (n_reads == 0) return QM_OK;
     QM_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -1563,6 +1566,9 @@ int qm_align_se(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8
         }
         ctx->se_n_parts = 0; ctx->se_pk = ctx->se_mk = nullptr;
         qm_prof_end(ctx, QM_ST_SEED, sp, st, n_seed_launches);
+        // each read has at most 2 x QM_MAX_REGS dependent tasks, so the loop always ends on one of its breaks; if it did not, reads
+        // would be left unfinished, and that is an error as it is in spec_finish_batch
+        bool finished = false;
         for (int round = 0; round < 4 * QM_MAX_REGS + 8; ++round) {
             sp = qm_prof_begin(ctx, QM_ST_ADVANCE, st);
             cudaMemsetAsync(sc.ctr, 0, sizeof(RoundCounters), st);
@@ -1573,7 +1579,7 @@ int qm_align_se(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8
             cudaMemcpyAsync(h_ctr, sc.ctr, kRoundHeader, cudaMemcpyDeviceToHost, st);
             cudaError_t e = cudaStreamSynchronize(st);
             if (e != cudaSuccess) { return qm_fail(ctx, QM_ECUDA, "qm_align_se round %d: %s", round, cudaGetErrorString(e)); }
-            if (h_ctr->n_tasks == 0) break;
+            if (h_ctr->n_tasks == 0) { finished = true; break; }
             static const bool round_log = getenv("QM_ROUND_LOG") != nullptr;       // diagnostics: the round's task counts per class
             if (round_log) {
                 fprintf(stderr, "[qm round %d] tasks %d max_score %d classes", round, h_ctr->n_tasks, h_ctr->max_score);
@@ -1599,6 +1605,7 @@ int qm_align_se(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8
                                                                                sc.st, d_regs + b0 * QM_MAX_REGS, d_n_regs + b0, over, 0, n_over,
                                                                                cursor2, (unsigned long long *)d_cells, nullptr, nullptr);
                 qm_prof_end(ctx, QM_ST_EXTEND, sp, st, 2);
+                finished = true;
                 break;
             }
             // between the two thresholds: every remaining seed ahead of the state machine (spec_finish_batch).  Below tail_min the
@@ -1610,6 +1617,7 @@ int qm_align_se(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8
                 rc = spec_finish_batch(ctx, idx, opt, P, codes, stride, lens, sc, d_regs + b0 * QM_MAX_REGS, d_n_regs + b0, d_cells, h_ctr,
                                        h_ctr->n_tasks, st);
                 if (rc) return rc;
+                finished = true;
                 break;
             }
             // The round's tasks sorted by (query length, rows, seed score): the classes become contiguous runs of one list, the
@@ -1630,6 +1638,7 @@ int qm_align_se(qm_ctx *ctx, const qm_index *idx, const qm_opt *opt, const uint8
             qm_prof_end(ctx, QM_ST_EXTEND, sp, st, n_launch);
             if (rc) return rc;
         }
+        if (!finished) return qm_fail(ctx, QM_ECUDA, "qm_align_se: reads still active after %d rounds", 4 * QM_MAX_REGS + 8);
     }
     QM_CUDA(ctx, cudaGetLastError());
     return QM_OK;
