@@ -590,6 +590,58 @@ int  qm_sample_allreduce_counts(qm_sample *s, void *stream);
  * collectives; errors of the decision (a repeated id) are reached by every rank alike.  Synchronous. */
 int  qm_sample_finish_comm(qm_sample *s, qm_comm *comm, int64_t *n_dup_pairs, int64_t *n_capped_reads, void *stream);
 
+/* ---- SNP truth set of a strain pair (replaces rule `nucmer`, rules/genome_diff.smk: `nucmer ref qry; show-snps -CTHlr
+ * <(delta-filter -r -q delta)`; SURVEY.md 8a row a13; contract DESIGN.md 5c) ----
+ * ref_idx: qm_index_build of the reference with k = opt->min_match (QM_EINVAL otherwise).  The query is h_qry_codes (0..3, contigs
+ * concatenated, at most QM_MAX_CONTIGS, fewer than 2^30 bases).
+ * Anchors are the maximal exact matches of at least min_match bases between either query strand and the reference that contain a
+ * k-mer unique in the reference (it occurs once and its reverse complement never): nucmer's default --mumreference, in the form the
+ * index answers.  They are chained into collinear clusters per (query contig, strand, reference contig) (max_gap, max_diag,
+ * diag_factor), clusters of fewer than min_cluster anchored bases are dropped, clusters within break_len on both sequences are
+ * merged, and every gap between consecutive anchors gets a global affine-gap alignment on the device; a gap whose score along its
+ * columns falls more than break_len below its best ends the alignment there.  Each alignment is extended past its outermost
+ * anchors with ksw_extend2 (qm_extend_batch; zdrop and band = break_len, windows of at most QM_EXT_MAX_QLEN query bases, again
+ * while an extension reaches the end of its window), and the extended stretches are aligned globally.  delta-filter -r -q becomes
+ * two heaviest chains (weight: matching columns = aligned length x identity), on reference then on query coordinates.
+ * Rows (show-snps -CTHlr): one per substitution and per indel base, indels left-aligned, P1 kept on the reference base in front
+ * of an insertion; rows at a position covered by more than one kept alignment are dropped (-C) unless QM_GDIFF_KEEP_AMBIGUOUS;
+ * QM_GDIFF_NO_INDELS leaves the indel rows out (-I).  Rows come sorted by (reference contig, P1) (-r), alignments by reference
+ * start.  QM_ELIMIT when max_rows / max_alns are too small; *n_rows / *n_alns then hold what is needed.  h_phase_ms (may be
+ * NULL, else 5 doubles): milliseconds of anchors, clustering, gap alignment, end extension and rows.  Synchronous. */
+typedef struct {
+    int32_t min_match;            /* nucmer -l (20)                                                        */
+    int32_t min_cluster;          /* -c (65): anchored bases a cluster needs                               */
+    int32_t max_gap;              /* -g (90): longest gap between neighbouring anchors of a cluster        */
+    int32_t break_len;            /* -b (200): longest gap bridged between clusters                        */
+    float   diag_factor;          /* -d (0.12): diagonal difference / gap, above max_diag                  */
+    int32_t max_diag;             /* -D (5): diagonal difference always allowed                            */
+    int32_t match, mismatch;      /* gap DP and end extension: + match (>= 1), - mismatch (1, 4)            */
+    int32_t gap_open, gap_extend; /* a gap of l bases costs gap_open + l * gap_extend (6, 1)               */
+    int32_t flags;                /* QM_GDIFF_*                                                            */
+    int32_t reserved[5];
+} qm_gdiff_opt;
+#define QM_GDIFF_NO_INDELS      1 /* show-snps -I */
+#define QM_GDIFF_KEEP_AMBIGUOUS 2 /* show-snps without -C */
+typedef struct {
+    int32_t p1, p2;               /* 1-based reference / query position (query forward strand)              */
+    int32_t buff, dist;           /* distance to the nearest other difference or alignment end; to the nearest sequence end */
+    char    sub_r, sub_q;         /* A C G T, '.' on the gap side; sub_q on the aligned query strand        */
+    int8_t  frm_r, frm_q;         /* 1; -1 for a query on the reverse strand                                */
+    int32_t rid, qid;             /* reference / query contig                                              */
+} qm_gdiff_row;                   /* 28 B */
+typedef struct {
+    int32_t rid, qid;
+    int32_t rs, re;               /* 1-based first / last reference base                                   */
+    int32_t qs, qe;               /* 1-based query positions aligned to rs / re (qs > qe on the reverse strand, as in a delta file) */
+    int32_t strand;               /* 1 / -1 */
+    int32_t edits, matches;       /* mismatching columns + indel bases; matching columns                   */
+    int32_t pad;
+} qm_gdiff_aln;                   /* 40 B */
+void qm_gdiff_opt_default(qm_gdiff_opt *opt);
+int  qm_genome_diff_host(qm_ctx *ctx, const qm_index *ref_idx, const uint8_t *h_qry_codes, int n_qry_contigs, const int64_t *h_qry_lens,
+                         const qm_gdiff_opt *opt, qm_gdiff_row *h_rows, int64_t max_rows, int64_t *n_rows, qm_gdiff_aln *h_alns,
+                         int64_t max_alns, int64_t *n_alns, double *h_phase_ms);
+
 /* ---- stage timers: CUDA events recorded on the launching stream around every kernel group ----
  * stages: 0 seed+chain, 1 advance (extension state machine), 2 extend (ksw_extend2 kernels), 3 pair+CIGAR,
  * 4 pileup, 5 h2d, 6 d2h, 7 other, 8 mate rescue.  qm_profile_collect synchronises the device and returns + clears the totals;

@@ -43,6 +43,13 @@ class BamPairs(C.Structure):
                 ("n_capped", C.c_int64)]
 
 
+class GdiffOpt(C.Structure):
+    """qm_gdiff_opt: nucmer's -l -c -g -b -d -D, the gap DP's scores, QM_GDIFF_* flags"""
+    _fields_ = [("min_match", C.c_int32), ("min_cluster", C.c_int32), ("max_gap", C.c_int32), ("break_len", C.c_int32),
+                ("diag_factor", C.c_float), ("max_diag", C.c_int32), ("match", C.c_int32), ("mismatch", C.c_int32),
+                ("gap_open", C.c_int32), ("gap_extend", C.c_int32), ("flags", C.c_int32), ("reserved", C.c_int32 * 5)]
+
+
 class CallOpt(C.Structure):
     _fields_ = [("min_dp", C.c_int32), ("min_alt", C.c_int32), ("min_af", C.c_float), ("reserved", C.c_int32)]
 
@@ -74,6 +81,13 @@ CAP_KEY_DTYPE = np.dtype([("key", "<u8"), ("read_id", "<i4"), ("end", "<i4")])
 assert DUP_KEY_DTYPE.itemsize == 32 and CAP_KEY_DTYPE.itemsize == 16
 PESTAT_DTYPE = np.dtype([("low", "<i4"), ("high", "<i4"), ("failed", "<i4"), ("pad", "<i4"), ("avg", "<f8"), ("std", "<f8")])
 assert REG_DTYPE.itemsize == 64 and ALN_DTYPE.itemsize == 128 and SEED_DTYPE.itemsize == 16 and PESTAT_DTYPE.itemsize == 32
+GDIFF_ROW_DTYPE = np.dtype([("p1", "<i4"), ("p2", "<i4"), ("buff", "<i4"), ("dist", "<i4"), ("sub_r", "S1"), ("sub_q", "S1"),
+                            ("frm_r", "i1"), ("frm_q", "i1"), ("rid", "<i4"), ("qid", "<i4")])
+GDIFF_ALN_DTYPE = np.dtype([("rid", "<i4"), ("qid", "<i4"), ("rs", "<i4"), ("re", "<i4"), ("qs", "<i4"), ("qe", "<i4"),
+                            ("strand", "<i4"), ("edits", "<i4"), ("matches", "<i4"), ("pad", "<i4")])
+assert GDIFF_ROW_DTYPE.itemsize == 28 and GDIFF_ALN_DTYPE.itemsize == 40
+GDIFF_NO_INDELS, GDIFF_KEEP_AMBIGUOUS = 1, 2
+GDIFF_PHASES = ("anchors", "clusters", "gaps", "ends", "rows")
 QM_EXT_BAND_RETRY = 1
 QM_EXT_PREV_H0 = 2
 
@@ -179,6 +193,8 @@ SIGNATURES = {
     "qm_sample_indel_table": (_P, [_P]),
     "qm_sample_set_comm": (C.c_int, [_P, _P]),
     "qm_sample_allreduce_counts": (C.c_int, [_P, _P]),
+    "qm_gdiff_opt_default": (None, [_P]),
+    "qm_genome_diff_host": (C.c_int, [_P, _P, _P, C.c_int, _P, _P, _P, _L, C.POINTER(C.c_int64), _P, _L, C.POINTER(C.c_int64), _P]),
     "qm_dpx_peak_sync": (C.c_int, [_P, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }
 EXPORTS = sorted(SIGNATURES)
@@ -202,6 +218,12 @@ def lib():
 def default_opt():
     o = Opt()
     lib().qm_opt_default(C.byref(o))
+    return o
+
+
+def default_gdiff_opt():
+    o = GdiffOpt()
+    lib().qm_gdiff_opt_default(C.byref(o))
     return o
 
 

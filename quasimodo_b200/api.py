@@ -369,6 +369,32 @@ class Context:
     def sample(self, idx, opt=None, popt=None):
         return Sample(self, idx, opt, popt)
 
+    # ---- genome diff (rule `nucmer`: nucmer; delta-filter -r -q; show-snps -CTHlr) ----
+    def genome_diff(self, ref_idx, qry_genome, opt=None, phases=None):
+        """rows (GDIFF_ROW_DTYPE, show-snps -CTHlr) and kept alignments (GDIFF_ALN_DTYPE) of qry_genome against the reference of
+        ref_idx, whose k must be opt.min_match (default opt: nucmer's, min_match 20).  phases: a dict that receives the
+        milliseconds of each phase (_lib.GDIFF_PHASES)."""
+        opt = opt or _lib.default_gdiff_opt()
+        codes = np.ascontiguousarray(qry_genome.codes, dtype=np.uint8)
+        lens = np.ascontiguousarray(qry_genome.lens, dtype=np.int64)
+        n_rows, n_alns = C.c_int64(), C.c_int64()
+        ms = (C.c_double * len(_lib.GDIFF_PHASES))()
+        max_rows, max_alns = 1 << 16, 1 << 10
+        L = _lib.lib()
+        while True:
+            rows = np.zeros(max_rows, _lib.GDIFF_ROW_DTYPE)
+            alns = np.zeros(max_alns, _lib.GDIFF_ALN_DTYPE)
+            rc = L.qm_genome_diff_host(self._h, ref_idx._h, codes.ctypes.data, len(lens), lens.ctypes.data, C.byref(opt),
+                                       rows.ctypes.data, max_rows, C.byref(n_rows), alns.ctypes.data, max_alns, C.byref(n_alns), ms)
+            if rc == -5 and (n_rows.value > max_rows or n_alns.value > max_alns):      # QM_ELIMIT: room for what it reported
+                max_rows, max_alns = max(max_rows, n_rows.value), max(max_alns, n_alns.value)
+                continue
+            _check(self._h, rc, "qm_genome_diff_host")
+            break
+        if phases is not None:
+            phases.update(zip(_lib.GDIFF_PHASES, list(ms)))
+        return rows[:n_rows.value].copy(), alns[:n_alns.value].copy()
+
     def profile_enable(self, on=True):
         _check(self._h, _lib.lib().qm_profile_enable(self._h, 1 if on else 0), "qm_profile_enable")
 

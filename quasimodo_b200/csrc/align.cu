@@ -82,20 +82,9 @@ struct PackedRead {                 // per-thread view of the block's shared arr
     }
 };
 
-// reverse the order of the 32 two-bit groups of x
-__device__ __forceinline__ uint64_t grouprev(uint64_t x)
-{
-    const uint64_t y = __brevll(x);
-    return ((y >> 1) & 0x5555555555555555ull) | ((y & 0x5555555555555555ull) << 1);
-}
-
 __device__ __forceinline__ uint64_t ref_get2(const IndexView &V, int64_t b)
 {   // 32 reference bases starting at forward position b >= -32
-    const int64_t x = b + 32;
-    const uint64_t *w = V.ref2p + (x >> 5);
-    const int sh = 2 * (int)(x & 31);
-    const uint64_t lo = __ldg(w);
-    return sh ? (lo >> sh) | (__ldg(w + 1) << (64 - sh)) : lo;
+    return qm_get2_padded(V.ref2p, b);
 }
 __device__ __forceinline__ uint32_t uniq_get(const uint32_t *__restrict__ map, int64_t b)
 {   // flags of the 32 k-mers starting at forward positions b .. b+31, b >= -32 (map = V.uniqp or V.uniq2p)
@@ -270,7 +259,7 @@ __device__ __forceinline__ void seed_walk_step(const IndexView &V, const qm_opt 
         for (int t = 0; t < 4; ++t) {
             if (t >= nt) break;
             const bool r = (tpass >> t) & 1u;
-            const uint64_t x = rbits ^ (r ? ~grouprev(ref_get2(V, tp[t] - 32)) : ref_get2(V, tp[t] + k));
+            const uint64_t x = rbits ^ (r ? ~qm_grouprev(ref_get2(V, tp[t] - 32)) : ref_get2(V, tp[t] + k));
             const uint64_t mm = (x | (x >> 1)) & 0x5555555555555555ull;
             const int m_b = mm ? (__ffsll((long long)mm) - 1) >> 1 : 32;
             const int64_t lim = r ? tp[t] : V.l_pac - k - tp[t];
@@ -319,7 +308,7 @@ __device__ __forceinline__ void seed_walk_step(const IndexView &V, const qm_opt 
         }
         if (two || trk_pass) {                      // a reverse-complement hit at pr: positions pr-1 .. 0
             const int64_t pr = two ? trk_p2 : trk_p;
-            const uint64_t x = rbits ^ ~grouprev(ref_get2(V, pr - 32));
+            const uint64_t x = rbits ^ ~qm_grouprev(ref_get2(V, pr - 32));
             const uint64_t mm = (x | (x >> 1)) & 0x5555555555555555ull;
             const int m_b = mm ? (__ffsll((long long)mm) - 1) >> 1 : 32;
             m = m < m_b ? m : m_b; m = (int64_t)m > pr ? (int)pr : m;
@@ -369,7 +358,7 @@ __device__ __forceinline__ void seed_walk_step(const IndexView &V, const qm_opt 
         for (int g = 0; g < kBloomBatch; ++g) {
             if (g < gmax) {
                 const uint64_t vg = R.get2(q + g) & mask;
-                const uint64_t fg = grouprev(vg) >> (64 - 2 * k), rg = ~vg & mask;
+                const uint64_t fg = qm_grouprev(vg) >> (64 - 2 * k), rg = ~vg & mask;
                 uint32_t bp[3];
                 qm_bloom_pos(fg < rg ? fg : rg, V.bloom_bits, bp);
 #pragma unroll
@@ -390,7 +379,7 @@ __device__ __forceinline__ void seed_walk_step(const IndexView &V, const qm_opt 
         // position q passed the filter (and its k-mer holds no N)
     }
     const uint64_t v = R.get2(q) & mask;            // first base in the lowest bits
-    const uint64_t fw = grouprev(v) >> (64 - 2 * k);  // first base in the highest bits: the table's key order
+    const uint64_t fw = qm_grouprev(v) >> (64 - 2 * k);  // first base in the highest bits: the table's key order
     const uint64_t rc = ~v & mask;                  // reverse complement in the same order
     // the first table slot of both strands, fetched together (two dependent L2 round trips become one)
     const uint64_t slot0[2] = {(fw * 0x9E3779B97F4A7C15ull) >> V.shift, (rc * 0x9E3779B97F4A7C15ull) >> V.shift};

@@ -56,6 +56,12 @@
 //          checkpoints and samples built on the device, qm_index_build_fm), P.pac, P.ann, P.amb, and X.fa.fai; --prefix defaults
 //          to the FASTA path, as in bwa.  The FASTA is read and validated on the host before a CUDA context exists (A/C/G/T only,
 //          line lengths samtools faidx accepts, at most QM_MAX_CONTIGS contigs, 2 x length < 2^31)
+//   qm_driver genome-diff --ref R.fa --qry Q.fa [--snps OUT] [--vcf OUT.vcf] [--indels 0|1] [-l -c -g -b -d] [--gpu I] [-t THREADS]
+//        = rules/genome_diff.smk (rule nucmer: nucmer; show-snps -CTHlr <(delta-filter -r -q); mummer2vcf.py -n --output-header;
+//          bgzip; tabix): the strain pair's differences computed on the device (qm_genome_diff_host, DESIGN.md 5c).  --snps: the
+//          12 columns of show-snps -CTHlr (--indels 0: of -CTHIlr, the rows the custom evaluator reads); --vcf: mummer2vcf.py's
+//          records plus .gz and .tbi.  -l -c -g -b -d: nucmer's options of those letters.  Both FASTAs are read and checked as
+//          `index` reads them, before a CUDA context exists
 //   qm_driver bam-from-records --ref .. --r1 .. --r2 .. --alns ALNS.bin [--perm PERM.bin] --bam OUT.bam
 //        = the BAM/BAI writer alone on given qm_aln records (test entry; with --perm no GPU is touched)
 //   qm_driver fastq-check --r1 .. --r2 .. [-t THREADS] [-K N [--batch-pairs M]]
@@ -2614,6 +2620,133 @@ int cmd_index(const Args &a)
     return 0;
 }
 
+// ------------------------------------------------------------------------------------------------
+// `qm_driver genome-diff`: rule nucmer (rules/genome_diff.smk: nucmer; show-snps -CTHlr <(delta-filter -r -q); mummer2vcf.py;
+// bgzip; tabix) on the device (qm_genome_diff_host, DESIGN.md 5c).  mummer2vcf.py is not part of this project: the VCF header and
+// record shape are those of the truth VCFs it wrote for the reference (quasimodo_b200/data/truth/*.vcf.gz), without ##fileDate.
+void write_gdiff_vcf(const std::string &path, const std::string &ref_path, const Genome &r, const Genome &q, const std::vector<qm_gdiff_row> &rows)
+{
+    FILE *f = fopen(path.c_str(), "w");
+    if (!f) die(2, "cannot create %s", path.c_str());
+    fprintf(f, "##fileformat=VCFv4.2\n##source=mummer2vcf.py\n##reference=%s\n", ref_path.c_str());
+    for (size_t c = 0; c < r.names.size(); ++c) fprintf(f, "##contig=<ID=%s,length=%lld>\n", r.names[c].c_str(), (long long)r.lens[c]);
+    fputs("##INFO=<ID=DP,Number=1,Type=Integer,Description=\"Total depth of quality bases\">\n"
+          "##INFO=<ID=REF1,Number=1,Type=String,Description=\"The name of the 1st reference sequence\">\n"
+          "##INFO=<ID=REF2,Number=1,Type=String,Description=\"The name of the 2nd reference sequence\">\n"
+          "##INFO=<ID=ORIG,Number=1,Type=String,Description=\"The original position of variant at 2nd reference sequence\">\n"
+          "##INFO=<ID=TYPE,Number=1,Type=String,Description=\"Indicates that the variant is an INDEL or SNV.\">\n"
+          "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\n", f);
+    auto base = [&](int rid, int64_t p1) { return "ACGT"[r.codes[(size_t)(r.offs[rid] + p1 - 1)]]; };
+    for (size_t i = 0; i < rows.size();) {
+        const qm_gdiff_row &w = rows[i];
+        size_t j = i + 1;
+        int64_t pos;
+        std::string ref, alt;
+        const char *type = "INDEL";
+        auto indel_row = [](const qm_gdiff_row &x) { return x.sub_r == '.' || x.sub_q == '.'; };
+        if (!indel_row(w)) {                       // SNP rows of one position: one record, ALTs joined by ','
+            alt = std::string(1, w.sub_q);
+            while (j < rows.size() && rows[j].rid == w.rid && rows[j].p1 == w.p1 && !indel_row(rows[j])) {
+                if (alt.find(rows[j].sub_q) == std::string::npos) { alt += ','; alt += rows[j].sub_q; }
+                ++j;
+            }
+            pos = w.p1; ref = std::string(1, w.sub_r); type = "SNV";
+        } else if (w.sub_q == '.') {               // deletion: consecutive reference bases at one query position, anchor base first
+            while (j < rows.size() && rows[j].rid == w.rid && rows[j].sub_q == '.' && rows[j].p2 == w.p2 && rows[j].p1 == rows[j - 1].p1 + 1) ++j;
+            pos = w.p1 - 1;
+            ref = std::string(1, base(w.rid, pos));
+            for (size_t t = i; t < j; ++t) ref += rows[t].sub_r;
+            alt = std::string(1, base(w.rid, pos));
+        } else {                                   // insertion: consecutive query bases after one reference base
+            while (j < rows.size() && rows[j].rid == w.rid && rows[j].sub_r == '.' && rows[j].p1 == w.p1 && std::abs(rows[j].p2 - rows[j - 1].p2) == 1) ++j;
+            pos = w.p1;
+            ref = std::string(1, base(w.rid, pos));
+            alt = ref;
+            for (size_t t = i; t < j; ++t) alt += rows[t].sub_q;
+        }
+        const char *rn = r.names[w.rid].c_str(), *qn = q.names[w.qid].c_str();
+        fprintf(f, "%s\t%lld\t.\t%s\t%s\t30\tPASS\tDP=30;REF1=%s;REF2=%s;ORIG=%s:%d;TYPE=%s\n", rn, (long long)pos, ref.c_str(), alt.c_str(), rn, qn, qn,
+                w.p2, type);
+        i = j;
+    }
+    if (fclose(f) != 0) die(2, "cannot write %s", path.c_str());
+}
+
+int cmd_genome_diff(const Args &a)
+{
+    PhaseClock pc;
+    require_known(a, "genome-diff", {"ref", "qry", "snps", "vcf", "indels", "l", "c", "g", "b", "d", "gpu", "t", "threads"});
+    if (!a.has("ref") || !a.has("qry")) die(1, "--ref and --qry are required");
+    if (!a.has("snps") && !a.has("vcf")) die(1, "nothing to write: give --snps and / or --vcf");
+    g_threads = std::max(1, atoi(a.get("t", a.get("threads", "2")).c_str()));
+    qm_gdiff_opt o;
+    qm_gdiff_opt_default(&o);
+    auto one = [&](const char *k, int32_t &x) { if (a.has(k)) x = parse_int(k, a.get(k)); };
+    one("l", o.min_match); one("c", o.min_cluster); one("g", o.max_gap); one("b", o.break_len);
+    if (a.has("d")) {
+        char *end = nullptr;
+        const std::string v = a.get("d");
+        o.diag_factor = strtof(v.c_str(), &end);
+        if (v.empty() || *end || !(o.diag_factor >= 0.f) || !std::isfinite(o.diag_factor)) die(1, "option -d: '%s' is not a non-negative number", v.c_str());
+    }
+    if (o.min_match < 8 || o.min_match > 31) die(1, "option -l: 8 <= l <= 31 (anchors are looked up as k-mers of the index)");
+    if (o.max_gap > 4096 || o.break_len > 4096) die(1, "options -g and -b: at most 4096");
+    const int indels = a.has("indels") ? parse_int("indels", a.get("indels")) : 1;
+    if (indels > 1) die(1, "option --indels: 0 or 1");
+    if (!indels) o.flags |= QM_GDIFF_NO_INDELS;
+    Genome r, q;
+    std::vector<std::string> annos;
+    std::vector<FaiRow> fai;
+    read_fasta_for_index(a.get("ref"), r, annos, fai);
+    annos.clear(); fai.clear();
+    read_fasta_for_index(a.get("qry"), q, annos, fai);
+    pc.mark("FASTA");
+    Lib L;
+    const int dev = atoi(a.get("gpu", "0").c_str());
+    const int rc = qm_ctx_create(dev, &L.ctx);
+    if (rc != QM_OK) die(3, "qm_ctx_create(%d) failed (%d): no usable B200 (there is no CPU fallback)", dev, rc);
+    pc.mark("context");
+    qm_index *idx = nullptr;
+    L.check(qm_index_build(L.ctx, r.codes.data(), (int)r.names.size(), r.lens.data(), o.min_match, &idx), "qm_index_build");
+    pc.mark("reference index");
+    // room for one difference per 50 query bases and one alignment per 2 kb; a pair that needs more is run again at its size
+    int64_t n_rows = 0, n_alns = 0;
+    int64_t qbases = 0;
+    for (auto l : q.lens) qbases += l;
+    std::vector<qm_gdiff_row> rows((size_t)(qbases / 50 + 1024));
+    std::vector<qm_gdiff_aln> alns((size_t)(qbases / 2000 + 256));
+    double ms[5];
+    int err = qm_genome_diff_host(L.ctx, idx, q.codes.data(), (int)q.names.size(), q.lens.data(), &o, rows.data(), (int64_t)rows.size(), &n_rows,
+                                  alns.data(), (int64_t)alns.size(), &n_alns, ms);
+    if (err == QM_ELIMIT && (n_rows > (int64_t)rows.size() || n_alns > (int64_t)alns.size())) {
+        rows.resize((size_t)n_rows); alns.resize((size_t)n_alns);
+        err = qm_genome_diff_host(L.ctx, idx, q.codes.data(), (int)q.names.size(), q.lens.data(), &o, rows.data(), n_rows, &n_rows, alns.data(), n_alns,
+                                  &n_alns, ms);
+    }
+    L.check(err, "qm_genome_diff_host");
+    rows.resize((size_t)n_rows); alns.resize((size_t)n_alns);
+    qm_index_destroy(L.ctx, idx);
+    qm_ctx_destroy(L.ctx);
+    fprintf(stderr, "[qm_driver] genome-diff: %lld alignments, %lld rows; anchors %.1f ms, clusters %.1f ms, gaps %.1f ms, ends %.1f ms, rows %.1f ms\n",
+            (long long)n_alns, (long long)n_rows, ms[0], ms[1], ms[2], ms[3], ms[4]);
+    pc.mark("genome diff");
+    if (a.has("snps")) {
+        FILE *f = fopen(a.get("snps").c_str(), "w");
+        if (!f) die(2, "cannot create %s", a.get("snps").c_str());
+        for (const qm_gdiff_row &w : rows)
+            fprintf(f, "%d\t%c\t%c\t%d\t%d\t%d\t%lld\t%lld\t%d\t%d\t%s\t%s\n", w.p1, w.sub_r, w.sub_q, w.p2, w.buff, w.dist, (long long)r.lens[w.rid],
+                    (long long)q.lens[w.qid], w.frm_r, w.frm_q, r.names[w.rid].c_str(), q.names[w.qid].c_str());
+        if (fclose(f) != 0) die(2, "cannot write %s", a.get("snps").c_str());
+    }
+    if (a.has("vcf")) {
+        write_gdiff_vcf(a.get("vcf"), a.get("ref"), r, q, rows);
+        write_vcf_gz_tbi(a.get("vcf"), a.get("vcf") + ".gz", g_threads);
+    }
+    pc.mark("files");
+    pc.report();
+    return 0;
+}
+
 }  // namespace
 
 // --benchmark FILE (any command): the job's resources in the shape of a Snakemake `benchmark:` file (one header line, one row:
@@ -2656,7 +2789,7 @@ int main(int argc, char **argv)
 {
     g_benchmark_t0 = std::chrono::steady_clock::now();
     g_benchmark_cpu0 = clock();
-    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|rmdup|index|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
+    if (argc < 2) die(1, "usage: qm_driver sample|decontam|pileup|rmdup|index|genome-diff|bam-from-records|vcf-index|fastq-check|selftest [options]   (%s)", qm_version());
     std::string cmdline;
     for (int i = 0; i < argc; ++i) { if (i) cmdline += ' '; cmdline += argv[i]; }
     const std::string cmd = argv[1];
@@ -2672,6 +2805,7 @@ int main(int argc, char **argv)
     if (cmd == "pileup") return cmd_pileup(a);
     if (cmd == "rmdup") return cmd_rmdup(a, cmdline);
     if (cmd == "index") return cmd_index(a);
+    if (cmd == "genome-diff") return cmd_genome_diff(a);
     if (cmd == "fastq-check") {                        // host only: parse the two mate files as `sample` would, report what is there
         // -K N: bwa mem's input chunks of N bases as `sample -K N` cuts them, one line "chunks: size size ..." (pairs per chunk)
         require_known(a, "fastq-check", {"r1", "r2", "t", "threads", "K", "batch-pairs"});

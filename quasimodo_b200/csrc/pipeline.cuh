@@ -45,6 +45,22 @@ static __device__ __forceinline__ int qm_ref_base(const IndexView &V, int64_t x)
 {   // bwa's doubled coordinates: [l_pac, 2 l_pac) is the reverse complement strand
     return x < V.l_pac ? V.refb[x] : 3 - V.refb[2 * V.l_pac - 1 - x];
 }
+// 32 bases starting at position b >= -32 of a padded 2-bit sequence (IndexView::ref2p's layout: base x at bits 2*((x+32)&31) of
+// word (x+32)>>5); the seeding walk and the genome diff's anchors (gdiff.cu) extend exact matches through it
+static __device__ __forceinline__ uint64_t qm_get2_padded(const uint64_t *__restrict__ p, int64_t b)
+{
+    const int64_t x = b + 32;
+    const uint64_t *w = p + (x >> 5);
+    const int sh = 2 * (int)(x & 31);
+    const uint64_t lo = __ldg(w);
+    return sh ? (lo >> sh) | (__ldg(w + 1) << (64 - sh)) : lo;
+}
+// reverse the order of the 32 two-bit groups of x
+static __device__ __forceinline__ uint64_t qm_grouprev(uint64_t x)
+{
+    const uint64_t y = __brevll(x);
+    return ((y >> 1) & 0x5555555555555555ull) | ((y & 0x5555555555555555ull) << 1);
+}
 static __device__ __forceinline__ int qm_pos2rid(const IndexView &V, int64_t fpos)
 {
     int r = -1;

@@ -6,7 +6,8 @@ tests/test_driver_gpu.py checks that the command really writes every path.  pile
 `bcftools` one `qm_driver pileup` job each, on the .rmdup.bam a separate alignment step left; rmdup_command gives rule `rmdup`
 one `qm_driver rmdup` job on the sorted BAM of any aligner; index_command gives rule `build_idx` (rules/index.smk:12-14) one
 `qm_driver index` job in place of `bwa index` + `samtools faidx`; decontam_sample_command puts the decontamination rules
-`rm_phix` and `rm_human_ecoli` (rules/decontamination.smk) in front of the four in the same job."""
+`rm_phix` and `rm_human_ecoli` (rules/decontamination.smk) in front of the four in the same job; genome_diff_command gives
+rule `nucmer` (rules/genome_diff.smk) one `qm_driver genome-diff` job that writes the mixture's truth VCF."""
 import os
 
 # rule -> {output name ("" = the rule's single unnamed output): (directory variable, path pattern)}
@@ -154,3 +155,28 @@ def index_command(driver, ref_fa, threads=4, extra=(), benchmark=None):
         os.makedirs(os.path.dirname(os.path.abspath(benchmark)), exist_ok=True)
         argv += ["--benchmark", benchmark]
     return argv + list(extra), [ref_fa + s for s in BWA_INDEX_SUFFIXES] + [ref_fa + FAIDX_SUFFIX]
+
+
+# rule `nucmer` (rules/genome_diff.smk:10-11; SURVEY.md 8b, "truth"): the truth VCF of mixture {mix} and what `bgzip` and
+# `tabix -p vcf` leave next to it.  Apart from RULE_OUTPUTS, whose table is checked against the reference's read-level rules.
+NUCMER_OUTPUT = ("snp_dir", "/nucmer/{mix}.maskrepeat.variants.vcf")
+NUCMER_SIDE_FILES = (".gz", ".gz.tbi")
+# rules/genome_diff.smk:3-4: the reference of each mixture; the query is always TB40E
+NUCMER_REF = {"TM": "Merlin", "TA": "AD169"}
+NUCMER_QUERY = "TB40E"
+
+
+def genome_diff_command(driver, dirs, mix, ref_fa, qry_fa, threads=2, extra=(), snps=None, benchmark=None):
+    """-> (argv, [the VCF, its .gz and .gz.tbi]) of the replacement of rule `nucmer` for mixture `mix`: `qm_driver genome-diff` of
+    qry_fa (TB40E in the reference's workflow) against ref_fa; snps=PATH also writes the show-snps -CTHlr rows there (not part of
+    the returned list), benchmark=PATH adds `--benchmark PATH`"""
+    var, pat = NUCMER_OUTPUT
+    vcf = dirs[var] + pat.format(mix=mix)
+    os.makedirs(os.path.dirname(vcf), exist_ok=True)
+    argv = [driver, "genome-diff", "--ref", ref_fa, "--qry", qry_fa, "--vcf", vcf, "-t", str(threads)]
+    if snps:
+        argv += ["--snps", snps]
+    if benchmark:
+        os.makedirs(os.path.dirname(os.path.abspath(benchmark)), exist_ok=True)
+        argv += ["--benchmark", benchmark]
+    return argv + list(extra), [vcf] + [vcf + s for s in NUCMER_SIDE_FILES]
